@@ -15,8 +15,8 @@ legs may import it.  The product package ``photoverse_b200`` never imports ``ora
 
 Pinning: the reference ships NO tests, golden vectors or fixtures for this path (SURVEY.md §4).
 The oracle is therefore pinned against the *reference implementation itself*, imported verbatim
-from /root/reference in the build container by ``oracle/ref_loader.py`` and compared in
+from the upstream checkout named by PHOTOVERSE_REFERENCE_ROOT by ``oracle/ref_loader.py`` and compared in
 ``oracle/make_golden.py`` (which also writes ``tests/golden/*.npz``; re-run it to regenerate).
 ``tests/test_oracle_golden.py`` re-checks the oracle against those committed outputs everywhere
-(the GPU box has no /root/reference) and against the live reference when it is present.
+and against the live reference when PHOTOVERSE_REFERENCE_ROOT is set.
 """

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY -- generate tests/golden/*.npz from the VERBATIM reference.
 
-Run in the build container (needs /root/reference):
+Needs a checkout of the upstream project:
 
-    python -m oracle.make_golden
+    PHOTOVERSE_REFERENCE_ROOT=<checkout> python -m oracle.make_golden
 
 For every case in oracle/cases.py this
   1. runs the unmodified reference files (imported by oracle/ref_loader.py) in fp32 and fp64,
@@ -10,9 +10,10 @@ For every case in oracle/cases.py this
   3. asserts oracle == reference (fp64: <= 1e-12 abs; fp32: <= 2e-6 abs), i.e. pins the oracle,
   4. stores the reference's fp64-run outputs (rounded to fp32) as the golden vectors and the
      fp32-run deviation in manifest.json.
+It also records the state-dict layout, constructor defaults and constructor errors of the reference classes
+(class_layout.json).
 
-The GPU box has no /root/reference; tests there compare the oracle and the CUDA path against these
-committed outputs.
+Without a checkout, the tests compare the oracle and the CUDA path against these committed outputs.
 """
 import json
 import os
@@ -67,8 +68,29 @@ def run_reference_adapter(c: cases.AdapterCase, dtype):
         return ad(embs, token_index=c.token_index)
 
 
+CTOR_BAD_ARGS = (dict(fusion_rules=(0.5, 0.6)), dict(fusion_rules=[0.5, 0.5]), dict(scale=[1.0, 2.0]))
+
+
+def class_layout(processor_cls, adapter_cls):
+    """What a checkpoint or a caller sees of a processor / adapter class pair (attention_processor.py:27-56,
+    adapters.py:14-28): state-dict shapes and key order, constructor defaults (repr keeps their types) and the texts of
+    the constructor's ValueErrors (None where a bad argument is not rejected)."""
+    p = processor_cls(hidden_size=320, cross_attention_dim=768, num_tokens=(5,))
+    errors = []
+    for bad in CTOR_BAD_ARGS:
+        try:
+            processor_cls(320, 768, **bad)
+            errors.append(None)
+        except ValueError as e:
+            errors.append(str(e))
+    return {"processor_state_dict": [[k, list(v.shape)] for k, v in p.state_dict().items()],
+            "processor_defaults": repr((p.scale, p.fusion_rule1, p.fusion_rule2, p.num_tokens)),
+            "processor_ctor_errors": errors,
+            "adapter_state_dict_keys": list(adapter_cls(num_tokens=3).state_dict().keys())}
+
+
 def main():
-    assert ref_loader.reference_available(), "needs /root/reference"
+    assert ref_loader.reference_available(), "set PHOTOVERSE_REFERENCE_ROOT to a checkout of the upstream project"
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     manifest = {"generator": "oracle/make_golden.py", "torch": torch.__version__, "cases": {}}
     torch.set_num_threads(8)
@@ -121,6 +143,11 @@ def main():
     manifest["cases"]["inject_concept"] = {"kind": "inject", "note": "verbatim models/clip.py:_inject_concept_embeddings, "
                                                                      "first 32 of 768 channels stored"}
     print("inject_concept                   : oracle == reference (bit exact)")
+
+    layout = class_layout(ref_loader.load_reference_processor_module().PhotoVerseAttnProcessor2_0,
+                          ref_loader.load_reference_adapter_module().PhotoVerseAdapter)
+    with open(os.path.join(GOLDEN_DIR, "class_layout.json"), "w") as f:
+        json.dump({"provenance": "upstream classes, written by oracle/make_golden.py", "layout": layout}, f, indent=1)
 
     with open(os.path.join(GOLDEN_DIR, "manifest.json"), "w") as f:
         json.dump(manifest, f, indent=1, sort_keys=True)

@@ -1,4 +1,5 @@
-"""TEST INFRASTRUCTURE ONLY -- import the UNMODIFIED reference hot-path files from /root/reference.
+"""TEST INFRASTRUCTURE ONLY -- import the UNMODIFIED reference hot-path files from a checkout of the upstream project
+(idonahum/photoVerse) named by the environment variable PHOTOVERSE_REFERENCE_ROOT.
 
 The reference is pure Python; ``models/adapters.py`` needs only torch, ``models/attention_processor.py``
 imports three diffusers symbols (attention_processor.py:5-9) that are absent from this image
@@ -7,9 +8,8 @@ names and drive the verbatim file through a minimal stand-in for diffusers' ``At
 (fields listed in SURVEY.md §8b) and a stand-in for peft 0.10.0 ``lora.Linear``.
 
 Nothing here is copied from the reference: the files are executed where they lie.  This module is
-used only in the build container (``oracle/make_golden.py`` and the "live reference" leg of
-``tests/test_oracle_golden.py``); the GPU box has no /root/reference and relies on the committed
-golden outputs instead.
+used only by ``oracle/make_golden.py`` and by the "live reference" legs of the tests; without a checkout the tests
+compare against the reference outputs committed under ``tests/golden/``.
 """
 import importlib.util
 import os
@@ -19,11 +19,11 @@ import types
 import torch
 from torch import nn
 
-REFERENCE_ROOT = os.environ.get("PHOTOVERSE_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("PHOTOVERSE_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "attention_processor.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "attention_processor.py"))
 
 
 def _install_diffusers_stub():

@@ -1,9 +1,9 @@
-"""GPU x2 (B200, `gpurun --gpus 2`): the data-parallel contracts of SURVEY 4.3 / 8e on real devices with NCCL --
+"""GPU x2 (two B200s on one node): the data-parallel contracts of SURVEY 4.3 / 8e on real devices with NCCL --
   * generation: per-sample latents of a 2-rank run are BIT-IDENTICAL to one process generating the same two shards one
     after the other (samples are seeded by global index, shards are contiguous, there is no collective in the loop;
     invariance to the BATCH a sample is generated in is test_gpu_pipeline's engine test, to bf16 tolerance);
   * training: the allreduced gradients of a 2-rank step == the mean of the two single-rank gradients.
-Skipped on a single-GPU box (the driver's 1-GPU test run); the N > 1 host logic is covered on CPU by test_parallel_cpu."""
+Skipped on a machine with fewer than two GPUs; the N > 1 host logic is covered on CPU by test_parallel_cpu."""
 import json
 import os
 import socket
@@ -101,7 +101,7 @@ def _run(world, tmp):
     return [json.load(open(os.path.join(tmp, f"w{world}_r{k}.json"))) for k in range(world)]
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_two_ranks_reproduce_the_single_rank_run(cuda_device, tmp_path):
     one = _run(1, str(tmp_path))[0]
     two = _run(2, str(tmp_path))

@@ -1,5 +1,6 @@
 """CPU: the oracle restatement against the committed golden vectors (generated from the verbatim reference by
-oracle/make_golden.py) and, when /root/reference is mounted, against the live reference."""
+oracle/make_golden.py) and, when PHOTOVERSE_REFERENCE_ROOT names a checkout of the upstream project, against the live
+reference."""
 import numpy as np
 import pytest
 import torch
@@ -46,28 +47,38 @@ def test_manifest_records_reference_noise_floor():
             assert v["ref_f32_vs_f64_maxabs"] < 2e-6
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference not mounted")
+def _assert_rounds_to(y64, g32):
+    """The golden vectors are the reference's fp64 run rounded to fp32: an fp64 result equal to that run within 1e-12
+    lies within half an fp32 ulp of the stored value."""
+    assert (np.abs(y64 - g32) <= 0.5 * np.spacing(np.abs(g32)) + 1e-12).all()
+
+
 @pytest.mark.parametrize("case", cases.PROC_CASES[:3] + cases.PROC_CASES[4:7], ids=lambda c: c.name)
 def test_processor_oracle_matches_live_reference(case):
-    from oracle.make_golden import run_reference_processor
-    y_ref, n_ref = run_reference_processor(case, torch.float64)
     w = cases.proc_weights(case, torch.float64)
     x, text, img = cases.proc_inputs(case, torch.float64)
     with torch.no_grad():
         y, vn = dual_branch_attention(x, text, img, w, case.w_text, case.w_img)
-    assert (y - y_ref).abs().max().item() <= 1e-12
-    assert (vn - n_ref).abs().max().item() <= 1e-12
+    g = golden(case.name)
+    _assert_rounds_to(y.numpy(), g["y"])
+    _assert_rounds_to(vn.numpy(), g["vnorm"])
+    if ref_loader.reference_available():
+        from oracle.make_golden import run_reference_processor
+        y_ref, n_ref = run_reference_processor(case, torch.float64)
+        assert (y - y_ref).abs().max().item() <= 1e-12
+        assert (vn - n_ref).abs().max().item() <= 1e-12
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference not mounted")
 def test_adapter_oracle_matches_live_reference():
-    from oracle.make_golden import run_reference_adapter
     case = cases.ADAPTER_CASES[3]
-    y_ref = run_reference_adapter(case, torch.float64)
     sd = adapter_oracle.make_state_dict(case.T, case.seed, dtype=torch.float64)
     with torch.no_grad():
         y = adapter_oracle.adapter_forward(cases.adapter_inputs(case, torch.float64), sd, case.token_index)
-    assert (y - y_ref).abs().max().item() <= 1e-11
+    _assert_rounds_to(y.numpy(), golden(case.name)["y"])
+    if ref_loader.reference_available():
+        from oracle.make_golden import run_reference_adapter
+        y_ref = run_reference_adapter(case, torch.float64)
+        assert (y - y_ref).abs().max().item() <= 1e-11
 
 
 def test_fusion_rule_table():

@@ -256,7 +256,13 @@ int pv_dropout_bwd_acc(pv_dtype dt, void* dst, const void* src, const uint8_t* k
  * (frozen affine; mean / rstd are recomputed from the row).
  * pv_geglu_fwd: y[m, n] = h[m, n] * gelu(h[m, N + n]) with the exact (erf) GELU, gelu(.) rounded to bf16 before the
  * product like the two-kernel torch sequence; h: [M, 2N] with row stride ldh (elements), y: [M, N] dense; N % 8 == 0.
- * pv_geglu_bwd: dh [M, 2N] dense = [dy * gelu(gate) | dy * hidden * gelu'(gate)] from h and dy [M, N] dense. */
+ * pv_geglu_bwd: dh [M, 2N] dense = [dy * gelu(gate) | dy * hidden * gelu'(gate)] from h and dy [M, N] dense.
+ * pv_linear_geglu_fwd: y[m, n] = h[m, n] * gelu(h[m, N + n]) for the projection h = x W^T + b of an nn.Linear(K, 2N), in one
+ * launch without writing h: x [M, K] bf16 (row stride ldx), y [M, N] bf16 (row stride ldy).  w_packed [2N, K] bf16 dense and
+ * b_packed fp32 [2N] (or NULL) are W and b with their rows regrouped per 80 output columns: packed rows [160 j, 160 j + 80)
+ * are rows [80 j, 80 j + 80) of W, packed rows [160 j + 80, 160 j + 160) are rows N + [80 j, 80 j + 80).  h is rounded
+ * to bf16 after the bias and the rest rounds like pv_geglu_fwd.  N % 80 == 0, K % 64 == 0; a row's result does not
+ * depend on M.  The packed weight must not be written by the kernel launched just before (it is read ahead of it). */
 int64_t pv_group_norm_nhwc_ws_bytes(int64_t B, int64_t HW, int C, int groups);
 int pv_group_norm_nhwc_fwd(pv_dtype dt, const void* x, const float* add_bc, const float* gamma, const float* beta, void* y,
                            float* save_stats, void* ws, int64_t B, int64_t HW, int C, int groups, float eps, int silu,
@@ -272,6 +278,8 @@ int pv_layer_norm_bwd(pv_dtype dt, const void* x, const void* dy, const float* g
                       void* stream);
 int pv_geglu_fwd(pv_dtype dt, const void* h, void* y, int64_t M, int N, int64_t ldh, void* stream);
 int pv_geglu_bwd(pv_dtype dt, const void* h, const void* dy, void* dh, int64_t M, int N, int64_t ldh, void* stream);
+int pv_linear_geglu_fwd(pv_dtype dt, const void* x, const void* w_packed, const float* b_packed, void* y, int64_t M, int64_t N,
+                        int64_t K, int64_t ldx, int64_t ldy, void* stream);
 
 #ifdef __cplusplus
 }

@@ -90,6 +90,8 @@ int layer_norm_bf16(const void* x, const void* res, void* sum_out, const float* 
 int layer_norm_bwd_bf16(const void* x, const void* dy, const float* gamma, void* dx, long long rows, int C, float eps,
                         cudaStream_t stream);
 int geglu(const void* h, void* y, long long M, int N, long long ldh, cudaStream_t stream);
+int linear_geglu_bf16(const void* x, const void* Wp, const float* bp, void* y, long long M, long long N, long long K,
+                      long long ldx, long long ldy, cudaStream_t stream);
 int geglu_bwd(const void* h, const void* dy, void* dh, long long M, int N, long long ldh, cudaStream_t stream);
 int dropout_bwd_acc(bool bf16, void* dst, const void* src, const uint8_t* mask, float alpha, long long n,
                     cudaStream_t stream);
@@ -562,6 +564,13 @@ int pv_geglu_bwd(pv_dtype dt, const void* h, const void* dy, void* dh, int64_t M
   PV_REQUIRE(h && dy && dh, "null pointer");
   PV_REQUIRE(dt == PV_BF16, "bf16 activations only");
   return geglu_bwd(h, dy, dh, M, N, ldh, as_stream(stream));
+}
+
+int pv_linear_geglu_fwd(pv_dtype dt, const void* x, const void* w_packed, const float* b_packed, void* y, int64_t M, int64_t N,
+                        int64_t K, int64_t ldx, int64_t ldy, void* stream) {
+  PV_REQUIRE(x && w_packed && y, "null pointer");
+  PV_REQUIRE(dt == PV_BF16, "bf16 activations only");
+  return linear_geglu_bf16(x, w_packed, b_packed, y, M, N, K, ldx, ldy, as_stream(stream));
 }
 
 }  // extern "C"

@@ -11,6 +11,9 @@
 //   * epilogue warps (2 x 4 per CTA): TMEM -> +bias -> bf16 -> per-warp staging tile -> TMA store
 // The single-CTA kernel of pv_gemm.cu spends most of a K = 320 tile in its prologue / epilogue (5 K-blocks) and is bound
 // by TMA ingest (36 KB per K-block); this one has neither problem.
+//
+// linear_geglu_bf16 runs the same pipeline with the GEGLU epilogue: the feed-forward projection of a transformer block and
+// its `a * gelu(gate)` in one launch, so the [M, 2N] projection never goes through global memory.
 #include "pv_common.cuh"
 #include "pv_outproj.cuh"
 #include "pv_host.h"
@@ -22,7 +25,9 @@ constexpr int G3_THREADS = 384;          // warp 0 TMA, warp 1 MMA (leader), war
 
 // The pipeline itself is outproj_phase (pv_outproj.cuh) -- the same code that runs as the second phase of the fused
 // processor kernels -- here without row-block counters (every A tile is ready when the kernel starts).
-template <typename Cfg>
+// EPI = OP_EPI_GEGLU: D[M, N / 2] = GEGLU of the packed projection (see pv_outproj.cuh); a pair's tiles are the contiguous
+// share [T p / npairs, T (p + 1) / npairs) of the T = G V (group, unit) entries instead of the units of one group.
+template <typename Cfg, int EPI>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G3_THREADS, 1)
 gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                              const __grid_constant__ CUtensorMap tmD, const float* __restrict__ bias, int G, int V, int K,
@@ -30,19 +35,30 @@ gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gr
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (Cfg::BYTES + 15) / 16 * 16);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + OP_BAR_BYTES / 8);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + OP_BAR_BYTES / 8 + (EPI == OP_EPI_GEGLU ? 1 : 0));   // after w_free
   const int warp = threadIdx.x >> 5;
   const int pair = blockIdx.x >> 1;
   const int npairs = gridDim.x >> 1;
-  const int g = pair % G;
-  const int r_pair = pair / G;
-  const int npair_g = (npairs - g + G - 1) / G;
+  int g, u0, u1;
+  if constexpr (EPI == OP_EPI_GEGLU) {
+    const long long T = static_cast<long long>(G) * V;
+    u0 = static_cast<int>(T * pair / npairs);
+    u1 = static_cast<int>(T * (pair + 1) / npairs);
+    g = u0 / V;
+  } else {
+    g = pair % G;
+    const int r_pair = pair / G;
+    const int npair_g = (npairs - g + G - 1) / G;
+    u0 = static_cast<int>((static_cast<long long>(V) * r_pair) / npair_g);
+    u1 = static_cast<int>((static_cast<long long>(V) * (r_pair + 1)) / npair_g);
+  }
 
   if (warp == 0 && (threadIdx.x & 31) == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmW);
     tma_prefetch_desc(&tmD);
     op_mbar_init(bars);
+    if constexpr (EPI == OP_EPI_GEGLU) mbar_init(bars + OP_W_FREE, 1);
     fence_barrier_init();
   }
   if (warp == 2) tmem_alloc_2sm<512>(tmem_slot);
@@ -51,8 +67,6 @@ gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gr
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
-  const int u0 = static_cast<int>((static_cast<long long>(V) * r_pair) / npair_g);
-  const int u1 = static_cast<int>((static_cast<long long>(V) * (r_pair + 1)) / npair_g);
   // Nothing above reads global memory.  `w_static` (set only by the processor's own out-projection call, whose Wo was
   // packed many kernels earlier): the resident W half is requested before the dependency wait, under the predecessor's
   // tail; on the generic pv_linear_fwd route W, bias, A and D are all touched only after the predecessor has completed.
@@ -76,7 +90,7 @@ gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gr
   oa.ready_target = 0;
   oa.w_preloaded = Cfg::WSTAT && w_static && u0 < u1;
   oa.trace = nullptr; oa.trace_cap = 0; oa.trace_block = 0;
-  outproj_phase<Cfg>(smem, bars, tmem, &tmA, &tmW, &tmD, oa);
+  outproj_phase<Cfg, EPI>(smem, bars, tmem, &tmA, &tmW, &tmD, oa);
 
   tc_fence_before();
   __syncthreads();
@@ -85,13 +99,13 @@ gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gr
   if (warp == 2) tmem_dealloc_2sm<512>(tmem);
 }
 
-template <int KB_RES, int STAGES>
+template <int KB_RES, int STAGES, int EPI = OP_EPI_BIAS>
 static int launch_g3(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorMap& tmD, const float* bias, int G, int V,
                      int K, int w_static, cudaStream_t stream) {
   using Cfg = OutProjCfg<KB_RES, STAGES>;
   constexpr int SMEM_BYTES = (Cfg::BYTES + 15) / 16 * 16 + 256 + 1024;
-  static_assert(OP_BAR_BYTES + 8 <= 256 && SMEM_BYTES <= 227 * 1024, "shared memory budget");
-  auto kern = gemm3_pair_persistent_kernel<Cfg>;
+  static_assert(OP_BAR_BYTES + 8 + 8 <= 256 && SMEM_BYTES <= 227 * 1024, "shared memory budget");
+  auto kern = gemm3_pair_persistent_kernel<Cfg, EPI>;
   PV_CUDA(set_max_smem_once(kern, SMEM_BYTES));
   const long long units = static_cast<long long>(G) * V;
   const long long max_pairs = sm_count() / 2;
@@ -116,6 +130,29 @@ int gemm3_bf16(const void* A, const void* W, const float* bias, void* D, long lo
   if (K == 320) return launch_g3<5, 8>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream);
   if (K == 640) return launch_g3<10, 5>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream);
   return launch_g3<0, 7>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream);
+}
+
+// y[M, N] (bf16, row stride ldy) = GEGLU of x[M, K] (ldx) * Wp[2N, K]^T + bp, with Wp / bp packed per 80 output columns
+// (rows [160 j, 160 j + 80) = value rows [80 j, 80 j + 80) of the nn.Linear(K, 2N), rows [160 j + 80, 160 j + 160) = gate rows
+// N + [80 j, 80 j + 80)); N % 80 == 0, K % 64 == 0.  No split-K: a row's result does not depend on M or on its tile.
+int linear_geglu_bf16(const void* x, const void* Wp, const float* bp, void* y, long long M, long long N, long long K,
+                      long long ldx, long long ldy, cudaStream_t stream) {
+  PV_REQUIRE(M > 0 && N > 0 && K > 0 && N % (OP_BN / 2) == 0 && K % OP_BK == 0,
+             "linear_geglu: need M > 0, N %% 80 == 0 and K %% 64 == 0 (M=%lld N=%lld K=%lld)", M, N, K);
+  PV_REQUIRE(ldx >= K && ldy >= N && ldx % 8 == 0 && ldy % 8 == 0, "linear_geglu: row strides must be >= the row and 16-byte multiples (ldx=%lld ldy=%lld)", ldx, ldy);
+  PV_REQUIRE((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(Wp) | reinterpret_cast<uintptr_t>(y)) % 16 == 0,
+             "linear_geglu: pointers must be 16-byte aligned");
+  const long long G = 2 * N / OP_BN;
+  const long long V = (M + 255) / 256;
+  PV_REQUIRE(V * G < (1ll << 30), "too many tiles");
+  CUtensorMap tmA, tmW, tmD;
+  if (make_tmap_3d(&tmA, x, 2, K, M, 1, ldx * 2, ldx * M * 2, OP_BK, 128, 1, Swz::B128)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmW, Wp, 2, K, 2 * N, 1, K * 2, K * 2 * N * 2, OP_BK, OP_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmD, y, 2, N, M, 1, ldy * 2, ldy * M * 2, 40, 32, 1, Swz::None)) return PV_ERR_CUDA;
+  // the packed weight is a cached copy of a parameter, never written by the kernel this launch may overlap (w_static)
+  if (K == 320) return launch_g3<5, 8, OP_EPI_GEGLU>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
+  if (K == 640) return launch_g3<10, 5, OP_EPI_GEGLU>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
+  return launch_g3<0, 7, OP_EPI_GEGLU>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
 }
 
 }  // namespace pv

@@ -8,6 +8,12 @@
 // The pipeline is the persistent CTA-pair GEMM of pv_gemm3.cu (W slice split across the pair and resident for C <= 640,
 // deep A ring, M = 256 cta_group::2 MMAs into double-buffered TMEM accumulators, bias / bf16 / TMA-store epilogue under
 // the next tile's MMAs) with 3-D (channel, row, sample) coordinates so that tiles coincide with attention units.
+//
+// The same pipeline with the GEGLU epilogue (OP_EPI_GEGLU, pv_gemm3.cu only) computes a transformer block's feed-forward
+// projection y = (x Wa^T + ba) * gelu(x Wg^T + bg) in one launch: the weight is packed so that the 160 rows of column group
+// g are the 80 value rows of output columns [80 g, 80 g + 80) followed by their 80 gate rows, and each epilogue warp group
+// holds both operands of its 40 outputs.  There a pair's tiles are a contiguous range of the flattened (group, unit)
+// list, which may cross into the next column group (the resident W slice is then reloaded).
 #pragma once
 #include "pv_common.cuh"
 #include "pv_softmax.cuh"
@@ -20,6 +26,10 @@ constexpr int OP_A_BYTES = 128 * OP_BK * 2;
 constexpr int OP_WH_BYTES = (OP_BN / 2) * OP_BK * 2;
 constexpr int OP_MAX_STAGES = 8;
 constexpr int OP_BAR_BYTES = (2 * OP_MAX_STAGES + 5) * 8;     // full[8] empty[8] acc_full[2] slot_free[2] w_full
+constexpr int OP_W_FREE = 2 * OP_MAX_STAGES + 5;              // GEGLU only: w_free (resident W slice read by the last MMA)
+
+constexpr int OP_EPI_BIAS = 0;     // D = acc + bias                                   (D: 160 columns per group)
+constexpr int OP_EPI_GEGLU = 1;    // D = bf16(acc_a + b_a) * bf16(gelu(bf16(acc_g + b_g)))  (D: 80 columns per group)
 
 template <int KB_RES, int NSTAGES>                            // resident K-blocks of the W half (0: streamed)
 struct OutProjCfg {
@@ -45,6 +55,7 @@ struct OutProjArgs {
   int G, MTP, C;
   int V;                   // units per column group = B * MTP
   int u0, u1;              // this pair's tiles: units [u0, u1) of column group g
+                           // (OP_EPI_GEGLU: entries [u0, u1) of the flattened list, entry f = unit f % V of group f / V)
   int g;
   unsigned int ready_target;   // arrivals that complete a row block: (draining warps per unit) x G
   int w_preloaded;             // the resident W half has already been requested (op_preload_w)
@@ -100,26 +111,125 @@ __device__ __forceinline__ void bulk_wait_all() {             // groups complete
   asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
 }
 
+// The exact (erf) GELU of a bf16 value, in the expression of geglu_kernel (pv_backbone.cu) so that both round alike.
+__device__ __forceinline__ float op_gelu_erf(float g) { return 0.5f * g * (1.f + erff(g * 0.70710678118654752f)); }
+
+// The GEGLU epilogue (warps 4..11 of both CTAs).  Warp group w takes the value columns [40 w, 40 w + 40) and the gate
+// columns [80 + 40 w, 80 + 40 w + 40) of the accumulator, i.e. output columns [80 g + 40 w, 80 g + 40 w + 40) of its 32
+// rows; the staging tile is 32 rows x 80 bytes (16-byte stores of a quarter warp land in 8 distinct bank quads).
+// Rounding points of the two-launch path (bf16 projection, then geglu_kernel): h_a and h_g are rounded to bf16 after the
+// bias, gelu(h_g) is rounded to bf16, and the product of the two bf16 values is rounded once (fma.rn.bf16x2 with -0).
+__device__ __forceinline__ void op_geglu_epilogue(uint8_t* smem_ost, float* sbias, uint64_t* acc_full, uint64_t* slot_free,
+                                                  uint32_t tmem, const CUtensorMap* tmD, const OutProjArgs& a) {
+  const int warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const uint32_t rank = cluster_ctarank();
+  const int w = (warp - 4) >> 2;
+  const int q = warp & 3;
+  const uint32_t tlane = tmem + (static_cast<uint32_t>(q * 32) << 16);
+  uint8_t* ost = smem_ost + (warp - 4) * (32 * 80 * 2);
+  float* gbias = sbias + 80 * w;                             // [0, 40): value bias, [40, 80): gate bias of this group
+  const uint32_t bias_a = smem_u32(gbias);
+  const uint32_t ost_a = smem_u32(ost);
+  auto load_bias = [&](int g) {
+    for (int c = q * 32 + lane; c < 80; c += 128)
+      gbias[c] = a.bias ? a.bias[g * OP_BN + (c < 40 ? 40 * w + c : 80 + 40 * w + (c - 40))] : 0.f;
+  };
+  int gb = a.u0 < a.u1 ? a.u0 / a.V : 0;                    // group whose bias is in shared memory
+  load_bias(gb);
+  named_bar_sync(9 + w, 128);
+  int i = 0;
+  for (int f = a.u0; f < a.u1; ++f, ++i) {
+    const int g = f / a.V;
+    const int u = f - g * a.V;
+    const int slot = i & 1;
+    const int m0 = (2 * u + static_cast<int>(rank)) * 128;
+    if (g != gb) {                                          // the range crossed into the next column group
+      named_bar_sync(9 + w, 128);
+      gb = g;
+      load_bias(gb);
+      named_bar_sync(9 + w, 128);
+    }
+    mbar_wait(&acc_full[slot], (i >> 1) & 1);
+    tc_fence_after();
+    uint32_t v[80];                                          // [0, 40): value accumulators, [40, 80): gate accumulators
+    const uint32_t src = tlane + slot * OP_BN + 40 * w;
+    tmem_ld32_raw(src, v);
+    tmem_ld_x8(src + 32, *reinterpret_cast<uint32_t(*)[8]>(v + 32));
+    tmem_ld32_raw(src + 80, v + 40);
+    tmem_ld_x8(src + 112, *reinterpret_cast<uint32_t(*)[8]>(v + 72));
+    tmem_ld_wait();
+    tc_fence_before();
+    __syncwarp();
+    if (elect_one()) mbar_arrive_cluster(mapa_u32(smem_u32(&slot_free[slot]), 0));   // accumulator is in registers
+    if (elect_one()) bulk_wait_read<0>();                // previous TMA store of this warp has read the staging tile
+    __syncwarp();
+    uint32_t y[20];                                          // word k = output columns 2k, 2k + 1
+#pragma unroll
+    for (int c = 0; c < 10; ++c) {
+      float4 ba, bg;
+      asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(ba.x), "=f"(ba.y), "=f"(ba.z), "=f"(ba.w) : "r"(bias_a + c * 16));
+      asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(bg.x), "=f"(bg.y), "=f"(bg.z), "=f"(bg.w) : "r"(bias_a + 160 + c * 16));
+      const float bav[4] = {ba.x, ba.y, ba.z, ba.w};
+      const float bgv[4] = {bg.x, bg.y, bg.z, bg.w};
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        const int j = 4 * c + 2 * k;
+        const uint32_t ha = pack_bf16x2(__uint_as_float(v[j]) + bav[2 * k], __uint_as_float(v[j + 1]) + bav[2 * k + 1]);
+        const uint32_t hg = pack_bf16x2(__uint_as_float(v[40 + j]) + bgv[2 * k], __uint_as_float(v[41 + j]) + bgv[2 * k + 1]);
+        const uint32_t ge = pack_bf16x2(op_gelu_erf(__uint_as_float(hg << 16)), op_gelu_erf(__uint_as_float(hg & 0xffff0000u)));
+        uint32_t p;
+        asm("fma.rn.bf16x2 %0, %1, %2, %3;" : "=r"(p) : "r"(ha), "r"(ge), "r"(0x80008000u));
+        y[2 * c + k] = p;
+      }
+    }
+    const uint32_t row_a = ost_a + lane * 80;
+#pragma unroll
+    for (int c = 0; c < 5; ++c) st_shared_v4_a(row_a + c * 16, y[4 * c], y[4 * c + 1], y[4 * c + 2], y[4 * c + 3]);
+    fence_proxy_async_smem();
+    __syncwarp();
+    if (elect_one()) {
+      tma_store_3d(tmD, ost, 80 * g + 40 * w, m0 + q * 32, 0);
+      bulk_commit();
+    }
+    __syncwarp();
+  }
+  if (elect_one()) bulk_wait_read<0>();
+  __syncwarp();
+}
+
 // Runs the out-projection tiles of this pair.  Every thread of BOTH CTAs of the pair calls it after a CTA + cluster
 // barrier that closed the attention phase (shared memory [0, Cfg::BYTES) and all 512 TMEM columns are free, the barriers
 // at `pb` were initialised by op_mbar_init at kernel start and never used).  Roles: warp 0 producer (both CTAs),
 // warp 1 MMA issuer (leader), warps 4..11 epilogue (both CTAs); other warps return at once.
-template <typename Cfg>
+// OP_EPI_GEGLU (plain GEMM only, a.sync == nullptr) also needs the w_free barrier at pb[OP_W_FREE], initialised with count 1.
+template <typename Cfg, int EPI = OP_EPI_BIAS>
 __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint32_t tmem, const CUtensorMap* tmA,
                                               const CUtensorMap* tmW, const CUtensorMap* tmD, const OutProjArgs& a) {
   constexpr bool WSTAT = Cfg::WSTAT;
+  constexpr bool GEGLU = EPI == OP_EPI_GEGLU;
   constexpr int nst = Cfg::STAGES;
   uint64_t* full = pb;
   uint64_t* empty = full + OP_MAX_STAGES;
   uint64_t* acc_full = empty + OP_MAX_STAGES;
   uint64_t* slot_free = acc_full + 2;
   uint64_t* w_full = slot_free + 2;
+  uint64_t* w_free = pb + OP_W_FREE;
   float* sbias = reinterpret_cast<float*>(smem + Cfg::OFF_BIAS);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
   const int kblocks = a.C / OP_BK;
   const int n0 = a.g * OP_BN;
+  // tile index -> (column group, unit): the identity on a.g for the bias epilogue, the flattened list for GEGLU
+  auto group_of = [&](int u) -> int {
+    if constexpr (GEGLU) return u / a.V;
+    else return a.g;
+  };
+  auto unit_of = [&](int u) -> int {
+    if constexpr (GEGLU) return u - (u / a.V) * a.V;
+    else return u;
+  };
 
   if (warp == 0) {
     // ===================== producer (both CTAs): resident W half, then the A (= O) tiles as they become ready ==========
@@ -156,9 +266,21 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
       if (!a.w_preloaded && a.u0 < a.u1 && elect_one()) op_preload_w<Cfg>(smem, pb, tmW, a.g, rank);
       __syncwarp();
     }
+    [[maybe_unused]] int gw = a.g;                // column group of the resident W slice
+    [[maybe_unused]] uint32_t w_loads = 0;
     for (int u = a.u0; u < a.u1; ++u) {
-      const int b = u / a.MTP;
-      const int mt = 2 * (u - b * a.MTP) + static_cast<int>(rank);
+      if constexpr (GEGLU && WSTAT) {
+        if (group_of(u) != gw) {
+          // the range crossed into the next column group: once the MMAs have read the old slice, load the new one
+          mbar_wait(w_free, w_loads & 1);
+          ++w_loads;
+          gw = group_of(u);
+          if (elect_one()) op_preload_w<Cfg>(smem, pb, tmW, gw, rank);
+          __syncwarp();
+        }
+      }
+      const int b = unit_of(u) / a.MTP;
+      const int mt = 2 * (unit_of(u) - b * a.MTP) + static_cast<int>(rank);
       const int t = u - a.u0;
       if (has_sync) {
         bool observed = false;
@@ -199,7 +321,7 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
           if (rank == 0) mbar_expect_tx(&full[s], 2 * Cfg::STAGE_BYTES);
           tma_load_3d_2sm_hint(a_dst, tmA, bar, kb * OP_BK, mt * 128, b, pol_a);
           if constexpr (!WSTAT)
-            tma_load_3d_2sm(a_dst + OP_A_BYTES, tmW, bar, kb * OP_BK, n0 + static_cast<int>(rank) * (OP_BN / 2), 0);
+            tma_load_3d_2sm(a_dst + OP_A_BYTES, tmW, bar, kb * OP_BK, group_of(u) * OP_BN + static_cast<int>(rank) * (OP_BN / 2), 0);
         }
         __syncwarp();
       }
@@ -228,9 +350,18 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
       if constexpr (WSTAT) {
         if (a.u0 < a.u1) mbar_wait(w_full, 0);
       }
+      [[maybe_unused]] int gw = a.g;
+      [[maybe_unused]] uint32_t w_loads = 0;
       for (int u = a.u0; u < a.u1; ++u, ++i) {
         const int slot = i & 1;
         if (i >= 2) mbar_wait(&slot_free[slot], ((i >> 1) - 1) & 1);
+        if constexpr (GEGLU && WSTAT) {
+          if (group_of(u) != gw) {                 // the producer has reloaded the resident W slice for this group
+            ++w_loads;
+            gw = group_of(u);
+            mbar_wait(w_full, w_loads & 1);
+          }
+        }
         tc_fence_after();
         for (int kb = 0; kb < kblocks; ++kb, ++it) {
           const int s = it % nst;
@@ -246,6 +377,9 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
             for (int k = 0; k < OP_BK / 16; ++k) umma_bf16_ss_2sm(tmem + slot * OP_BN, da + 2 * k, dw + 2 * k, idesc, (kb | k) != 0);
             umma_commit_2sm(&empty[s]);
             if (kb == kblocks - 1) umma_commit_2sm(&acc_full[slot]);
+            if constexpr (GEGLU && WSTAT) {
+              if (kb == kblocks - 1 && u + 1 < a.u1 && group_of(u + 1) != gw) umma_commit_2sm(w_free);
+            }
           }
           __syncwarp();
         }
@@ -253,6 +387,8 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
       }
       a3_trace_done_raw(a.trace, tr, 5);
     }
+  } else if (GEGLU && warp >= 4 && warp < 12) {
+    op_geglu_epilogue(smem + Cfg::OFF_OST, sbias, acc_full, slot_free, tmem, tmD, a);
   } else if (warp >= 4 && warp < 12) {
     // ===================== epilogue (both CTAs): group w handles columns [80 w, 80 w + 80) =====================
     const int w = (warp - 4) >> 2;

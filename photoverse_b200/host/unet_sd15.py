@@ -212,7 +212,23 @@ class GEGLU(nn.Module):
         super().__init__()
         self.proj = nn.Linear(dim_in, dim_out * 2)
 
+    def _packed(self):
+        """The projection's weight and bias in the row order of ops.linear_geglu, refreshed when a parameter changes."""
+        ps = (self.proj.weight, self.proj.bias)
+        key = tuple((p.data_ptr(), p._version) for p in ps)
+        cached = getattr(self, "_pv_geglu", None)
+        if cached is None or cached[0] != key:
+            from .. import ops
+            cached = (key, ops.pack_geglu_weight(*ps))
+            self._pv_geglu = cached
+        return cached[1]
+
     def forward(self, x):
+        if (_fused(self, x) and x.is_contiguous() and x.shape[-1] % 64 == 0 and self.proj.out_features % 160 == 0
+                and self.proj.bias is not None):
+            # inference: projection and GEGLU product in one launch; the [M, 2N] projection is never written
+            from .. import ops
+            return ops.linear_geglu(x, *self._packed())
         h = self.proj(x)
         if _enabled(self, h) and h.is_contiguous() and h.shape[-1] % 16 == 0:
             if torch.is_grad_enabled() and h.requires_grad:

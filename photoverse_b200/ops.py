@@ -491,6 +491,42 @@ def geglu(h: torch.Tensor) -> torch.Tensor:
     return y
 
 
+def pack_geglu_weight(w: torch.Tensor, b: Optional[torch.Tensor]):
+    """The ``nn.Linear(K, 2N)`` weight ``[2N, K]`` and bias of a GEGLU projection in the row order :func:`linear_geglu` reads:
+    per 80 output columns j, the 80 value rows ``[80 j, 80 j + 80)`` then the 80 gate rows ``N + [80 j, 80 j + 80)``.
+    Returns (bf16 contiguous weight, fp32 bias or None).  N % 80 == 0."""
+    two_n, K = w.shape
+    N = two_n // 2
+    if two_n % 2 or N % 80:
+        raise ValueError(f"pack_geglu_weight: need 2N rows with N % 80 == 0 (got {two_n})")
+    def regroup(t):
+        return torch.stack([t[:N].reshape(N // 80, 80, *t.shape[1:]), t[N:].reshape(N // 80, 80, *t.shape[1:])], 1).reshape(t.shape)
+    wp = regroup(w.detach()).to(torch.bfloat16).contiguous()
+    bp = None if b is None else regroup(b.detach()).float().contiguous()
+    return wp, bp
+
+
+def linear_geglu(x: torch.Tensor, w_packed: torch.Tensor, b_packed: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """``h[..., :N] * gelu(h[..., N:])`` with ``h = x @ W.T + b`` in one launch (the projection is never written):
+    ``x`` ``[..., K]`` contiguous bf16; ``w_packed`` / ``b_packed`` from :func:`pack_geglu_weight`.  Rounds like
+    ``linear`` to a bf16 ``h`` followed by :func:`geglu`."""
+    if not (x.is_cuda and x.dtype == torch.bfloat16 and x.is_contiguous()):
+        raise _lib.PhotoverseB200Error("linear_geglu: contiguous CUDA bfloat16 input required (there is no CPU path)")
+    if not (w_packed.dtype == torch.bfloat16 and w_packed.dim() == 2 and w_packed.is_contiguous()):
+        raise _lib.PhotoverseB200Error("linear_geglu: contiguous bfloat16 [2N, K] packed weight required")
+    two_n, K = w_packed.shape
+    if x.shape[-1] != K:
+        raise _lib.PhotoverseB200Error(f"linear_geglu: input has {x.shape[-1]} features, the weight {K}")
+    if b_packed is not None and not (b_packed.dtype == torch.float32 and b_packed.is_contiguous() and b_packed.numel() == two_n):
+        raise _lib.PhotoverseB200Error("linear_geglu: contiguous float32 [2N] packed bias required")
+    N = two_n // 2
+    M = x.numel() // K
+    y = torch.empty(*x.shape[:-1], N, device=x.device, dtype=x.dtype)
+    check(_lib.lib().pv_linear_geglu_fwd(PV_BF16, _ptr(x), _ptr(w_packed), _ptr(b_packed), _ptr(y), M, N, K, K, N, _stream()),
+          "pv_linear_geglu_fwd")
+    return y
+
+
 def geglu_bwd(h: torch.Tensor, dy: torch.Tensor) -> torch.Tensor:
     """Gradient of :func:`geglu` with respect to the ``[..., 2N]`` projection ``h`` from ``dy`` ``[..., N]`` (both contiguous bf16)."""
     if not (h.is_cuda and h.dtype == torch.bfloat16 and h.is_contiguous() and dy.dtype == h.dtype and dy.is_contiguous()):

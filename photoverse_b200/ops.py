@@ -60,7 +60,9 @@ def pack_weight(w: torch.Tensor, out: torch.Tensor, lora_A=None, lora_B=None, sc
 def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None,
            out: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """out[..., N] = a[..., K] @ w[..., N, K]^T + bias.  a: [M,K] or [batch,M,K]; w: [N,K] or [batch,N,K];
-    bias fp32 [N] or [batch,N].  Inner-most dims must be contiguous; ``out`` may be a strided view."""
+    bias fp32 [N] or [batch,N].  Inner-most dims must be contiguous; ``out`` may be a strided view whose rows are 16-byte
+    aligned.  Rows are stored in whole 16-byte units: when N elements are not a multiple of 16 bytes, the columns from N up
+    to the next 16-byte boundary of each row are set to zero (the zero K extension autograd._skinny_linear relies on)."""
     batched = a.dim() == 3
     if not batched:
         a3 = a.unsqueeze(0)
@@ -227,12 +229,16 @@ def _workspace(nbytes: int, device) -> torch.Tensor:
 
 
 def transpose(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """out[c, r] = x[r, c] for a 2-D tensor with contiguous rows."""
+    """out[c, r] = x[r, c] for a 2-D tensor with contiguous rows.  ``out`` must have dense rows (row stride R): the kernel
+    zero-fills every column up to the row stride, which for a row-padded ``out`` lies outside the view."""
     R, C = x.shape
     assert x.stride(1) == 1
     if out is None:
         out = torch.empty(C, R, device=x.device, dtype=x.dtype)
     assert out.shape == (C, R) and out.stride(1) == 1
+    if out.stride(0) != R:
+        raise ValueError(f"transpose: out must have row stride {R} (got {out.stride(0)}); columns up to the row stride "
+                         "would be zero-filled")
     check(_lib.lib().pv_transpose_2d(_dt(x), _ptr(x), _ptr(out), R, C, x.stride(0), out.stride(0), _stream()), "pv_transpose_2d")
     return out
 

@@ -24,7 +24,11 @@ def _lib_loaded():
 @pytest.mark.parametrize("swz", [0, 1])
 @pytest.mark.parametrize("out_f32", [False, True])
 @pytest.mark.parametrize("M,N,K,bn", [(256, 320, 320, 0), (300, 640, 768, 0), (128, 1280, 1280, 256), (77 * 2, 640, 768, 160),
-                                      (1000, 768, 2048, 128), (64, 64, 64, 64), (8, 1024, 1024, 0)])
+                                      (1000, 768, 2048, 128), (64, 64, 64, 64), (8, 1024, 1024, 0),
+                                      # K % 64 != 0 of the LoRA-dropout training path: K = C + pad8(r) (the low-rank columns
+                                      # appended to the projection input) and K = pad8(r) (the (dY B) A product)
+                                      (4103, 320, 8, 0), (1000, 768, 16, 0), (4096, 320, 328, 0), (1232, 640, 776, 0),
+                                      (1232, 640, 784, 0), (256, 1280, 1288, 0)])
 def test_linear_bf16(cuda_device, M, N, K, bn, out_f32, swz):
     from photoverse_b200 import _lib, ops
     _lib.set_option("epi_swizzle", swz)

@@ -19,6 +19,11 @@
  *   - pv_dtype selects the arithmetic path:
  *        PV_BF16  bf16 storage, tcgen05 tensor-core MMAs with fp32 accumulation in TMEM (throughput mode)
  *        PV_F32   fp32 storage, fp32 FFMA arithmetic (parity mode: <= 1e-4 of the fp32 reference)
+ *        PV_F16   fp16 storage, the PV_BF16 kernels with fp16 operands (kind::f16 MMAs, fp32 accumulation), for models
+ *                 run in float16.  Inference only: pv_pack_weight, pv_linear_fwd, pv_kv_tile_bytes, pv_kv_pack_fwd,
+ *                 pv_dual_attn_fwd, pv_dual_attn_core_fwd, pv_ln_lrelu_fwd and pv_group_mean_fwd accept it (wherever
+ *                 they say PV_BF16 below, the same holds for PV_F16); every other entry point returns PV_ERR_UNSUPPORTED.
+ *                 Values are rounded to fp16 (to nearest) exactly where the PV_BF16 path rounds to bf16.
  *   - there is NO CPU fallback: without a CUDA device every compute entry point returns PV_ERR_CUDA
  */
 #ifndef PHOTOVERSE_B200_H_
@@ -33,7 +38,7 @@ extern "C" {
 #define PV_ABI_VERSION 2
 
 enum { PV_OK = 0, PV_ERR_INVALID = 1, PV_ERR_CUDA = 2, PV_ERR_UNSUPPORTED = 3 };
-typedef enum { PV_F32 = 0, PV_BF16 = 1 } pv_dtype;
+typedef enum { PV_F32 = 0, PV_BF16 = 1, PV_F16 = 2 } pv_dtype;
 
 /* Keys are zero-padded to this many rows per (sample, head) in the packed K/V tiles. */
 #define PV_KEYS_PAD 96
@@ -75,7 +80,8 @@ int pv_pack_weight(pv_dtype out_dt, const float* W, const float* lora_A, const f
  * D[b] = A[b] * W[b]^T + bias[b]     A:[batch,M,K] (row stride lda, batch stride strideA, elements)
  *                                    W:[batch,N,K] (ldw, strideW; strideW == 0 -> one shared weight)
  *                                    bias fp32 [batch,N] (strideBias) or NULL;  D:[batch,M,N] (ldd, strideD)
- * dt is the type of A and W; out_dt the type of D.  PV_BF16: K % 8 == 0 and 16-byte aligned rows.
+ * dt is the type of A and W; out_dt the type of D (dt or, for PV_BF16 / PV_F16, PV_F32).  PV_BF16 / PV_F16: K % 8 == 0
+ * and 16-byte aligned rows.
  * Replaces nn.Linear (attention_processor.py:297,304,305,392,393,423; adapters.py:14-28).
  * Stream-ordering precondition: W and bias must not be the OUTPUT of the kernel enqueued immediately before this
  * call on `stream` (they are weights: the persistent kernels fetch them before their programmatic-dependent-launch
@@ -127,7 +133,7 @@ int pv_dual_attn_core_fwd(pv_dtype dt, const void* XorQ, const void* Wq, const v
 
 /* ---- adapter epilogues (adapters.py:15-16,18-19: LayerNorm(1024) -> LeakyReLU(0.01)) ----------------
  * y = leaky_relu(layer_norm(x) * gamma + beta); x:[rows,cols] fp32 (row stride ldx), y:[rows,cols] out_dt
- * (row stride ldy); cols % 128 == 0, cols <= 4096.  Optional mean / rstd [rows] fp32 saved for backward.
+ * (row stride ldy; PV_F32, PV_BF16 or PV_F16); cols % 128 == 0, cols <= 4096.  Optional mean / rstd [rows] fp32 saved for backward.
  * gamma/beta:[groups,cols]; row i uses group i / rows_per_group (rows_per_group <= 0: one shared gamma/beta) --
  * the T token heads of an adapter are normalised in one launch.
  * One warp per row, 16-byte vector loads, warp-shuffle reductions.                                        */
@@ -136,7 +142,7 @@ int pv_ln_lrelu_fwd(pv_dtype out_dt, const float* x, const float* gamma, const f
                     int64_t rows_per_group, float eps, float slope, void* stream);
 /* y[g, :] = mean over the P rows of group g: x:[groups,P,cols] (in_dt) -> y:[groups,cols] (out_dt, row stride ldy)
  * (adapters.py:36,41 `.mean(dim=1, keepdim=True)` over the 256 patch tokens, commuted in front of the last
- * Linear: mean(L3(h)) == L3(mean(h)), SURVEY 2.2 A8).                                                       */
+ * Linear: mean(L3(h)) == L3(mean(h)), SURVEY 2.2 A8).  A 16-bit in_dt and a 16-bit out_dt must be the same type.   */
 int pv_group_mean_fwd(pv_dtype in_dt, pv_dtype out_dt, const void* x, void* y, int64_t groups, int P, int cols,
                       int64_t ldy, void* stream);
 

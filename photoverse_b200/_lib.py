@@ -11,6 +11,7 @@ LIB_PATH = os.environ.get("PV_LIB_PATH") or os.path.join(_HERE, "libphotoverse_b
 
 PV_F32 = 0
 PV_BF16 = 1
+PV_F16 = 2          # inference only (include/photoverse_b200.h)
 PV_KEYS_PAD = 96
 
 

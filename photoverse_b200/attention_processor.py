@@ -9,7 +9,8 @@ and diffusers' ``Attention.forward`` can install and call it unchanged.  All ari
 Differences in *how* (not what) it computes, see DESIGN.md:
   * the two SDPA calls + add (:317-319, :400-402, :412) are one kernel: QK^T over the concatenated text+image keys,
     softmax normalised per segment, branch weights folded into P, one PV contraction;
-  * LoRA on to_q/to_k/to_v is merged into the packed bf16/fp32 weights on the GPU whenever a factor changes;
+  * LoRA on to_q/to_k/to_v is merged into the packed bf16/fp16/fp32 weights on the GPU whenever a factor changes;
+  * float16 models run the bf16 tensor-core kernels with fp16 operands (inference only: grad mode raises);
   * K/V projections can be cached across denoising steps (``kv_cache`` context) because
     ``encoder_hidden_states`` is constant during generation (models/infer.py:89-98).
 """
@@ -21,7 +22,9 @@ from torch import nn
 from . import ops
 from .lora import linear_parts
 
-_SUPPORTED = (torch.bfloat16, torch.float32)
+_SUPPORTED = (torch.bfloat16, torch.float16, torch.float32)
+_F16_TRAINING = ("float16 runs the inference (no_grad) path only: training runs in bfloat16 or float32 "
+                 "(cast the model, or run the forward under torch.no_grad() without LoRA dropout)")
 
 
 class PhotoVerseAttnProcessor(nn.Module):
@@ -277,7 +280,7 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         if getattr(attn, "residual_connection", False) or getattr(attn, "rescale_output_factor", 1.0) != 1.0:
             raise NotImplementedError("residual_connection / rescale_output_factor != 1 unsupported")
         if hidden_states.dtype not in _SUPPORTED:
-            raise TypeError(f"hidden_states must be bfloat16 or float32, got {hidden_states.dtype}")
+            raise TypeError(f"hidden_states must be bfloat16, float16 or float32, got {hidden_states.dtype}")
         if not hidden_states.is_cuda:
             raise RuntimeError("photoverse_b200 runs on CUDA only (no CPU fallback)")
 
@@ -293,6 +296,8 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
             or any(p.requires_grad for p in self.parameters())
             or any(p.requires_grad for m in (attn.to_q, attn.to_k, attn.to_v, attn.to_out[0]) for p in m.parameters()))
         if needs_grad or self.lora_dropout_active(attn):
+            if dtype == torch.float16:
+                raise NotImplementedError(_F16_TRAINING)
             from .autograd import dual_attn_autograd
             y, vnorm = dual_attn_autograd(self, attn, x, text, img, w_text, w_img)
             self.to_v_ip_norm = vnorm.to(dtype).unsqueeze(-1)

@@ -75,7 +75,7 @@ struct Attn3Cfg {
 struct Attn3Params {
   const uint8_t* Kp;
   const uint8_t* Vp;
-  __nv_bfloat16* O;        // [B,S,C]
+  void* O;                 // [B,S,C]
   float* stats;            // optional [B,H,S,4]
   int S, C, H, Lt, Li;
   int G, MT;               // head groups per sample (C/160), row tiles per sample
@@ -86,7 +86,7 @@ struct Attn3Params {
   int trace_cap;
 };
 
-template <int D, bool LT77, bool WSTAT>
+template <int D, bool LT77, bool WSTAT, typename T>
 __global__ void __launch_bounds__(A3_THREADS, 1)
 dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmWq,
                                 const __grid_constant__ CUtensorMap tmO, const Attn3Params p) {
@@ -203,7 +203,7 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
     }
   } else if (warp == 1) {
     // ===================== projection MMA issuer: Q(unit) = X Wq^T  (M=128, N=160, K=C) =====================
-    constexpr uint32_t idesc_q = umma_idesc_bf16(A3_BM, A3_BN);
+    constexpr uint32_t idesc_q = umma_idesc<T>(A3_BM, A3_BN);
     A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 0);
     uint32_t it = 0;
     int i = 0;
@@ -244,8 +244,8 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
     // The tensor pipe executes the MMAs of this thread in order, which is what makes the TMEM re-use legal:
     //   S/P buffer of nn+2 <- overwritten only after PV(nn) has read P(nn);   O(w) columns <- overwritten only after
     //   the QK^T MMAs that read the packed Q living there.
-    constexpr uint32_t idesc_s = umma_idesc_bf16(A3_BM, A3_KEYS);
-    constexpr uint32_t idesc_o = umma_idesc_bf16(A3_BM, (D == 160) ? 80 : D_PAD);
+    constexpr uint32_t idesc_s = umma_idesc<T>(A3_BM, A3_KEYS);
+    constexpr uint32_t idesc_o = umma_idesc<T>(A3_BM, (D == 160) ? 80 : D_PAD);
     A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 1);
     const int nheads = (u1 - u0) * HPC;
     int issued_qk = 0;
@@ -351,7 +351,7 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
         for (int k = 0; k < 4; ++k) {
           float a, b2;
           f2_unpack(f2_mul(f2_pack(__uint_as_float(v[c * 8 + 2 * k]), __uint_as_float(v[c * 8 + 2 * k + 1])), sc2), a, b2);
-          w4[k] = pack_bf16x2(a, b2);
+          w4[k] = pack_x2<T>(a, b2);
         }
         st_shared_v4(ost + lane * (Cfg::OW * 2) + (col0 + c * 8) * 2, w4[0], w4[1], w4[2], w4[3]);
       }
@@ -412,8 +412,8 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
           tmem_ld_x32(tslot + 40 * j, a);
           tmem_ld_x8(tslot + 40 * j + 32, c8);
           tmem_ld_wait();
-          pack_pairs3<32>(a, o);
-          pack_pairs3<8>(c8, o + 16);
+          pack_pairs3<32, T>(a, o);
+          pack_pairs3<8, T>(c8, o + 16);
           o[20] = o[21] = o[22] = o[23] = 0u;          // dims 40..47 pad the K = 48 contraction
           tmem_st_x16(tslot + 40 * j + 16, o);
           tmem_st_x8(tslot + 40 * j + 32, o + 16);
@@ -426,9 +426,9 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
         tmem_ld_x32(tslot + wg * 80 + 32, b2);
         tmem_ld_x16(tslot + wg * 80 + 64, c16);
         tmem_ld_wait();
-        pack_pairs3<32>(a, o);
-        pack_pairs3<32>(b2, o + 16);
-        pack_pairs3<16>(c16, o + 32);
+        pack_pairs3<32, T>(a, o);
+        pack_pairs3<32, T>(b2, o + 16);
+        pack_pairs3<16, T>(c16, o + 32);
         const uint32_t dstc = tslot + ((D == 80) ? (wg * 80 + 40) : (40 + wg * 40));
         tmem_st_x16(dstc, o);
         tmem_st_x16(dstc + 16, o + 16);
@@ -567,11 +567,11 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
             for (int k = 0; k < 16; ++k) {
               const int e = 32 * c + 2 * k;
               if (e < A3_IMG_OFF) {
-                pk[k] = text_on ? pack_bf16x2(__uint_as_float(sr[e]), __uint_as_float(sr[e + 1])) : 0u;
+                pk[k] = text_on ? pack_x2<T>(__uint_as_float(sr[e]), __uint_as_float(sr[e + 1])) : 0u;
               } else {
                 float a, b2;
                 f2_unpack(f2_mul(f2_pack(__uint_as_float(sr[e]), __uint_as_float(sr[e + 1])), fi2), a, b2);
-                pk[k] = pack_bf16x2(a, b2);
+                pk[k] = pack_x2<T>(a, b2);
               }
             }
             tmem_st_x16(sbuf + 16 * c, pk);
@@ -608,11 +608,11 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
 extern unsigned long long* g_attn3_trace;
 extern int g_attn3_trace_cap;
 
-template <int D, bool LT77, bool WSTAT>
+template <int D, bool LT77, bool WSTAT, typename T>
 static int launch_attn3(const CUtensorMap& tmX, const CUtensorMap& tmWq, const CUtensorMap& tmO, const Attn3Params& p,
                         cudaStream_t stream) {
   using Cfg = Attn3Cfg<D, WSTAT>;
-  auto kern = dual_attn_fwd_persistent_kernel<D, LT77, WSTAT>;
+  auto kern = dual_attn_fwd_persistent_kernel<D, LT77, WSTAT, T>;
   PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
   const long long sms = sm_count();
   const int grid = static_cast<int>(p.units < sms ? p.units : sms);
@@ -623,7 +623,7 @@ static int launch_attn3(const CUtensorMap& tmX, const CUtensorMap& tmWq, const C
 
 int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats,
                                    int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                                   cudaStream_t stream) {
+                                   cudaStream_t stream, bool f16) {
   PV_REQUIRE(B > 0 && S > 0 && H > 0 && C % H == 0, "bad shape B=%d S=%d C=%d H=%d", B, S, C, H);
   const int d = C / H;
   PV_REQUIRE(d == 40 || d == 80 || d == 160, "head_dim %d unsupported (40/80/160)", d);
@@ -633,13 +633,13 @@ int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp
   PV_REQUIRE((reinterpret_cast<uintptr_t>(X) | reinterpret_cast<uintptr_t>(Wq) | reinterpret_cast<uintptr_t>(Kp) |
               reinterpret_cast<uintptr_t>(Vp) | reinterpret_cast<uintptr_t>(O)) % 16 == 0, "pointers must be 16-byte aligned");
   CUtensorMap tmX, tmWq, tmO;
-  if (make_tmap_3d(&tmX, X, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, A3_BK, A3_BM, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmWq, Wq, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, A3_BK, A3_BN, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmO, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, d == 160 ? 80 : d, 32, 1, Swz::None)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmX, X, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, A3_BK, A3_BM, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmWq, Wq, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, A3_BK, A3_BN, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmO, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, d == 160 ? 80 : d, 32, 1, Swz::None, f16)) return PV_ERR_CUDA;
   Attn3Params p;
   p.Kp = static_cast<const uint8_t*>(Kp);
   p.Vp = static_cast<const uint8_t*>(Vp);
-  p.O = static_cast<__nv_bfloat16*>(O);
+  p.O = O;
   p.stats = stats;
   p.S = S; p.C = C; p.H = H; p.Lt = Lt; p.Li = Li;
   p.G = C / A3_BN;
@@ -651,14 +651,17 @@ int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp
   p.trace = g_attn3_trace;
   p.trace_cap = g_attn3_trace_cap;
   p.scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(d));
+#define PV_A3_LAUNCH(DD, LT, WS)                                                                  \
+  (f16 ? launch_attn3<DD, LT, WS, __half>(tmX, tmWq, tmO, p, stream)                              \
+       : launch_attn3<DD, LT, WS, __nv_bfloat16>(tmX, tmWq, tmO, p, stream))
   switch (d) {
     case 40:
-      if (C == A3_KB_WSTAT * A3_BK)
-        return Lt == 77 ? launch_attn3<40, true, true>(tmX, tmWq, tmO, p, stream) : launch_attn3<40, false, true>(tmX, tmWq, tmO, p, stream);
-      return Lt == 77 ? launch_attn3<40, true, false>(tmX, tmWq, tmO, p, stream) : launch_attn3<40, false, false>(tmX, tmWq, tmO, p, stream);
-    case 80: return Lt == 77 ? launch_attn3<80, true, false>(tmX, tmWq, tmO, p, stream) : launch_attn3<80, false, false>(tmX, tmWq, tmO, p, stream);
-    default: return Lt == 77 ? launch_attn3<160, true, false>(tmX, tmWq, tmO, p, stream) : launch_attn3<160, false, false>(tmX, tmWq, tmO, p, stream);
+      if (C == A3_KB_WSTAT * A3_BK) return Lt == 77 ? PV_A3_LAUNCH(40, true, true) : PV_A3_LAUNCH(40, false, true);
+      return Lt == 77 ? PV_A3_LAUNCH(40, true, false) : PV_A3_LAUNCH(40, false, false);
+    case 80: return Lt == 77 ? PV_A3_LAUNCH(80, true, false) : PV_A3_LAUNCH(80, false, false);
+    default: return Lt == 77 ? PV_A3_LAUNCH(160, true, false) : PV_A3_LAUNCH(160, false, false);
   }
+#undef PV_A3_LAUNCH
 }
 
 }  // namespace pv

@@ -79,7 +79,7 @@ struct Attn4Params {
   unsigned int* sync;          // [2 * V] row-block counters, zero between launches (pv_outproj.cuh)
 };
 
-template <int D, bool LT77, bool WSTAT, bool FUSE>
+template <int D, bool LT77, bool WSTAT, bool FUSE, typename T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(A4_THREADS, 1)
 dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmWq,
                           const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmOa,
@@ -244,7 +244,7 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
     }
   } else if (warp == 1 && rank == 0) {
     // ===================== projection MMA issuer (leader): Q = X Wq^T for BOTH CTAs, M = 256, N = 160 =====================
-    constexpr uint32_t idesc_q = umma_idesc_bf16(2 * A4_BM, A4_BN);
+    constexpr uint32_t idesc_q = umma_idesc<T>(2 * A4_BM, A4_BN);
     A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 0);
     uint32_t it = 0;
     int i = 0;
@@ -279,8 +279,8 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
     a3_trace_done_raw(p.trace, tr, 0);
   } else if (warp == 2 && rank == 0) {
     // ===================== attention MMA issuer (leader), flat loop over the heads (see pv_attn3.cu) =====================
-    constexpr uint32_t idesc_s = umma_idesc_bf16(2 * A4_BM, A4_KEYS);
-    constexpr uint32_t idesc_o = umma_idesc_bf16(2 * A4_BM, Cfg::NB);
+    constexpr uint32_t idesc_s = umma_idesc<T>(2 * A4_BM, A4_KEYS);
+    constexpr uint32_t idesc_o = umma_idesc<T>(2 * A4_BM, Cfg::NB);
     A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 1);
     const int nheads = (u1 - u0) * HPC;
     int issued_qk = 0;
@@ -384,7 +384,7 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
         for (int k = 0; k < 4; ++k) {
           float a, b2;
           f2_unpack(f2_mul(f2_pack(__uint_as_float(v[c * 8 + 2 * k]), __uint_as_float(v[c * 8 + 2 * k + 1])), sc2), a, b2);
-          w4[k] = pack_bf16x2(a, b2);
+          w4[k] = pack_x2<T>(a, b2);
         }
         st_shared_v4(ost + lane * (Cfg::OW * 2) + (col0 + c * 8) * 2, w4[0], w4[1], w4[2], w4[3]);
       }
@@ -437,8 +437,8 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
           tmem_ld_x32(tslot + 40 * j, a);
           tmem_ld_x8(tslot + 40 * j + 32, c8);
           tmem_ld_wait();
-          pack_pairs3<32>(a, o);
-          pack_pairs3<8>(c8, o + 16);
+          pack_pairs3<32, T>(a, o);
+          pack_pairs3<8, T>(c8, o + 16);
           o[20] = o[21] = o[22] = o[23] = 0u;          // dims 40..47 pad the K = 48 contraction
           tmem_st_x16(tslot + 40 * j + 16, o);
           tmem_st_x8(tslot + 40 * j + 32, o + 16);
@@ -451,9 +451,9 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
         tmem_ld_x32(tslot + wg * 80 + 32, b2);
         tmem_ld_x16(tslot + wg * 80 + 64, c16);
         tmem_ld_wait();
-        pack_pairs3<32>(a, o);
-        pack_pairs3<32>(b2, o + 16);
-        pack_pairs3<16>(c16, o + 32);
+        pack_pairs3<32, T>(a, o);
+        pack_pairs3<32, T>(b2, o + 16);
+        pack_pairs3<16, T>(c16, o + 32);
         const uint32_t dstc = tslot + ((D == 80) ? (wg * 80 + 40) : (40 + wg * 40));
         tmem_st_x16(dstc, o);
         tmem_st_x16(dstc + 16, o + 16);
@@ -610,11 +610,11 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
             for (int k = 0; k < 16; ++k) {
               const int e = 32 * c + 2 * k;
               if (e < A4_IMG_OFF) {
-                pk[k] = text_on ? pack_bf16x2(__uint_as_float(sr[e]), __uint_as_float(sr[e + 1])) : 0u;
+                pk[k] = text_on ? pack_x2<T>(__uint_as_float(sr[e]), __uint_as_float(sr[e + 1])) : 0u;
               } else {
                 float a, b2;
                 f2_unpack(f2_mul(f2_pack(__uint_as_float(sr[e]), __uint_as_float(sr[e + 1])), fi2), a, b2);
-                pk[k] = pack_bf16x2(a, b2);
+                pk[k] = pack_x2<T>(a, b2);
               }
             }
             tmem_st_x16(sbuf + 16 * c, pk);
@@ -681,7 +681,7 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
     oa.w_preloaded = 0;
     oa.ready_target = static_cast<unsigned int>(16 * p.G);       // 8 softmax warps x 2 CTAs announce every unit
     oa.trace = p.trace; oa.trace_cap = p.trace_cap; oa.trace_block = 0;
-    outproj_phase<typename Cfg::OP>(smem, reinterpret_cast<uint64_t*>(smem + Cfg::OFF_BAR + Cfg::OP_BAR_OFF), tmem, &tmOa, &tmWo,
+    outproj_phase<typename Cfg::OP, OP_EPI_BIAS, T>(smem, reinterpret_cast<uint64_t*>(smem + Cfg::OFF_BAR + Cfg::OP_BAR_OFF), tmem, &tmOa, &tmWo,
                                     &tmY, oa);
   }
 
@@ -695,12 +695,12 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
 extern unsigned long long* g_attn3_trace;
 extern int g_attn3_trace_cap;
 
-template <int D, bool LT77, bool WSTAT, bool FUSE>
+template <int D, bool LT77, bool WSTAT, bool FUSE, typename T>
 static int launch_attn4(const CUtensorMap& tmX, const CUtensorMap& tmWq, const CUtensorMap& tmO, const CUtensorMap& tmOa,
                         const CUtensorMap& tmWo, const CUtensorMap& tmY, const Attn4Params& p, long long unit_pairs,
                         cudaStream_t stream) {
   using Cfg = Attn4Cfg<D, WSTAT>;
-  auto kern = dual_attn_fwd_pair_kernel<D, LT77, WSTAT, FUSE>;
+  auto kern = dual_attn_fwd_pair_kernel<D, LT77, WSTAT, FUSE, T>;
   PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
   const long long max_pairs = sm_count() / 2;
   const int npairs = static_cast<int>(unit_pairs < max_pairs ? unit_pairs : max_pairs);
@@ -714,7 +714,7 @@ static int launch_attn4(const CUtensorMap& tmX, const CUtensorMap& tmWq, const C
 // (pv_outproj.cuh), O also left in global memory, `sync` = 2 * B * ceil(S / 256) zeroed counters (left zeroed).
 int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats, int B,
                              int S, int C, int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream,
-                             const void* Wo, const float* bo, void* Y, unsigned int* sync) {
+                             const void* Wo, const float* bo, void* Y, unsigned int* sync, bool f16) {
   PV_REQUIRE(B > 0 && S > 0 && H > 0 && C % H == 0, "bad shape B=%d S=%d C=%d H=%d", B, S, C, H);
   const int d = C / H;
   PV_REQUIRE(d == 40 || d == 80 || d == 160, "head_dim %d unsupported (40/80/160)", d);
@@ -727,13 +727,13 @@ int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, cons
               reinterpret_cast<uintptr_t>(Vp) | reinterpret_cast<uintptr_t>(O) | reinterpret_cast<uintptr_t>(Wo) |
               reinterpret_cast<uintptr_t>(Y)) % 16 == 0, "pointers must be 16-byte aligned");
   CUtensorMap tmX, tmWq, tmO, tmOa, tmWo, tmY;
-  if (make_tmap_3d(&tmX, X, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, A4_BK, A4_BM, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmWq, Wq, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, A4_BK, A4_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmO, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, d == 160 ? 80 : d, 32, 1, Swz::None)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmX, X, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, A4_BK, A4_BM, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmWq, Wq, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, A4_BK, A4_BN / 2, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmO, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, d == 160 ? 80 : d, 32, 1, Swz::None, f16)) return PV_ERR_CUDA;
   if (fuse) {
-    if (make_tmap_3d(&tmOa, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, OP_BK, 128, 1, Swz::B128)) return PV_ERR_CUDA;
-    if (make_tmap_3d(&tmWo, Wo, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, OP_BK, OP_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
-    if (make_tmap_3d(&tmY, Y, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, 80, 32, 1, Swz::None)) return PV_ERR_CUDA;
+    if (make_tmap_3d(&tmOa, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, OP_BK, 128, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+    if (make_tmap_3d(&tmWo, Wo, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, OP_BK, OP_BN / 2, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+    if (make_tmap_3d(&tmY, Y, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, 80, 32, 1, Swz::None, f16)) return PV_ERR_CUDA;
   } else {
     tmOa = tmO; tmWo = tmO; tmY = tmO;
   }
@@ -754,7 +754,9 @@ int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, cons
   p.scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(d));
   p.bias = bo;
   p.sync = sync;
-#define PV_A4_LAUNCH(DD, LT, WS, FU) launch_attn4<DD, LT, WS, FU>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)
+#define PV_A4_LAUNCH(DD, LT, WS, FU)                                                                          \
+  (f16 ? launch_attn4<DD, LT, WS, FU, __half>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)         \
+       : launch_attn4<DD, LT, WS, FU, __nv_bfloat16>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream))
 #define PV_A4_LT(DD, WS, FU) (Lt == 77 ? PV_A4_LAUNCH(DD, true, WS, FU) : PV_A4_LAUNCH(DD, false, WS, FU))
   switch (d) {
     case 40:

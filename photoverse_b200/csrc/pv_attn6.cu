@@ -92,7 +92,7 @@ struct Attn6Params {
   int mufu_token;          // d = 40: the two softmax groups take turns on the exponentials
 };
 
-template <int D, bool LT77, bool FUSE>
+template <int D, bool LT77, bool FUSE, typename T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(A6_THREADS, 1)
 dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmWq,
                                 const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmOa,
@@ -277,7 +277,7 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
     } else if (warp == 1) {
       if (rank == 0) {
         // ===================== projection MMA issuer (leader): Q = X Wq^T for BOTH CTAs, M = 256, N = 160 =====================
-        constexpr uint32_t idesc_q = umma_idesc_bf16(2 * A6_BM, A6_BN);
+        constexpr uint32_t idesc_q = umma_idesc<T>(2 * A6_BM, A6_BN);
         A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 0, p.trace_block);
         a3_trace(tr, 1, static_cast<int>(t_sync - t_entry));      // prologue: barrier init, TMEM allocation, cluster sync
         a3_trace(tr, 2, static_cast<int>(t_pdl - t_entry));       // ... + wait for the predecessor grid
@@ -315,7 +315,7 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
       if (rank == 0) {
         // ===================== QK^T issuer (leader): S(nn) = Q_head K_head^T, one head ahead of each softmax group ============
         // Needs: packed bf16 Q of the unit (q_ready), the sample's K/V (kv_both), S buffer nn & 1 read out (s_free).
-        constexpr uint32_t idesc_s = umma_idesc_bf16(2 * A6_BM, A6_KEYS);
+        constexpr uint32_t idesc_s = umma_idesc<T>(2 * A6_BM, A6_KEYS);
         A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 1, p.trace_block);
         const uint64_t kdesc0 = umma_desc(smem_u32(kv), 48 * 16, 128, UMMA_LAYOUT_NONE);
         uint32_t kv_gen = 0;
@@ -353,7 +353,7 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
       // Needs: P tile + row scales in shared memory (p_ready), the group's O accumulator drained (o_free).  PV(nn)
       // overwrites TMEM columns that held the packed Q of heads 0 / 1 of the slot: their QK^T completed before the
       // softmax group could read S, i.e. before p_ready.
-      constexpr uint32_t idesc_o = umma_idesc_bf16(2 * A6_BM, A6_DPAD);
+      constexpr uint32_t idesc_o = umma_idesc<T>(2 * A6_BM, A6_DPAD);
       const uint64_t vdesc0 = umma_desc(smem_u32(kv + A6_KH_BYTES), (A6_DPAD / 2) * 16, 128, UMMA_LAYOUT_NONE);
       const uint64_t pdesc0 = umma_desc(smem_u32(smem + A6_OFF_P), A6_BM * 16, 128, UMMA_LAYOUT_NONE);
       A3Trace tr = a3_trace_init_raw(p.trace, p.trace_cap, 6, p.trace_block);   // (role 6 belongs to phase 2 in the fused kernels)
@@ -598,13 +598,13 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
             if (c < A6_IMG_OFF / 8) {
 #pragma unroll
               for (int k = 0; k < 4; ++k)
-                pk[k] = text ? pack_bf16x2(__uint_as_float(sr[8 * c + 2 * k]), __uint_as_float(sr[8 * c + 2 * k + 1])) : 0u;
+                pk[k] = text ? pack_x2<T>(__uint_as_float(sr[8 * c + 2 * k]), __uint_as_float(sr[8 * c + 2 * k + 1])) : 0u;
             } else {
 #pragma unroll
               for (int k = 0; k < 4; ++k) {
                 float a, b2;
                 f2_unpack(f2_mul(f2_pack(__uint_as_float(sr[8 * c + 2 * k]), __uint_as_float(sr[8 * c + 2 * k + 1])), fi2), a, b2);
-                pk[k] = pack_bf16x2(a, b2);
+                pk[k] = pack_x2<T>(a, b2);
               }
             }
             st_shared_v4_a(ptile_a + c * (A6_BM * 16), pk[0], pk[1], pk[2], pk[3]);
@@ -679,8 +679,8 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
           tmem_ld_x32(tslot + 40 * j, a);
           tmem_ld_x8(tslot + 40 * j + 32, c8);
           tmem_ld_wait();
-          pack_pairs3<32>(a, o);
-          pack_pairs3<8>(c8, o + 16);
+          pack_pairs3<32, T>(a, o);
+          pack_pairs3<8, T>(c8, o + 16);
           o[20] = o[21] = o[22] = o[23] = 0u;
           tmem_st_x16(tslot + 40 * j + 16, o);
           tmem_st_x8(tslot + 40 * j + 32, o + 16);
@@ -691,8 +691,8 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
             tmem_ld_x32(tslot + 80 * j + 40 * hh, a);
             tmem_ld_x8(tslot + 80 * j + 40 * hh + 32, c8);
             tmem_ld_wait();
-            pack_pairs3<32>(a, o);
-            pack_pairs3<8>(c8, o + 16);
+            pack_pairs3<32, T>(a, o);
+            pack_pairs3<8, T>(c8, o + 16);
             tmem_st_x16(tslot + 80 * j + 40 + 20 * hh, o);
             tmem_st_x4(tslot + 80 * j + 40 + 20 * hh + 16, o + 16);
           }
@@ -731,7 +731,7 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
           for (int k = 0; k < 4; ++k) {
             float x0, x1;
             f2_unpack(f2_mul(f2_pack(__uint_as_float(v[c * 8 + 2 * k]), __uint_as_float(v[c * 8 + 2 * k + 1])), sc2), x0, x1);
-            w4[k] = pack_bf16x2(x0, x1);
+            w4[k] = pack_x2<T>(x0, x1);
           }
           st_shared_v4(slab + lane * (A6_D * 2) + (col0 + c * 8) * 2, w4[0], w4[1], w4[2], w4[3]);
         }
@@ -819,7 +819,7 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
     oa.w_preloaded = 1;
     oa.ready_target = static_cast<unsigned int>(8 * p.G);        // 4 epilogue warps x 2 CTAs announce every unit
     oa.trace = p.trace; oa.trace_cap = p.trace_cap; oa.trace_block = p.trace_block;
-    outproj_phase<typename Cfg::OP>(smem, reinterpret_cast<uint64_t*>(smem + A6_OFF_BAR + Cfg::OP_BAR_OFF), tmem, &tmOa, &tmWo,
+    outproj_phase<typename Cfg::OP, OP_EPI_BIAS, T>(smem, reinterpret_cast<uint64_t*>(smem + A6_OFF_BAR + Cfg::OP_BAR_OFF), tmem, &tmOa, &tmWo,
                                     &tmY, oa);
     a3_pair_time(p.trace, p.trace_block, 3);     // the producer (thread 0's warp) has issued its last load
   }
@@ -838,11 +838,11 @@ extern int g_opt_trace_block;
 extern int g_opt_attn6_prefetch;
 extern int g_opt_attn6_token;
 
-template <int D, bool LT77, bool FUSE>
+template <int D, bool LT77, bool FUSE, typename T>
 static int launch_attn6(const CUtensorMap& tmX, const CUtensorMap& tmWq, const CUtensorMap& tmO, const CUtensorMap& tmOa,
                         const CUtensorMap& tmWo, const CUtensorMap& tmY, const Attn6Params& p, long long unit_pairs,
                         cudaStream_t stream) {
-  auto kern = dual_attn_fwd_pair_roles_kernel<D, LT77, FUSE>;
+  auto kern = dual_attn_fwd_pair_roles_kernel<D, LT77, FUSE, T>;
   PV_CUDA(set_max_smem_once(kern, Attn6Cfg<D>::SMEM_BYTES));
   const long long max_pairs = sm_count() / 2;
   const int npairs = static_cast<int>(unit_pairs < max_pairs ? unit_pairs : max_pairs);
@@ -869,7 +869,8 @@ bool dual_attn_pair_roles_fused_supported(int S, int C, int H) {
 // zero-initialised counters that the kernel leaves zeroed.
 int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats,
                                    int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                                   cudaStream_t stream, const void* Wo, const float* bo, void* Y, unsigned int* sync) {
+                                   cudaStream_t stream, const void* Wo, const float* bo, void* Y, unsigned int* sync,
+                                   bool f16) {
   PV_REQUIRE(B > 0 && dual_attn_pair_roles_supported(S, C, H), "needs head_dim 40 with C=320 or head_dim 80, S>128 (B=%d S=%d C=%d H=%d)",
              B, S, C, H);
   const bool fuse = Wo != nullptr;
@@ -882,13 +883,13 @@ int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp
               reinterpret_cast<uintptr_t>(Vp) | reinterpret_cast<uintptr_t>(O) | reinterpret_cast<uintptr_t>(Wo) |
               reinterpret_cast<uintptr_t>(Y)) % 16 == 0, "pointers must be 16-byte aligned");
   CUtensorMap tmX, tmWq, tmO, tmOa, tmWo, tmY;
-  if (make_tmap_3d(&tmX, X, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, A6_BK, A6_BM, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmWq, Wq, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, A6_BK, A6_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmO, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, d, 32, 1, Swz::None)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmX, X, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, A6_BK, A6_BM, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmWq, Wq, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, A6_BK, A6_BN / 2, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmO, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, d, 32, 1, Swz::None, f16)) return PV_ERR_CUDA;
   if (fuse) {
-    if (make_tmap_3d(&tmOa, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, OP_BK, 128, 1, Swz::B128)) return PV_ERR_CUDA;
-    if (make_tmap_3d(&tmWo, Wo, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, OP_BK, OP_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
-    if (make_tmap_3d(&tmY, Y, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, 80, 32, 1, Swz::None)) return PV_ERR_CUDA;
+    if (make_tmap_3d(&tmOa, O, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, OP_BK, 128, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+    if (make_tmap_3d(&tmWo, Wo, 2, C, C, 1, C * 2ull, static_cast<uint64_t>(C) * C * 2, OP_BK, OP_BN / 2, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+    if (make_tmap_3d(&tmY, Y, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, 80, 32, 1, Swz::None, f16)) return PV_ERR_CUDA;
   } else {
     tmOa = tmO; tmWo = tmO; tmY = tmO;
   }
@@ -912,7 +913,9 @@ int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp
   p.sync = sync;
   p.prefetch_s = g_opt_attn6_prefetch;
   p.mufu_token = g_opt_attn6_token;
-#define PV_A6_LAUNCH(DD, LT, FU) launch_attn6<DD, LT, FU>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)
+#define PV_A6_LAUNCH(DD, LT, FU)                                                                         \
+  (f16 ? launch_attn6<DD, LT, FU, __half>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)        \
+       : launch_attn6<DD, LT, FU, __nv_bfloat16>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream))
   if (d == 40) {
     if (fuse) return Lt == 77 ? PV_A6_LAUNCH(40, true, true) : PV_A6_LAUNCH(40, false, true);
     return Lt == 77 ? PV_A6_LAUNCH(40, true, false) : PV_A6_LAUNCH(40, false, false);

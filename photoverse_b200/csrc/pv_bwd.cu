@@ -16,7 +16,8 @@ namespace pv {
 
 int gemm_bf16(const void* A, const void* W, const float* bias, void* D, bool out_f32, long long M, long long N,
               long long K, long long batch, long long lda, long long ldw, long long ldd, long long strideA,
-              long long strideW, long long strideBias, long long strideD, cudaStream_t stream, bool w_static = false);
+              long long strideW, long long strideBias, long long strideD, cudaStream_t stream, bool w_static = false,
+              bool f16 = false);
 
 template <typename T> __device__ __forceinline__ float ldf(const T* p);
 template <> __device__ __forceinline__ float ldf<float>(const float* p) { return *p; }

@@ -4,9 +4,12 @@
 
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+
+#include <type_traits>
 
 namespace pv {
 
@@ -19,6 +22,18 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);   // .x = lo -> low 16 bits -> lower address
   return *reinterpret_cast<uint32_t*>(&v);
+}
+__device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
+  __half2 v = __floats2half2_rn(lo, hi);               // round to nearest even, like pack_bf16x2
+  return *reinterpret_cast<uint32_t*>(&v);
+}
+// The 16-bit operand type T of the tcgen05 kind::f16 kernels: __nv_bfloat16 (PV_BF16) or __half (PV_F16).  pack_x2<T> is
+// the one fp32 -> 16-bit conversion of those kernels (two values, lo at the lower address).
+template <typename T>
+__device__ __forceinline__ uint32_t pack_x2(float lo, float hi) {
+  static_assert(std::is_same<T, __nv_bfloat16>::value || std::is_same<T, __half>::value, "bf16 or fp16");
+  if constexpr (std::is_same<T, __half>::value) return pack_f16x2(lo, hi);
+  else return pack_bf16x2(lo, hi);
 }
 __device__ __forceinline__ void st_shared_v4(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(smem_u32(p)), "r"(a), "r"(b), "r"(c), "r"(d)
@@ -264,6 +279,14 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(const void* tile_1024_aligne
 //   [17,23) N>>3  [24,29) M>>4
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(uint32_t M, uint32_t N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+// The same with A=B=fp16: a_format = b_format = 0 (F16); nothing else of the instruction changes.
+__host__ __device__ constexpr uint32_t umma_idesc_f16(uint32_t M, uint32_t N) {
+  return (1u << 4) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+template <typename T>
+__host__ __device__ constexpr uint32_t umma_idesc(uint32_t M, uint32_t N) {
+  return std::is_same<T, __half>::value ? umma_idesc_f16(M, N) : umma_idesc_bf16(M, N);
 }
 
 // D[tmem] (+)= A[smem] * B[smem]^T ; issued by ONE thread

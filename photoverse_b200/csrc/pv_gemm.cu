@@ -38,7 +38,8 @@ struct GemmCfg {
   static constexpr uint32_t TMEM_COLS = BN <= 32 ? 32 : BN <= 64 ? 64 : BN <= 128 ? 128 : 256;
 };
 
-template <int BN, int STAGES_, bool OUT_F32, bool EPI_SWZ>
+// T: the 16-bit type of A, W and (OUT_F32 == false) D: __nv_bfloat16 or __half
+template <int BN, int STAGES_, bool OUT_F32, bool EPI_SWZ, typename T>
 __global__ void __launch_bounds__(GEMM_THREADS, (STAGES_ == 2 ? 2 : 1))
 gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                          const __grid_constant__ CUtensorMap tmD, const float* __restrict__ bias,
@@ -93,7 +94,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    constexpr uint32_t idesc = umma_idesc_bf16(GEMM_BM, BN);
+    constexpr uint32_t idesc = umma_idesc<T>(GEMM_BM, BN);
     for (int kb = 0; kb < kblocks; ++kb) {
       const int s = kb % Cfg::STAGES;
       const uint32_t ph = (kb / Cfg::STAGES) & 1;
@@ -156,9 +157,9 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
 #pragma unroll
         for (int ch = 0; ch < 4; ++ch) {
           const int pch = EPI_SWZ ? (ch ^ ((row >> 1) & 3)) : ch;
-          st_shared_v4(buf + row * 64 + pch * 16, pack_bf16x2(f[ch * 8 + 0], f[ch * 8 + 1]),
-                       pack_bf16x2(f[ch * 8 + 2], f[ch * 8 + 3]), pack_bf16x2(f[ch * 8 + 4], f[ch * 8 + 5]),
-                       pack_bf16x2(f[ch * 8 + 6], f[ch * 8 + 7]));
+          st_shared_v4(buf + row * 64 + pch * 16, pack_x2<T>(f[ch * 8 + 0], f[ch * 8 + 1]),
+                       pack_x2<T>(f[ch * 8 + 2], f[ch * 8 + 3]), pack_x2<T>(f[ch * 8 + 4], f[ch * 8 + 5]),
+                       pack_x2<T>(f[ch * 8 + 6], f[ch * 8 + 7]));
         }
       }
       fence_proxy_async_smem();
@@ -185,11 +186,11 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
 extern int g_opt_epi_swizzle;
 extern int g_opt_force_bn;
 
-template <int BN, int STAGES_, bool OUT_F32, bool EPI_SWZ>
+template <int BN, int STAGES_, bool OUT_F32, bool EPI_SWZ, typename T>
 static int launch_one(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorMap& tmD, const float* bias,
                       long long strideBias, int M, int N, int K, int batch, int w_batched, cudaStream_t stream) {
   using Cfg = GemmCfg<BN, STAGES_>;
-  auto kern = gemm_bf16_tcgen05_kernel<BN, STAGES_, OUT_F32, EPI_SWZ>;
+  auto kern = gemm_bf16_tcgen05_kernel<BN, STAGES_, OUT_F32, EPI_SWZ, T>;
   PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
   dim3 grid((N + BN - 1) / BN, (M + GEMM_BM - 1) / GEMM_BM, batch);
   kern<<<grid, GEMM_THREADS, Cfg::SMEM_BYTES, stream>>>(tmA, tmW, tmD, bias, strideBias, N, K, w_batched);
@@ -200,9 +201,9 @@ static int launch_one(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUte
 extern int g_opt_gemm_two_cta;
 extern int g_opt_gemm_persistent;
 int gemm3_bf16(const void* A, const void* W, const float* bias, void* D, long long M, long long N, long long K, long long lda,
-               long long ldw, long long ldd, cudaStream_t stream, bool w_static);
+               long long ldw, long long ldd, cudaStream_t stream, bool w_static, bool f16);
 
-template <int BN>
+template <int BN, typename T>
 static int launch_bn(bool out_f32, bool swz, const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorMap& tmD,
                      const float* bias, long long strideBias, int M, int N, int K, int batch, int w_batched,
                      cudaStream_t stream) {
@@ -210,12 +211,12 @@ static int launch_bn(bool out_f32, bool swz, const CUtensorMap& tmA, const CUten
   // deep-ring bf16-out kernel only (A/B switch `epi_swizzle`, validated identical on B200)
   const bool two = g_opt_gemm_two_cta != 0 && (K + GEMM_BK - 1) / GEMM_BK <= 8;
   if (two) {
-    return out_f32 ? launch_one<BN, 2, true, true>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream)
-                   : launch_one<BN, 2, false, true>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
+    return out_f32 ? launch_one<BN, 2, true, true, T>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream)
+                   : launch_one<BN, 2, false, true, T>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
   }
-  if (out_f32) return launch_one<BN, 0, true, true>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
-  return swz ? launch_one<BN, 0, false, true>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream)
-             : launch_one<BN, 0, false, false>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
+  if (out_f32) return launch_one<BN, 0, true, true, T>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
+  return swz ? launch_one<BN, 0, false, true, T>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream)
+             : launch_one<BN, 0, false, false, T>(tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
 }
 
 static int pick_bn(long long M, long long N, long long batch, bool two_cta) {
@@ -238,10 +239,10 @@ static int pick_bn(long long M, long long N, long long batch, bool two_cta) {
   return best;
 }
 
-// D[b] = A[b] W[b]^T + bias ; bf16 operands, bf16 or fp32 output.
+// D[b] = A[b] W[b]^T + bias ; bf16 (f16: fp16) operands, output of the operand type or fp32.
 int gemm_bf16(const void* A, const void* W, const float* bias, void* D, bool out_f32, long long M, long long N,
               long long K, long long batch, long long lda, long long ldw, long long ldd, long long strideA,
-              long long strideW, long long strideBias, long long strideD, cudaStream_t stream, bool w_static) {
+              long long strideW, long long strideBias, long long strideD, cudaStream_t stream, bool w_static, bool f16) {
   PV_REQUIRE(M > 0 && N > 0 && K > 0 && batch > 0, "empty problem M=%lld N=%lld K=%lld batch=%lld", M, N, K, batch);
   PV_REQUIRE(K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0, "bf16 rows must be 16-byte multiples (K=%lld lda=%lld ldw=%lld)",
              K, lda, ldw);
@@ -253,27 +254,31 @@ int gemm_bf16(const void* A, const void* W, const float* bias, void* D, bool out
   PV_REQUIRE(batch <= 65535 && (M + GEMM_BM - 1) / GEMM_BM <= 65535, "grid too large");
   // persistent CTA-pair kernel (pv_gemm3.cu): the out projection shapes (bf16 out, N % 160 == 0, K % 64 == 0, tall M)
   if (g_opt_gemm_persistent != 0 && g_opt_force_bn == 0 && !out_f32 && batch == 1 && M >= 512 && N % 160 == 0 && K % 64 == 0)
-    return gemm3_bf16(A, W, bias, D, M, N, K, lda, ldw, ldd, stream, w_static);
+    return gemm3_bf16(A, W, bias, D, M, N, K, lda, ldw, ldd, stream, w_static, f16);
   const bool two_cta = g_opt_gemm_two_cta != 0 && (K + GEMM_BK - 1) / GEMM_BK <= 8;
   const int bn = pick_bn(M, N, batch, two_cta);
   const bool swz = g_opt_epi_swizzle != 0 || out_f32 || two_cta;
   const int w_batched = strideW != 0;
   CUtensorMap tmA, tmW, tmD;
   // batch stride 0 is not encodable: give un-batched operands a dummy stride with extent 1
-  if (make_tmap_3d(&tmA, A, 2, K, M, batch, lda * 2, (batch > 1 ? strideA : lda * M) * 2, GEMM_BK, GEMM_BM, 1, Swz::B128))
+  if (make_tmap_3d(&tmA, A, 2, K, M, batch, lda * 2, (batch > 1 ? strideA : lda * M) * 2, GEMM_BK, GEMM_BM, 1, Swz::B128, f16))
     return PV_ERR_CUDA;
   if (make_tmap_3d(&tmW, W, 2, K, N, w_batched ? batch : 1, ldw * 2, (w_batched ? strideW : ldw * N) * 2, GEMM_BK, bn, 1,
-                   Swz::B128))
+                   Swz::B128, f16))
     return PV_ERR_CUDA;
   if (make_tmap_3d(&tmD, D, oe, N, M, batch, ldd * oe, (batch > 1 ? strideD : ldd * M) * oe, 32, 32, 1,
-                   swz ? (out_f32 ? Swz::B128 : Swz::B64) : Swz::None))
+                   swz ? (out_f32 ? Swz::B128 : Swz::B64) : Swz::None, f16))
     return PV_ERR_CUDA;
+#define PV_GEMM_BN(BN)                                                                                         \
+  (f16 ? launch_bn<BN, __half>(out_f32, swz, tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream)        \
+       : launch_bn<BN, __nv_bfloat16>(out_f32, swz, tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream))
   switch (bn) {
-    case 256: return launch_bn<256>(out_f32, swz, tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
-    case 160: return launch_bn<160>(out_f32, swz, tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
-    case 128: return launch_bn<128>(out_f32, swz, tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
-    default:  return launch_bn<64>(out_f32, swz, tmA, tmW, tmD, bias, strideBias, M, N, K, batch, w_batched, stream);
+    case 256: return PV_GEMM_BN(256);
+    case 160: return PV_GEMM_BN(160);
+    case 128: return PV_GEMM_BN(128);
+    default:  return PV_GEMM_BN(64);
   }
+#undef PV_GEMM_BN
 }
 
 }  // namespace pv

@@ -8,7 +8,7 @@
 //     only A is streamed (16 KB per K-block per CTA) through a deep TMA ring;  K = 1280 streams 10 KB W halves as well
 //   * ONE tcgen05.mma stream of M = 256 issued by the leader into double-buffered TMEM accumulators (2 x 160 columns):
 //     the MMAs of tile i+1 run under the epilogue of tile i
-//   * epilogue warps (2 x 4 per CTA): TMEM -> +bias -> bf16 -> per-warp staging tile -> TMA store
+//   * epilogue warps (2 x 4 per CTA): TMEM -> +bias -> bf16 (fp16 for fp16 operands) -> per-warp staging tile -> TMA store
 // The single-CTA kernel of pv_gemm.cu spends most of a K = 320 tile in its prologue / epilogue (5 K-blocks) and is bound
 // by TMA ingest (36 KB per K-block); this one has neither problem.
 //
@@ -27,7 +27,7 @@ constexpr int G3_THREADS = 384;          // warp 0 TMA, warp 1 MMA (leader), war
 // processor kernels -- here without row-block counters (every A tile is ready when the kernel starts).
 // EPI = OP_EPI_GEGLU: D[M, N / 2] = GEGLU of the packed projection (see pv_outproj.cuh); a pair's tiles are the contiguous
 // share [T p / npairs, T (p + 1) / npairs) of the T = G V (group, unit) entries instead of the units of one group.
-template <typename Cfg, int EPI>
+template <typename Cfg, int EPI, typename T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G3_THREADS, 1)
 gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                              const __grid_constant__ CUtensorMap tmD, const float* __restrict__ bias, int G, int V, int K,
@@ -90,7 +90,7 @@ gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gr
   oa.ready_target = 0;
   oa.w_preloaded = Cfg::WSTAT && w_static && u0 < u1;
   oa.trace = nullptr; oa.trace_cap = 0; oa.trace_block = 0;
-  outproj_phase<Cfg, EPI>(smem, bars, tmem, &tmA, &tmW, &tmD, oa);
+  outproj_phase<Cfg, EPI, T>(smem, bars, tmem, &tmA, &tmW, &tmD, oa);
 
   tc_fence_before();
   __syncthreads();
@@ -99,13 +99,13 @@ gemm3_pair_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gr
   if (warp == 2) tmem_dealloc_2sm<512>(tmem);
 }
 
-template <int KB_RES, int STAGES, int EPI = OP_EPI_BIAS>
+template <int KB_RES, int STAGES, int EPI, typename T>
 static int launch_g3(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUtensorMap& tmD, const float* bias, int G, int V,
                      int K, int w_static, cudaStream_t stream) {
   using Cfg = OutProjCfg<KB_RES, STAGES>;
   constexpr int SMEM_BYTES = (Cfg::BYTES + 15) / 16 * 16 + 256 + 1024;
   static_assert(OP_BAR_BYTES + 8 + 8 <= 256 && SMEM_BYTES <= 227 * 1024, "shared memory budget");
-  auto kern = gemm3_pair_persistent_kernel<Cfg, EPI>;
+  auto kern = gemm3_pair_persistent_kernel<Cfg, EPI, T>;
   PV_CUDA(set_max_smem_once(kern, SMEM_BYTES));
   const long long units = static_cast<long long>(G) * V;
   const long long max_pairs = sm_count() / 2;
@@ -115,21 +115,25 @@ static int launch_g3(const CUtensorMap& tmA, const CUtensorMap& tmW, const CUten
   return PV_OK;
 }
 
-// D[M,N] (bf16, row stride ldd) = A[M,K] (lda) * W[N,K]^T (ldw) + bias ; N % 160 == 0, K % 64 == 0
+// D[M,N] (bf16 or, with f16, fp16; row stride ldd) = A[M,K] (lda) * W[N,K]^T (ldw) + bias ; N % 160 == 0, K % 64 == 0
 int gemm3_bf16(const void* A, const void* W, const float* bias, void* D, long long M, long long N, long long K, long long lda,
-               long long ldw, long long ldd, cudaStream_t stream, bool w_static) {
+               long long ldw, long long ldd, cudaStream_t stream, bool w_static, bool f16) {
   PV_REQUIRE(M > 0 && N % OP_BN == 0 && K % OP_BK == 0 && N > 0 && K > 0, "gemm3: need N %% 160 == 0 and K %% 64 == 0 (N=%lld K=%lld)", N, K);
   PV_REQUIRE((lda * 2) % 16 == 0 && (ldw * 2) % 16 == 0 && (ldd * 2) % 16 == 0, "row strides must be 16-byte multiples");
   CUtensorMap tmA, tmW, tmD;
-  if (make_tmap_3d(&tmA, A, 2, K, M, 1, lda * 2, lda * M * 2, OP_BK, 128, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmW, W, 2, K, N, 1, ldw * 2, ldw * N * 2, OP_BK, OP_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
-  if (make_tmap_3d(&tmD, D, 2, N, M, 1, ldd * 2, ldd * M * 2, 80, 32, 1, Swz::None)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmA, A, 2, K, M, 1, lda * 2, lda * M * 2, OP_BK, 128, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmW, W, 2, K, N, 1, ldw * 2, ldw * N * 2, OP_BK, OP_BN / 2, 1, Swz::B128, f16)) return PV_ERR_CUDA;
+  if (make_tmap_3d(&tmD, D, 2, N, M, 1, ldd * 2, ldd * M * 2, 80, 32, 1, Swz::None, f16)) return PV_ERR_CUDA;
   const int G = static_cast<int>(N / OP_BN);
   const long long V = (M + 255) / 256;
   PV_REQUIRE(V * G < (1ll << 30), "too many tiles");
-  if (K == 320) return launch_g3<5, 8>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream);
-  if (K == 640) return launch_g3<10, 5>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream);
-  return launch_g3<0, 7>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream);
+#define PV_G3(KB, ST)                                                                                                    \
+  (f16 ? launch_g3<KB, ST, OP_EPI_BIAS, __half>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream) \
+       : launch_g3<KB, ST, OP_EPI_BIAS, __nv_bfloat16>(tmA, tmW, tmD, bias, G, static_cast<int>(V), static_cast<int>(K), w_static, stream))
+  if (K == 320) return PV_G3(5, 8);
+  if (K == 640) return PV_G3(10, 5);
+  return PV_G3(0, 7);
+#undef PV_G3
 }
 
 // y[M, N] (bf16, row stride ldy) = GEGLU of x[M, K] (ldx) * Wp[2N, K]^T + bp, with Wp / bp packed per 80 output columns
@@ -150,9 +154,9 @@ int linear_geglu_bf16(const void* x, const void* Wp, const float* bp, void* y, l
   if (make_tmap_3d(&tmW, Wp, 2, K, 2 * N, 1, K * 2, K * 2 * N * 2, OP_BK, OP_BN / 2, 1, Swz::B128)) return PV_ERR_CUDA;
   if (make_tmap_3d(&tmD, y, 2, N, M, 1, ldy * 2, ldy * M * 2, 40, 32, 1, Swz::None)) return PV_ERR_CUDA;
   // the packed weight is a cached copy of a parameter, never written by the kernel this launch may overlap (w_static)
-  if (K == 320) return launch_g3<5, 8, OP_EPI_GEGLU>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
-  if (K == 640) return launch_g3<10, 5, OP_EPI_GEGLU>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
-  return launch_g3<0, 7, OP_EPI_GEGLU>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
+  if (K == 320) return launch_g3<5, 8, OP_EPI_GEGLU, __nv_bfloat16>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
+  if (K == 640) return launch_g3<10, 5, OP_EPI_GEGLU, __nv_bfloat16>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
+  return launch_g3<0, 7, OP_EPI_GEGLU, __nv_bfloat16>(tmA, tmW, tmD, bp, static_cast<int>(G), static_cast<int>(V), static_cast<int>(K), 1, stream);
 }
 
 }  // namespace pv

@@ -50,9 +50,11 @@ enum class Swz { None, B64, B128 };
 //   strides = {stride of d1, stride of d2}                   in BYTES (multiples of 16)
 //   box     = {b0, b1, b2}                                   in elements (b0*elem_bytes <= swizzle span)
 // Out-of-bounds box elements read as zero and are skipped on store.
+// 2-byte elements are bf16, or fp16 with f16 = true.
 // Returns 0 on success; on failure sets the error string.
 int make_tmap_3d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t d0, uint64_t d1, uint64_t d2,
-                 uint64_t stride1_bytes, uint64_t stride2_bytes, uint32_t b0, uint32_t b1, uint32_t b2, Swz swz);
+                 uint64_t stride1_bytes, uint64_t stride2_bytes, uint32_t b0, uint32_t b1, uint32_t b2, Swz swz,
+                 bool f16 = false);
 
 int sm_count();                       // SM count of the CURRENT device (cached per device)
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-device function attribute: set once per (kernel, device)

@@ -203,11 +203,13 @@ __device__ __forceinline__ void op_geglu_epilogue(uint8_t* smem_ost, float* sbia
 // at `pb` were initialised by op_mbar_init at kernel start and never used).  Roles: warp 0 producer (both CTAs),
 // warp 1 MMA issuer (leader), warps 4..11 epilogue (both CTAs); other warps return at once.
 // OP_EPI_GEGLU (plain GEMM only, a.sync == nullptr) also needs the w_free barrier at pb[OP_W_FREE], initialised with count 1.
-template <typename Cfg, int EPI = OP_EPI_BIAS>
+// T: the 16-bit type of A, W and D (__nv_bfloat16 or __half; the GEGLU epilogue is bf16 only).
+template <typename Cfg, int EPI = OP_EPI_BIAS, typename T = __nv_bfloat16>
 __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint32_t tmem, const CUtensorMap* tmA,
                                               const CUtensorMap* tmW, const CUtensorMap* tmD, const OutProjArgs& a) {
   constexpr bool WSTAT = Cfg::WSTAT;
   constexpr bool GEGLU = EPI == OP_EPI_GEGLU;
+  static_assert(!GEGLU || std::is_same<T, __nv_bfloat16>::value, "the GEGLU epilogue rounds like the bf16 geglu_kernel");
   constexpr int nst = Cfg::STAGES;
   uint64_t* full = pb;
   uint64_t* empty = full + OP_MAX_STAGES;
@@ -343,7 +345,7 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
   } else if (warp == 1) {
     if (rank == 0) {
       // ===================== MMA issuer (leader): M = 256, N = 160 for both CTAs =====================
-      constexpr uint32_t idesc = umma_idesc_bf16(256, OP_BN);
+      constexpr uint32_t idesc = umma_idesc<T>(256, OP_BN);
       A3Trace tr = a3_trace_init_raw(a.trace, a.trace_cap, 5, a.trace_block);
       uint32_t it = 0;
       int i = 0;
@@ -423,17 +425,17 @@ __device__ __forceinline__ void outproj_phase(uint8_t* smem, uint64_t* pb, uint3
       if (elect_one()) bulk_wait_read<0>();              // previous TMA store of this warp has read the staging tile
       __syncwarp();
       a3_trace(tr, 74, i);
-      // + bias -> bf16 pairs, in place (word 4c + k = columns 8c + 2k, 8c + 2k + 1).  The tensor core's operand reads and
+      // + bias -> 16-bit pairs, in place (word 4c + k = columns 8c + 2k, 8c + 2k + 1).  The tensor core's operand reads and
       // the TMA writes leave little shared-memory bandwidth: the bias comes in 16-byte (broadcast) loads ...
 #pragma unroll
       for (int c = 0; c < 10; ++c) {
         float4 b0, b1;
         asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(b0.x), "=f"(b0.y), "=f"(b0.z), "=f"(b0.w) : "r"(bias_a + c * 32));
         asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(b1.x), "=f"(b1.y), "=f"(b1.z), "=f"(b1.w) : "r"(bias_a + c * 32 + 16));
-        v[4 * c + 0] = pack_bf16x2(__uint_as_float(v[8 * c + 0]) + b0.x, __uint_as_float(v[8 * c + 1]) + b0.y);
-        v[4 * c + 1] = pack_bf16x2(__uint_as_float(v[8 * c + 2]) + b0.z, __uint_as_float(v[8 * c + 3]) + b0.w);
-        v[4 * c + 2] = pack_bf16x2(__uint_as_float(v[8 * c + 4]) + b1.x, __uint_as_float(v[8 * c + 5]) + b1.y);
-        v[4 * c + 3] = pack_bf16x2(__uint_as_float(v[8 * c + 6]) + b1.z, __uint_as_float(v[8 * c + 7]) + b1.w);
+        v[4 * c + 0] = pack_x2<T>(__uint_as_float(v[8 * c + 0]) + b0.x, __uint_as_float(v[8 * c + 1]) + b0.y);
+        v[4 * c + 1] = pack_x2<T>(__uint_as_float(v[8 * c + 2]) + b0.z, __uint_as_float(v[8 * c + 3]) + b0.w);
+        v[4 * c + 2] = pack_x2<T>(__uint_as_float(v[8 * c + 4]) + b1.x, __uint_as_float(v[8 * c + 5]) + b1.y);
+        v[4 * c + 3] = pack_x2<T>(__uint_as_float(v[8 * c + 6]) + b1.z, __uint_as_float(v[8 * c + 7]) + b1.w);
       }
       // ... and the 16-byte staging stores of a quarter warp must not collide: rows are 160 bytes apart (8 l mod 32
       // banks), so lanes 4..7 of every quarter write the NEXT 16-byte chunk of their row in the same instruction

@@ -1,7 +1,7 @@
 // photoverse_b200 -- layout / packing kernels (HBM-bound, vectorised, coalesced).
 //
-//  * pack_weight      : W_eff = W + scaling * B A  (peft lora.Linear merged form) -> bf16 / fp32
-//  * kv_pack_bf16     : fp32 K/V projections -> per-(sample, head) UMMA operand images consumed by the fused
+//  * pack_weight      : W_eff = W + scaling * B A  (peft lora.Linear merged form) -> bf16 / fp16 / fp32
+//  * kv_pack_bf16     : fp32 K/V projections -> per-(sample, head) bf16 / fp16 UMMA operand images consumed by the fused
 //                       attention kernel via 1-D TMA bulk copies, + the `to_v_ip_norm` side output
 //                       (attention_processor.py:395-397)
 //  * kv_pack_f32      : same gather for the fp32 parity path ([B,H,L,d] fp32)
@@ -11,7 +11,8 @@
 
 namespace pv {
 
-template <bool OUT_BF16>
+// OUT16: 16-bit output of type T16 (__nv_bfloat16 or __half), else fp32
+template <bool OUT16, typename T16>
 __global__ void __launch_bounds__(256)
 pack_weight_kernel(const float* __restrict__ W, const float* __restrict__ A, const float* __restrict__ Bm,
                    float scaling, void* __restrict__ out, int out_f, int in_f, int r) {
@@ -32,15 +33,15 @@ pack_weight_kernel(const float* __restrict__ W, const float* __restrict__ A, con
     w.x = fmaf(scaling, dx, w.x); w.y = fmaf(scaling, dy, w.y);
     w.z = fmaf(scaling, dz, w.z); w.w = fmaf(scaling, dw, w.w);
   }
-  if constexpr (OUT_BF16) {
-    uint2 pk = make_uint2(pack_bf16x2(w.x, w.y), pack_bf16x2(w.z, w.w));
-    *reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(out) + idx) = pk;
+  if constexpr (OUT16) {
+    uint2 pk = make_uint2(pack_x2<T16>(w.x, w.y), pack_x2<T16>(w.z, w.w));
+    *reinterpret_cast<uint2*>(static_cast<T16*>(out) + idx) = pk;
   } else {
     *reinterpret_cast<float4*>(static_cast<float*>(out) + idx) = w;
   }
 }
 
-int pack_weight(bool out_bf16, const float* W, const float* A, const float* Bm, float scaling, void* out, int out_f,
+int pack_weight(pv_dtype out_dt, const float* W, const float* A, const float* Bm, float scaling, void* out, int out_f,
                 int in_f, int r, cudaStream_t stream) {
   PV_REQUIRE(out_f > 0 && in_f > 0 && in_f % 4 == 0 && r >= 0, "bad shape out=%d in=%d r=%d", out_f, in_f, r);
   PV_REQUIRE(r == 0 || (A != nullptr && Bm != nullptr), "LoRA rank %d without A/B", r);
@@ -48,8 +49,9 @@ int pack_weight(bool out_bf16, const float* W, const float* A, const float* Bm, 
              "pointers must be 16-byte aligned");
   const long long total4 = static_cast<long long>(out_f) * in_f / 4;
   const int blocks = static_cast<int>((total4 + 255) / 256);
-  if (out_bf16) pack_weight_kernel<true><<<blocks, 256, 0, stream>>>(W, A, Bm, scaling, out, out_f, in_f, r);
-  else pack_weight_kernel<false><<<blocks, 256, 0, stream>>>(W, A, Bm, scaling, out, out_f, in_f, r);
+  if (out_dt == PV_BF16) pack_weight_kernel<true, __nv_bfloat16><<<blocks, 256, 0, stream>>>(W, A, Bm, scaling, out, out_f, in_f, r);
+  else if (out_dt == PV_F16) pack_weight_kernel<true, __half><<<blocks, 256, 0, stream>>>(W, A, Bm, scaling, out, out_f, in_f, r);
+  else pack_weight_kernel<false, __nv_bfloat16><<<blocks, 256, 0, stream>>>(W, A, Bm, scaling, out, out_f, in_f, r);
   PV_LAUNCHED();
   return PV_OK;
 }
@@ -67,6 +69,7 @@ __device__ __forceinline__ float kv_fetch(const float* __restrict__ kv_text, con
   return 0.f;
 }
 
+template <typename T>   // __nv_bfloat16 or __half tiles
 __global__ void __launch_bounds__(256)
 kv_pack_bf16_kernel(const float* __restrict__ kv_text, const float* __restrict__ kv_img, uint8_t* __restrict__ Kp,
                     uint8_t* __restrict__ Vp, float* __restrict__ v_ip_norm, int Lt, int Li, int C, int H, int d,
@@ -87,7 +90,7 @@ kv_pack_bf16_kernel(const float* __restrict__ kv_text, const float* __restrict__
       v[i] = (dim < d) ? kv_fetch(kv_text, kv_img, b, key, h * d + dim, Lt, Li, C2, PV_IMG_KEY_OFFSET) : 0.f;
     }
     *reinterpret_cast<uint4*>(kt + static_cast<size_t>(idx) * 16) =
-        make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+        make_uint4(pack_x2<T>(v[0], v[1]), pack_x2<T>(v[2], v[3]), pack_x2<T>(v[4], v[5]), pack_x2<T>(v[6], v[7]));
   }
   // V^T tile: 12 * d_pad chunks
   for (int idx = threadIdx.x; idx < (PV_KEYS_PAD / 8) * d_pad; idx += blockDim.x) {
@@ -99,7 +102,7 @@ kv_pack_bf16_kernel(const float* __restrict__ kv_text, const float* __restrict__
       v[i] = (dim < d) ? kv_fetch(kv_text, kv_img, b, key, C + h * d + dim, Lt, Li, C2, PV_IMG_KEY_OFFSET) : 0.f;
     }
     *reinterpret_cast<uint4*>(vt + static_cast<size_t>(idx) * 16) =
-        make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+        make_uint4(pack_x2<T>(v[0], v[1]), pack_x2<T>(v[2], v[3]), pack_x2<T>(v[4], v[5]), pack_x2<T>(v[6], v[7]));
   }
   // ||V_img||_2 over head_dim, from the fp32 projections
   for (int li = threadIdx.x; li < Li; li += blockDim.x) {
@@ -130,15 +133,16 @@ kv_pack_f32_kernel(const float* __restrict__ kv_text, const float* __restrict__ 
   }
 }
 
-int kv_pack(bool bf16, const float* kv_text, const float* kv_img, void* Kp, void* Vp, float* v_ip_norm, int B, int Lt,
+int kv_pack(pv_dtype dt, const float* kv_text, const float* kv_img, void* Kp, void* Vp, float* v_ip_norm, int B, int Lt,
             int Li, int C, int H, cudaStream_t stream) {
   const int d = C / H;
   PV_REQUIRE(B <= 65535, "grid too large");
   dim3 grid(H, B);
-  if (bf16) {
+  if (dt != PV_F32) {
     const int d_pad = (d + 15) / 16 * 16;
-    kv_pack_bf16_kernel<<<grid, 256, 0, stream>>>(kv_text, kv_img, static_cast<uint8_t*>(Kp),
-                                                  static_cast<uint8_t*>(Vp), v_ip_norm, Lt, Li, C, H, d, d_pad);
+    auto kern = dt == PV_F16 ? kv_pack_bf16_kernel<__half> : kv_pack_bf16_kernel<__nv_bfloat16>;
+    kern<<<grid, 256, 0, stream>>>(kv_text, kv_img, static_cast<uint8_t*>(Kp), static_cast<uint8_t*>(Vp), v_ip_norm, Lt, Li,
+                                   C, H, d, d_pad);
   } else {
     kv_pack_f32_kernel<<<grid, 256, 0, stream>>>(kv_text, kv_img, static_cast<float*>(Kp), static_cast<float*>(Vp),
                                                  v_ip_norm, Lt, Li, C, H, d);

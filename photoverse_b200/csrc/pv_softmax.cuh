@@ -4,10 +4,10 @@
 
 namespace pv {
 
-template <int N>
+template <int N, typename T = __nv_bfloat16>
 __device__ __forceinline__ void pack_pairs3(const uint32_t* v, uint32_t* out) {
 #pragma unroll
-  for (int i = 0; i < N / 2; ++i) out[i] = pack_bf16x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1]));
+  for (int i = 0; i < N / 2; ++i) out[i] = pack_x2<T>(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1]));
 }
 
 // A drained-later O accumulator of one softmax group (the PV MMA runs while the group computes its next softmax).

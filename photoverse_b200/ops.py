@@ -9,19 +9,24 @@ from typing import Optional
 import torch
 
 from . import _lib
-from ._lib import PV_BF16, PV_F32, PV_KEYS_PAD, check
+from ._lib import PV_BF16, PV_F16, PV_F32, PV_KEYS_PAD, check
 
 
-def _dt(t: torch.Tensor) -> int:
-    if t.dtype == torch.bfloat16:
-        return PV_BF16
-    if t.dtype == torch.float32:
-        return PV_F32
-    raise _lib.PhotoverseB200Error(f"unsupported dtype {t.dtype}: photoverse_b200 computes in bfloat16 or float32")
+_CODES = {torch.bfloat16: PV_BF16, torch.float32: PV_F32, torch.float16: PV_F16}
+# the 16-bit compute dtypes: tensor-core kernels, fused Q projection, K/V operand tiles, single-launch processor
+HALF_DTYPES = (torch.bfloat16, torch.float16)
 
 
 def _code(dtype: torch.dtype) -> int:
-    return PV_BF16 if dtype == torch.bfloat16 else PV_F32
+    code = _CODES.get(dtype)
+    if code is None:
+        raise _lib.PhotoverseB200Error(f"unsupported dtype {dtype}: photoverse_b200 computes in bfloat16, float16 "
+                                       "(inference only) or float32")
+    return code
+
+
+def _dt(t: torch.Tensor) -> int:
+    return _code(t.dtype)
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -44,7 +49,7 @@ def _f32(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
 
 
 def pack_weight(w: torch.Tensor, out: torch.Tensor, lora_A=None, lora_B=None, scaling: float = 0.0) -> torch.Tensor:
-    """out[out_f, in_f] (bf16|f32) = w + scaling * lora_B @ lora_A  (fp32 masters)."""
+    """out[out_f, in_f] (bf16|f16|f32) = w + scaling * lora_B @ lora_A  (fp32 masters)."""
     out_f, in_f = w.shape
     assert out.shape == w.shape and out.is_contiguous() and w.is_contiguous() and w.dtype == torch.float32
     r = 0
@@ -157,7 +162,7 @@ def dual_attn(x: torch.Tensor, wq: torch.Tensor, kv: PackedKV, wo: torch.Tensor,
     """Y = (w_t softmax(QK_t^T/sqrt d) V_t + w_i softmax(QK_i^T/sqrt d) V_i) Wo^T + bo with Q = x Wq^T.
     Returns (Y, O, stats|None, Q|None); O (pre-out-projection) and Q (fp32 mode only) are kept for backward."""
     B, S, C = x.shape
-    sync = _sync_words(B, S, x.device) if x.dtype == torch.bfloat16 else None
+    sync = _sync_words(B, S, x.device) if x.dtype in HALF_DTYPES else None
     assert x.is_contiguous() and wq.is_contiguous() and wo.is_contiguous()
     assert x.dtype == wq.dtype == wo.dtype == kv.dtype and bo.dtype == torch.float32
     assert (kv.B, kv.C) == (B, C)
@@ -173,12 +178,12 @@ def dual_attn(x: torch.Tensor, wq: torch.Tensor, kv: PackedKV, wo: torch.Tensor,
 
 def dual_attn_core(x_or_q: torch.Tensor, wq: Optional[torch.Tensor], kv: PackedKV, w_text: float = 1.0,
                    w_img: float = 1.0, want_stats: bool = False):
-    """The attention kernel alone (no out projection).  bf16: ``x_or_q`` = X and ``wq`` is applied inside the kernel;
-    fp32: ``x_or_q`` = Q (already projected), ``wq`` ignored.  Returns (O [B,S,C], stats|None)."""
+    """The attention kernel alone (no out projection).  bf16 / fp16: ``x_or_q`` = X and ``wq`` is applied inside the
+    kernel; fp32: ``x_or_q`` = Q (already projected), ``wq`` ignored.  Returns (O [B,S,C], stats|None)."""
     B, S, C = x_or_q.shape
     assert x_or_q.is_contiguous() and x_or_q.dtype == kv.dtype and (kv.B, kv.C) == (B, C)
-    if x_or_q.dtype == torch.bfloat16:
-        assert wq is not None and wq.is_contiguous() and wq.dtype == torch.bfloat16 and wq.shape == (C, C)
+    if x_or_q.dtype in HALF_DTYPES:
+        assert wq is not None and wq.is_contiguous() and wq.dtype == x_or_q.dtype and wq.shape == (C, C)
     o = torch.empty_like(x_or_q)
     stats = torch.empty(B, kv.H, S, 4, device=o.device, dtype=torch.float32) if want_stats else None
     check(_lib.lib().pv_dual_attn_core_fwd(_dt(x_or_q), _ptr(x_or_q), _ptr(wq), _ptr(kv.Kp), _ptr(kv.Vp), _ptr(o),
@@ -189,7 +194,7 @@ def dual_attn_core(x_or_q: torch.Tensor, wq: Optional[torch.Tensor], kv: PackedK
 
 def ln_lrelu(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, out: torch.Tensor,
              rows_per_group: int = 0, eps: float = 1e-5, slope: float = 0.01, save_stats: bool = False):
-    """out = leaky_relu(layer_norm(x) * gamma + beta); x fp32 [rows, cols] (row-strided ok), out bf16|fp32."""
+    """out = leaky_relu(layer_norm(x) * gamma + beta); x fp32 [rows, cols] (row-strided ok), out bf16|f16|fp32."""
     rows, cols = x.shape
     assert x.dtype == torch.float32 and x.stride(1) == 1 and out.stride(1) == 1 and out.shape == x.shape
     assert gamma.dtype == beta.dtype == torch.float32 and gamma.is_contiguous() and beta.is_contiguous()

@@ -1,4 +1,4 @@
-"""Per-kernel SASS instruction mix of libphotoverse_b200.so -> profiles/r02_sass_summary.txt (no GPU needed).
+"""Per-kernel SASS instruction mix of libphotoverse_b200.so -> profiles/<argv[1]> (no GPU needed).
 Counts the mnemonics that prove the Blackwell path (B200_PROFILING.md): UTCHMMA (tcgen05.mma), UTCBAR (tcgen05.commit),
 LDTM / STTM (tcgen05.ld / st), UTMALDG / UTMASTG (TMA tensor load / store), UBLKCP (bulk copy), SYNCS (mbarrier),
 and the legacy tensor path HMMA / LDSM (mma.sync / ldmatrix), plus the packed fp32x2 arithmetic FFMA2 / FADD2 / FMUL2."""
@@ -35,15 +35,15 @@ names = subprocess.run(["c++filt"], input="\n".join(counts), capture_output=True
 rows = []
 for mangled, dem in zip(counts, names):
     c = counts[mangled]
-    short = re.sub(r"\(.*", "", dem.replace("void ", "").replace("pv::", ""))[:64]
+    short = re.sub(r"\(.*", "", dem.replace("void ", "").replace("pv::", ""))[:80]
     rows.append((short, c))
 rows.sort(key=lambda r: (-r[1]["UTCHMMA"], -r[1]["HMMA"], r[0]))
 with open(OUT, "w") as f:
     f.write("SASS instruction mix per kernel of photoverse_b200/libphotoverse_b200.so (cuobjdump -sass, sm_100a; tools/sass_summary.py)\n")
-    f.write(f"{'kernel':66s}" + "".join(f"{k:>9s}" for k in MNEM) + f"{'instrs':>9s}\n")
+    f.write(f"{'kernel':82s}" + "".join(f"{k:>9s}" for k in MNEM) + f"{'instrs':>9s}\n")
     tot = collections.Counter()
     for short, c in rows:
-        f.write(f"{short:66s}" + "".join(f"{c[k]:9d}" for k in MNEM) + f"{c['_total']:9d}\n")
+        f.write(f"{short:82s}" + "".join(f"{c[k]:9d}" for k in MNEM) + f"{c['_total']:9d}\n")
         tot.update(c)
-    f.write(f"{'TOTAL (' + str(len(rows)) + ' kernels)':66s}" + "".join(f"{tot[k]:9d}" for k in MNEM) + f"{tot['_total']:9d}\n")
+    f.write(f"{'TOTAL (' + str(len(rows)) + ' kernels)':82s}" + "".join(f"{tot[k]:9d}" for k in MNEM) + f"{tot['_total']:9d}\n")
 print(open(OUT).read()[:6000])

@@ -287,6 +287,13 @@ int pv_geglu_bwd(pv_dtype dt, const void* h, const void* dy, void* dh, int64_t M
 int pv_linear_geglu_fwd(pv_dtype dt, const void* x, const void* w_packed, const float* b_packed, void* y, int64_t M, int64_t N,
                         int64_t K, int64_t ldx, int64_t ldy, void* stream);
 
+/* ---- activation dtype conversion (torch.autocast over a float32 model, DESIGN.md 4.9) -------------------------------
+ * dst[i] = src[i] converted from in_dt to out_dt, n elements, both dense.  Pairs: PV_F32 -> PV_BF16, PV_F32 -> PV_F16,
+ * PV_BF16 -> PV_F32, PV_F16 -> PV_F32; any other pair returns PV_ERR_UNSUPPORTED.  Round to nearest even: bit-identical to
+ * torch.Tensor.to for every finite input; fp16 overflow gives +-inf; NaN stays NaN (payload not preserved).  Pointers need
+ * only element alignment (vector accesses start at the first common 32-byte / 16-byte boundary).  n == 0 launches nothing. */
+int pv_convert_fwd(pv_dtype in_dt, pv_dtype out_dt, const void* src, void* dst, int64_t n, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -70,6 +70,7 @@ _SIGNATURES = {
     "pv_geglu_fwd": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p]),
     "pv_geglu_bwd": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int64, c_void_p]),
     "pv_linear_geglu_fwd": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p] + [c_int64] * 5 + [c_void_p]),
+    "pv_convert_fwd": (c_int, [c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
 }
 
 # every declared symbol must be exported by the build

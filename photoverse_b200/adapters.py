@@ -6,7 +6,8 @@ so reference checkpoints load with ``load_state_dict`` unchanged (models/modelin
 
 Execution plan per call (all T selected token heads in the same launches, batched over heads):
     patches [T, B*256, 1024] --GEMM+bias--> fp32 --LN+LeakyReLU--> bf16 --GEMM+bias--> fp32 --LN+LeakyReLU--> bf16
-            (float16 embeddings, inference only: fp16 wherever this plan says bf16)
+            (float16 embeddings, inference only: fp16 wherever this plan says bf16; float32 embeddings under CUDA
+             autocast: converted to the autocast dtype first, DESIGN.md 4.9)
             --mean over the 256 patches-->  cat[:, :, 1024:2048]
     cls     [T, B,     1024] --same two layers-->                            cat[:, :,    0:1024]
     out[b, t, :] = cat[t, b, :] @ [W3_cls | W3_patch]^T + (b3_cls + b3_patch)            (one K=2048 GEMM)
@@ -121,9 +122,15 @@ class PhotoVerseAdapter(nn.Module):
             raise RuntimeError("photoverse_b200 runs on CUDA only (no CPU fallback)")
         if e0.dtype not in (torch.bfloat16, torch.float16, torch.float32):
             raise TypeError(f"embeddings must be bfloat16, float16 or float32, got {e0.dtype}")
-        if torch.is_grad_enabled() and (any(p.requires_grad for p in self.parameters())
-                                        or any(e.requires_grad for e in embs_sel)):
-            if e0.dtype == torch.float16:
+        train = torch.is_grad_enabled() and (any(p.requires_grad for p in self.parameters())
+                                             or any(e.requires_grad for e in embs_sel))
+        # under CUDA autocast float32 embeddings compute in the autocast dtype (DESIGN.md 4.9): converted once per call
+        dtype = ops.compute_dtype(e0.dtype, train)
+        if dtype != e0.dtype:
+            from .autograd import convert       # keeps requires_grad visible to adapter_autograd's check
+            embs_sel = [e if e.dtype == dtype else (convert if e.requires_grad else ops.convert)(e, dtype) for e in embs_sel]
+        if train:
+            if dtype == torch.float16:
                 raise NotImplementedError("float16 runs the inference (no_grad) path only: training runs in bfloat16 "
                                           "or float32")
             from .autograd import adapter_autograd

@@ -11,6 +11,8 @@ Differences in *how* (not what) it computes, see DESIGN.md:
     softmax normalised per segment, branch weights folded into P, one PV contraction;
   * LoRA on to_q/to_k/to_v is merged into the packed bf16/fp16/fp32 weights on the GPU whenever a factor changes;
   * float16 models run the bf16 tensor-core kernels with fp16 operands (inference only: grad mode raises);
+  * under CUDA autocast, float32 hidden states compute in the autocast dtype like the reference's autocast'd Linears and
+    SDPA (bf16 always, fp16 without grad; DESIGN.md 4.9): float32 activations are converted by a native kernel;
   * K/V projections can be cached across denoising steps (``kv_cache`` context) because
     ``encoder_hidden_states`` is constant during generation (models/infer.py:89-98).
 """
@@ -93,8 +95,10 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         self._kv_cache = {} if enabled else None
         self._kv_static = bool(static) and enabled
 
-    def _kv_key(self, text, img):
-        key = (text.data_ptr(), img.data_ptr(), tuple(text.shape), tuple(img.shape), text.dtype)
+    def _kv_key(self, text, img, dtype):
+        """Key of the caller's context tensors (not of their converted copies, which are new every call) and the compute
+        dtype."""
+        key = (text.data_ptr(), img.data_ptr(), tuple(text.shape), tuple(img.shape), text.dtype, img.dtype, dtype)
         if not getattr(self, "_kv_static", False):
             key += (text._version, img._version)
         return key
@@ -102,12 +106,16 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
     @torch.no_grad()
     def prepare_kv(self, attn, text, img):
         """(Re)compute the packed K/V of this layer for the given contexts into the cache (in place when the
-        entry exists).  Called once per generation by the denoise loop (SURVEY.md §0.1 D7)."""
+        entry exists).  Called once per generation by the denoise loop (SURVEY.md §0.1 D7).  The compute dtype is resolved
+        from the text states like the processor resolves it from the hidden states (float32 under autocast: 16-bit)."""
         if self._kv_cache is None:
             raise RuntimeError("enable_kv_cache() first")
-        pk = self._weights(attn, text.dtype, text.device)
-        ck = self._kv_key(text, img)
-        kv = ops.kv_pack(text, img, pk.wkv_text, pk.wkv_img, attn.heads, out=self._kv_cache.get(ck))
+        autocast = ops.autocast_dtype() is not None
+        dtype = ops.compute_dtype(text.dtype, False)
+        pk = self._weights(attn, dtype, text.device)
+        ck = self._kv_key(text, img, dtype)
+        kv = ops.kv_pack(_cast(text, dtype, autocast, False), _cast(img, dtype, autocast, False), pk.wkv_text, pk.wkv_img,
+                         attn.heads, out=self._kv_cache.get(ck))
         kv._keepalive = (text, img)
         self._kv_cache[ck] = kv
         return kv
@@ -284,37 +292,56 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         if not hidden_states.is_cuda:
             raise RuntimeError("photoverse_b200 runs on CUDA only (no CPU fallback)")
 
-        dtype, dev = hidden_states.dtype, hidden_states.device
-        x = hidden_states.contiguous()
-        text = encoder_hidden_states.to(dtype).contiguous()
-        img = ip_hidden_states[0].to(dtype).contiguous()
+        dev = hidden_states.device
+        text_in, img_in = encoder_hidden_states, ip_hidden_states[0]
         w_text, w_img = self._fusion_weights()
         self.last_fusion = (w_text, w_img)
 
-        needs_grad = torch.is_grad_enabled() and (
-            x.requires_grad or text.requires_grad or img.requires_grad
+        train = (torch.is_grad_enabled() and (
+            hidden_states.requires_grad or text_in.requires_grad or img_in.requires_grad
             or any(p.requires_grad for p in self.parameters())
             or any(p.requires_grad for m in (attn.to_q, attn.to_k, attn.to_v, attn.to_out[0]) for p in m.parameters()))
-        if needs_grad or self.lora_dropout_active(attn):
+        ) or self.lora_dropout_active(attn)
+        # the hidden states decide the compute dtype (DESIGN.md 4.9); under CUDA autocast a float32 X computes in 16 bits
+        autocast = ops.autocast_dtype() is not None
+        dtype = ops.compute_dtype(hidden_states.dtype, train)
+        if train:
             if dtype == torch.float16:
                 raise NotImplementedError(_F16_TRAINING)
             from .autograd import dual_attn_autograd
+            x, text, img = (_cast(t, dtype, autocast, True) for t in (hidden_states, text_in, img_in))
             y, vnorm = dual_attn_autograd(self, attn, x, text, img, w_text, w_img)
-            self.to_v_ip_norm = vnorm.to(dtype).unsqueeze(-1)
+            # side output (:397): [B, H, Li, 1] in the activation dtype, float32 under autocast (torch.norm's autocast dtype)
+            self.to_v_ip_norm = (vnorm if autocast else vnorm.to(dtype)).unsqueeze(-1)
             return y
 
+        x = _cast(hidden_states, dtype, autocast, False)
         pk = self._weights(attn, dtype, dev)
         kv = None
         ck = None
         if self._kv_cache is not None:
-            ck = self._kv_key(text, img)
+            ck = self._kv_key(text_in, img_in, dtype)
             kv = self._kv_cache.get(ck)
         if kv is None:
+            text, img = _cast(text_in, dtype, autocast, False), _cast(img_in, dtype, autocast, False)
             kv = ops.kv_pack(text, img, pk.wkv_text, pk.wkv_img, attn.heads)
             if self._kv_cache is not None:
-                kv._keepalive = (text, img)      # pin the storage so the data_ptr key cannot be recycled
+                kv._keepalive = (text_in, img_in)      # pin the storage so the data_ptr key cannot be recycled
                 self._kv_cache[ck] = kv
         y, _, _, _ = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, w_text, w_img)
-        # side output (:397): [B, H, Li, 1] in the activation dtype
-        self.to_v_ip_norm = kv.vnorm_act
+        # side output (:397): [B, H, Li, 1] in the activation dtype, float32 under autocast
+        self.to_v_ip_norm = kv.v_ip_norm.unsqueeze(-1) if autocast else kv.vnorm_act
         return y
+
+
+def _cast(t: torch.Tensor, dtype: torch.dtype, autocast: bool, grad: bool) -> torch.Tensor:
+    """``t`` as a contiguous tensor of the compute dtype.  Under autocast a float32 <-> 16-bit conversion is the native
+    kernel (differentiable in grad mode); outside autocast, and between the two 16-bit types, it stays ``Tensor.to``."""
+    if t.dtype == dtype:
+        return t.contiguous()
+    if autocast and torch.float32 in (t.dtype, dtype):
+        if grad:
+            from .autograd import convert
+            return convert(t, dtype)
+        return ops.convert(t, dtype)
+    return t.to(dtype).contiguous()

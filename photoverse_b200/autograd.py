@@ -46,10 +46,30 @@ def _pad_rows8(w: torch.Tensor) -> torch.Tensor:
     return out
 
 
+class _ConvertFn(torch.autograd.Function):
+    """A float32 activation entering the 16-bit path under autocast (and its gradient leaving it): both directions are
+    pv_convert_fwd."""
+
+    @staticmethod
+    def forward(ctx, x, dtype):
+        ctx.src_dtype = x.dtype
+        return ops.convert(x, dtype)
+
+    @staticmethod
+    def backward(ctx, g):
+        return (g if g.dtype == ctx.src_dtype else ops.convert(g, ctx.src_dtype)), None
+
+
+def convert(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
+    """Differentiable :func:`ops.convert`."""
+    return _ConvertFn.apply(x, dtype)
+
+
 class _DualAttnFn(torch.autograd.Function):
     """inputs: x, text, img, to_k_ip.w, to_v_ip.w, (A, B) of to_q, to_k, to_v (None when not injected), ctx object."""
 
     @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda")
     def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, meta):
         proc, attn = meta["proc"], meta["attn"]
         dtype, dev = x.dtype, x.device
@@ -69,6 +89,7 @@ class _DualAttnFn(torch.autograd.Function):
         return y, kv.v_ip_norm.clone()
 
     @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, dy, dvn):
         meta, pk = ctx.meta, ctx.pk
         Lt, Li, H = ctx.dims
@@ -146,6 +167,7 @@ class _DualAttnDropoutFn(torch.autograd.Function):
     consumes the CUDA Philox stream exactly like the reference.  Everything downstream of the masks is C-ABI calls."""
 
     @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda")
     def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, meta):
         proc, attn = meta["proc"], meta["attn"]
         dtype, dev = x.dtype, x.device
@@ -206,6 +228,7 @@ class _DualAttnDropoutFn(torch.autograd.Function):
         return y, kv.v_ip_norm.clone()
 
     @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, dy, dvn):
         meta, u = ctx.meta, ctx.u
         Lt, Li, H = ctx.dims
@@ -316,6 +339,7 @@ class _AdapterFn(torch.autograd.Function):
     weight, bias  (20 tensors per head).  Embeddings (frozen CLIP states) are passed through ``meta``."""
 
     @staticmethod
+    @torch.amp.custom_fwd(device_type="cuda")
     def forward(ctx, meta, *params):
         ad, embs_sel, heads = meta["adapter"], meta["embs"], meta["heads"]
         dtype, dev = embs_sel[0].dtype, embs_sel[0].device
@@ -353,6 +377,7 @@ class _AdapterFn(torch.autograd.Function):
         return out
 
     @staticmethod
+    @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, dout):
         meta, pk, sel, cat = ctx.meta, ctx.pk, ctx.sel, ctx.cat
         ad = meta["adapter"]

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ_DIR = os.path.join(CSRC, "build")
 LIB_PATH = os.path.join(HERE, "libphotoverse_b200.so")
-SOURCES = ["pv_api.cu", "pv_gemm.cu", "pv_gemm3.cu", "pv_attn3.cu", "pv_attn4.cu", "pv_attn6.cu", "pv_simt.cu", "pv_pack.cu", "pv_adapter.cu", "pv_bwd.cu", "pv_bwd_mma.cu", "pv_bwd_tc.cu", "pv_lora_bwd.cu", "pv_loss.cu", "pv_sattn.cu", "pv_backbone.cu"]
+SOURCES = ["pv_api.cu", "pv_gemm.cu", "pv_gemm3.cu", "pv_attn3.cu", "pv_attn4.cu", "pv_attn6.cu", "pv_simt.cu", "pv_pack.cu", "pv_adapter.cu", "pv_bwd.cu", "pv_bwd_mma.cu", "pv_bwd_tc.cu", "pv_lora_bwd.cu", "pv_loss.cu", "pv_sattn.cu", "pv_backbone.cu", "pv_convert.cu"]
 HEADERS = ["pv_common.cuh", "pv_softmax.cuh", "pv_outproj.cuh", "pv_host.h", os.path.join("..", "..", "include", "photoverse_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

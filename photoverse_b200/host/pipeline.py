@@ -15,6 +15,7 @@ What it does the B200 way:
   * one UNet evaluation is captured in a CUDA graph and replayed for the remaining steps (no host sync in the loop)
   * DDIM (BASELINE.json) instead of DPM-Solver++ -- same scheduler on both arms of every comparison
 """
+import contextlib
 from dataclasses import dataclass
 from typing import List, Optional
 
@@ -70,11 +71,30 @@ class _GraphedUNet:
         return self.out
 
 
+def _autocast(dtype: Optional[torch.dtype]):
+    """``torch.autocast("cuda", dtype)`` for a float32 model run in mixed precision; None leaves the caller's autocast state
+    as it is.  Autocast's weight-cast cache stays off: cast weights cached inside a CUDA-graph capture would be freed when
+    the region exits."""
+    if dtype is None:
+        return contextlib.nullcontext()
+    return torch.autocast("cuda", dtype=dtype, cache_enabled=False)
+
+
 @torch.no_grad()
 def run_generation(unet, image_adapter, text_adapter, inputs: GenInputs, num_steps: int = 50,
                    guidance_scale: float = 1.0, token_index=0, mode: str = "batched", use_cuda_graph: bool = True,
-                   kv_cache: bool = True, return_aux: bool = False, scheduler: str = "ddim"):
-    """Returns the final latents [B,4,h,w] (and the adapter outputs if ``return_aux``)."""
+                   kv_cache: bool = True, return_aux: bool = False, scheduler: str = "ddim",
+                   autocast_dtype: Optional[torch.dtype] = None):
+    """Returns the final latents [B,4,h,w] (and the adapter outputs if ``return_aux``).  ``autocast_dtype``: run the
+    adapters and every UNet evaluation (warm-up, graph capture and replay) under ``torch.autocast("cuda", autocast_dtype)``
+    -- a float32 model in the reference's mixed precision."""
+    with _autocast(autocast_dtype):
+        return _run_generation(unet, image_adapter, text_adapter, inputs, num_steps, guidance_scale, token_index, mode,
+                               use_cuda_graph, kv_cache, return_aux, scheduler)
+
+
+def _run_generation(unet, image_adapter, text_adapter, inputs, num_steps, guidance_scale, token_index, mode,
+                    use_cuda_graph, kv_cache, return_aux, scheduler):
     assert mode in ("batched", "two_call", "cond_only")
     if mode == "cond_only" and guidance_scale != 1.0:
         raise ValueError("mode='cond_only' drops the unconditional branch: only valid for guidance_scale == 1")
@@ -170,7 +190,10 @@ class GenerationEngine:
 
     def __init__(self, unet, image_adapter, text_adapter, batch: int, latent: int = 64, num_steps: int = 50,
                  guidance_scale: float = 1.0, token_index=0, mode: str = "batched", dtype=torch.bfloat16,
-                 device="cuda", num_heads_T: int = 5, use_cuda_graph: bool = True):
+                 device="cuda", num_heads_T: int = 5, use_cuda_graph: bool = True,
+                 autocast_dtype: Optional[torch.dtype] = None):
+        """``dtype``: the model's and the encoder buffers' dtype; ``autocast_dtype``: run the adapters and the UNet
+        evaluations (warm-up, capture, replay) under ``torch.autocast("cuda", autocast_dtype)`` (None: off)."""
         assert mode in ("batched", "two_call", "cond_only")
         if mode == "cond_only" and guidance_scale != 1.0:
             raise ValueError("mode='cond_only' is only valid for guidance_scale == 1")
@@ -178,6 +201,7 @@ class GenerationEngine:
         self.B, self.latent, self.num_steps, self.g = batch, latent, num_steps, float(guidance_scale)
         self.token_index, self.mode, self.dtype, self.dev = token_index, mode, dtype, torch.device(device)
         self.use_graph = use_cuda_graph
+        self.autocast_dtype = autocast_dtype
         self.sched = make_ddim_schedule(num_steps)
         self.ts_dev = torch.tensor(self.sched.timesteps, device=self.dev, dtype=torch.float32)
         self.inp = synthetic_inputs(batch, latent, T=num_heads_T, seed=0, device=self.dev, dtype=dtype)
@@ -224,6 +248,10 @@ class GenerationEngine:
 
     @torch.no_grad()
     def generate(self) -> torch.Tensor:
+        with _autocast(self.autocast_dtype):
+            return self._generate()
+
+    def _generate(self) -> torch.Tensor:
         inp, B = self.inp, self.B
         # adapters once per generation (infer.py:89-91)
         if self.text_adapter is not None:

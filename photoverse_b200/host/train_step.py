@@ -18,12 +18,14 @@ Data parallel: gradients are allreduced as bucketed slices of one flat buffer, l
 (photoverse_b200.host.parallel).  Without a ``text_encoder`` the step takes ``batch.text`` as a plain input (the text
 adapter is then trained by L_text alone -- the round-1 behaviour, kept for the kernels' unit tests).
 """
+import contextlib
 from dataclasses import dataclass
 from typing import List, Optional
 
 import torch
 import torch.nn.functional as F
 
+from ..autograd import convert
 from ..loss import train_loss
 from ..unet import get_visual_cross_attention_values_norm
 from .parallel import FlatGradBuffer, OverlappedGradReducer, trainable_named_parameters
@@ -59,7 +61,14 @@ class Trainer:
     GROUPS = ("text_adapter.", "image_adapter.", "unet.")
 
     def __init__(self, unet, image_adapter, text_adapter, lr: float = 1e-4, weight_decay: float = 1e-2, group=None,
-                 text_encoder=None):
+                 text_encoder=None, autocast_dtype: Optional[torch.dtype] = None):
+        """``autocast_dtype=torch.bfloat16``: the forward pass runs under ``torch.autocast("cuda", torch.bfloat16)``, the
+        reference's ``accelerate --mixed_precision bf16`` over float32 weights (DESIGN.md 4.9); float16 is refused, the
+        path has no fp16 backward."""
+        if autocast_dtype not in (None, torch.bfloat16):
+            raise ValueError(f"autocast_dtype must be None or torch.bfloat16 (training has no float16 backward), got "
+                             f"{autocast_dtype}")
+        self.autocast_dtype = autocast_dtype
         self.unet, self.image_adapter, self.text_adapter = unet, image_adapter, text_adapter
         self.text_encoder = text_encoder             # frozen CLIP text tower with concept injection (host/text_encoder.py)
         self.named = trainable_named_parameters(unet, image_adapter, text_adapter)
@@ -83,6 +92,9 @@ class Trainer:
         pred = self.unet(b.noisy_latents, b.timesteps, encoder_hidden_states=(text, img_tokens)).sample     # :505
         vnorms = get_visual_cross_attention_values_norm(self.unet)                    # :512 (stack of the 16 side outputs)
         if pred.is_cuda:      # :509-535 in one reduction kernel (+ one backward kernel): photoverse_b200.loss
+            if self.autocast_dtype is not None:     # :516 mse_loss(pred.float(), target.float()): the target is not rounded
+                pred = pred if pred.dtype == torch.float32 else convert(pred, torch.float32)
+                return train_loss(pred, b.noise.float(), concept, vnorms, 0.01, 0.001)
             return train_loss(pred, b.noise, concept, vnorms, 0.01, 0.001)
         l_text = concept.float().abs().mean()                                         # :509
         l_vis = vnorms.float().mean()                                                 # :513
@@ -107,7 +119,9 @@ class Trainer:
 
     def step(self, b: TrainBatch, max_grad_norm: float = 1.0):
         self.opt.zero_grad(set_to_none=True)
-        with torch.enable_grad():
+        autocast = (contextlib.nullcontext() if self.autocast_dtype is None
+                    else torch.autocast("cuda", dtype=self.autocast_dtype))
+        with torch.enable_grad(), autocast:
             loss, parts = self.loss(b)
         self.reducer.begin(self.expected_gradients())
         loss.backward()                                                               # :538

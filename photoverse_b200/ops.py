@@ -48,6 +48,38 @@ def _f32(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
     return t
 
 
+def resolve_compute_dtype(tensor_dtype: torch.dtype, grad_mode: bool, autocast_dtype: Optional[torch.dtype]) -> torch.dtype:
+    """The dtype the processor and the adapters compute in (DESIGN.md 4.9).  ``autocast_dtype``: the dtype of the
+    enclosing CUDA autocast region, None outside one.  Only float32 activations change dtype under autocast, and float16
+    only without a backward pass (there is no fp16 backward): float32 in grad mode under fp16 autocast stays float32."""
+    if autocast_dtype not in HALF_DTYPES or tensor_dtype != torch.float32:
+        return tensor_dtype
+    if autocast_dtype == torch.float16 and grad_mode:
+        return torch.float32
+    return autocast_dtype
+
+
+def autocast_dtype() -> Optional[torch.dtype]:
+    """The dtype of the enclosing CUDA autocast region, None outside one."""
+    return torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else None
+
+
+def compute_dtype(tensor_dtype: torch.dtype, grad_mode: bool) -> torch.dtype:
+    """:func:`resolve_compute_dtype` under the current CUDA autocast state."""
+    return resolve_compute_dtype(tensor_dtype, grad_mode, autocast_dtype())
+
+
+def convert(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
+    """``x`` converted to ``dtype`` by pv_convert_fwd: float32 -> bfloat16 / float16 (round to nearest even, bit-identical
+    to ``x.to(dtype)``) or bfloat16 / float16 -> float32 (exact).  Returns a new contiguous tensor."""
+    if not x.is_cuda:
+        raise _lib.PhotoverseB200Error("convert: CUDA tensor required (there is no CPU path)")
+    src = x.contiguous()
+    out = torch.empty(src.shape, device=src.device, dtype=dtype)
+    check(_lib.lib().pv_convert_fwd(_dt(src), _code(dtype), _ptr(src), _ptr(out), src.numel(), _stream()), "pv_convert_fwd")
+    return out
+
+
 def pack_weight(w: torch.Tensor, out: torch.Tensor, lora_A=None, lora_B=None, scaling: float = 0.0) -> torch.Tensor:
     """out[out_f, in_f] (bf16|f16|f32) = w + scaling * lora_B @ lora_A  (fp32 masters)."""
     out_f, in_f = w.shape

@@ -21,6 +21,7 @@ import torch
 from torch import nn
 
 from . import ops
+from .attention_processor import _F16_TRAINING, _cast
 
 LN_EPS = 1e-5
 LRELU_SLOPE = 0.01
@@ -94,19 +95,23 @@ class PhotoVerseAdapter(nn.Module):
         return pk
 
     # ------------------------------------------------------------------------------------------
-    def _mlp2(self, x, pk, branch, sel, out2d, act_dtype):
+    def _mlp2(self, x, pk, branch, sel, out2d, save):
         """Two (Linear -> LayerNorm -> LeakyReLU) layers for the selected heads.
-        x: [T, M, D] -> writes the second activation into ``out2d`` ([T*M, HIDDEN] view, may be row-strided)."""
+        x: [T, M, D] -> writes the second activation into ``out2d`` ([T*M, HIDDEN] view, may be row-strided).
+        Returns (x, h1, mean1, rstd1, a1, h2, mean2, rstd2); inference (``save`` False) reuses one fp32 buffer for both
+        layers and keeps no statistics."""
         T, M, _ = x.shape
         dev = x.device
-        h = torch.empty(T, M, HIDDEN, device=dev, dtype=torch.float32)
-        a = torch.empty(T, M, HIDDEN, device=dev, dtype=act_dtype)
-        ops.linear(x, pk[f"{branch}_w1"][sel], pk[f"{branch}_b1"][sel], out=h)
-        ops.ln_lrelu(h.view(T * M, HIDDEN), pk[f"{branch}_g1"][sel], pk[f"{branch}_be1"][sel], a.view(T * M, HIDDEN),
-                     rows_per_group=M, eps=LN_EPS, slope=LRELU_SLOPE)
-        ops.linear(a, pk[f"{branch}_w2"][sel], pk[f"{branch}_b2"][sel], out=h)
-        ops.ln_lrelu(h.view(T * M, HIDDEN), pk[f"{branch}_g2"][sel], pk[f"{branch}_be2"][sel], out2d,
-                     rows_per_group=M, eps=LN_EPS, slope=LRELU_SLOPE)
+        h1 = torch.empty(T, M, HIDDEN, device=dev, dtype=torch.float32)
+        a1 = torch.empty(T, M, HIDDEN, device=dev, dtype=x.dtype)
+        h2 = torch.empty_like(h1) if save else h1
+        ops.linear(x, pk[f"{branch}_w1"][sel], pk[f"{branch}_b1"][sel], out=h1)
+        _, m1, r1 = ops.ln_lrelu(h1.view(T * M, HIDDEN), pk[f"{branch}_g1"][sel], pk[f"{branch}_be1"][sel],
+                                 a1.view(T * M, HIDDEN), rows_per_group=M, eps=LN_EPS, slope=LRELU_SLOPE, save_stats=save)
+        ops.linear(a1, pk[f"{branch}_w2"][sel], pk[f"{branch}_b2"][sel], out=h2)
+        _, m2, r2 = ops.ln_lrelu(h2.view(T * M, HIDDEN), pk[f"{branch}_g2"][sel], pk[f"{branch}_be2"][sel], out2d,
+                                 rows_per_group=M, eps=LN_EPS, slope=LRELU_SLOPE, save_stats=save)
+        return x, h1, m1, r1, a1, h2, m2, r2
 
     def forward(self, embs: List[torch.Tensor], token_index: Optional[Union[int, str]] = None):
         if token_index is not None and token_index != "full":     # adapters.py:32-37
@@ -124,20 +129,21 @@ class PhotoVerseAdapter(nn.Module):
             raise TypeError(f"embeddings must be bfloat16, float16 or float32, got {e0.dtype}")
         train = torch.is_grad_enabled() and (any(p.requires_grad for p in self.parameters())
                                              or any(e.requires_grad for e in embs_sel))
-        # under CUDA autocast float32 embeddings compute in the autocast dtype (DESIGN.md 4.9): converted once per call
+        # under CUDA autocast float32 embeddings compute in the autocast dtype (DESIGN.md 4.9): converted once per call,
+        # differentiably where they require grad (which keeps that visible to adapter_autograd's check)
+        autocast = ops.autocast_dtype() is not None
         dtype = ops.compute_dtype(e0.dtype, train)
-        if dtype != e0.dtype:
-            from .autograd import convert       # keeps requires_grad visible to adapter_autograd's check
-            embs_sel = [e if e.dtype == dtype else (convert if e.requires_grad else ops.convert)(e, dtype) for e in embs_sel]
+        embs_sel = [_cast(e, dtype, autocast, e.requires_grad) for e in embs_sel]
         if train:
             if dtype == torch.float16:
-                raise NotImplementedError("float16 runs the inference (no_grad) path only: training runs in bfloat16 "
-                                          "or float32")
+                raise NotImplementedError(_F16_TRAINING)
             from .autograd import adapter_autograd
             return adapter_autograd(self, embs_sel, heads)
         return self._forward_impl(embs_sel, heads)
 
-    def _forward_impl(self, embs_sel, heads):
+    def _forward_impl(self, embs_sel, heads, save=False):
+        """The adapter on embeddings already in the compute dtype.  ``save``: also return what the backward needs,
+        (packed weights, head slice, per-branch activations and statistics of :meth:`_mlp2`, cat)."""
         dtype, dev = embs_sel[0].dtype, embs_sel[0].device
         B, tokens, D = embs_sel[0].shape
         P = tokens - 1
@@ -145,17 +151,17 @@ class PhotoVerseAdapter(nn.Module):
         pk = self._weights(dtype, dev)
         sel = slice(heads[0], heads[0] + 1) if T == 1 else slice(0, T)
         # gather the CLS rows and the patch rows of the selected heads (one strided copy each: plumbing)
-        stacked = torch.stack([e.to(dtype) for e in embs_sel]) if T > 1 else embs_sel[0].to(dtype).unsqueeze(0)
+        stacked = torch.stack(embs_sel) if T > 1 else embs_sel[0].unsqueeze(0)
         cls = stacked[:, :, 0, :].contiguous()                      # [T, B, D]
         patches = stacked[:, :, 1:, :].reshape(T, B * P, D)         # [T, B*P, D] (copy)
         cat = torch.empty(T, B, 2 * HIDDEN, device=dev, dtype=dtype)
         # CLS branch -> cat[..., :HIDDEN]
-        self._mlp2(cls, pk, "cls", sel, cat.view(T * B, 2 * HIDDEN)[:, :HIDDEN], dtype)
+        saved = {"cls": self._mlp2(cls, pk, "cls", sel, cat.view(T * B, 2 * HIDDEN)[:, :HIDDEN], save)}
         # patch branch -> mean over the P patches -> cat[..., HIDDEN:]
         a2 = torch.empty(T * B * P, HIDDEN, device=dev, dtype=dtype)
-        self._mlp2(patches, pk, "patch", sel, a2, dtype)
+        saved["patch"] = self._mlp2(patches, pk, "patch", sel, a2, save)
         ops.group_mean(a2.view(T * B, P, HIDDEN), cat.view(T * B, 2 * HIDDEN)[:, HIDDEN:])
         # last Linear of both branches in one K=2048 GEMM, written straight into [B, T, E]
         out = torch.empty(B, T, self.cross_attention_dim, device=dev, dtype=dtype)
         ops.linear(cat, pk["w3"][sel], pk["b3"][sel], out=out.permute(1, 0, 2))
-        return out
+        return (out, (pk, sel, saved, cat)) if save else out

@@ -16,6 +16,7 @@ Differences in *how* (not what) it computes, see DESIGN.md:
   * K/V projections can be cached across denoising steps (``kv_cache`` context) because
     ``encoder_hidden_states`` is constant during generation (models/infer.py:89-98).
 """
+import copy
 from typing import Optional
 
 import torch
@@ -63,14 +64,11 @@ class PhotoVerseAttnProcessor(nn.Module):
 
 
 class _PackedWeights:
-    __slots__ = ("key", "wq", "wkv_text", "wkv_img", "wo", "bo", "_t")
-
-
-class _UnmergedWeights:
-    """Packed weights of the LoRA-dropout training path: the low-rank branch is a K-extension of the base GEMM,
-    ``[x | dropout(x) A^T] @ [W | s B]^T`` (rank columns padded to 8), instead of a merged W + s B A."""
-    __slots__ = ("key", "wq", "wq_aug", "wkv_text", "wkv_text_aug", "wkv_img", "wkv_img_aug", "wo", "bo", "eye",
-                 "ranks", "_t")
+    """Packed weights of one layer in one compute dtype.  Merged: LoRA folded into ``wq`` / ``wkv_text`` (W + s B A).
+    Unmerged (the LoRA-dropout training path): ``wq`` / ``wkv_text`` hold the base weights and the low-rank branch is a
+    K-extension of the base GEMM, ``[x | dropout(x) A^T] @ [W | s B]^T`` (``*_aug``, rank columns padded to 8)."""
+    __slots__ = ("key", "wq", "wkv_text", "wkv_img", "wo", "bo", "_t",
+                 "wq_aug", "wkv_text_aug", "wkv_img_aug", "ranks", "eye")
 
 
 def _pad8(n: int) -> int:
@@ -81,7 +79,7 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
     def __init__(self, hidden_size, cross_attention_dim=None, num_tokens=(5,), scale=2.0, fusion_rules=(1 / 3, 2 / 3)):
         super().__init__(hidden_size, cross_attention_dim, num_tokens, scale, fusion_rules)
         self.to_v_ip_norm = None
-        self._packed = {}          # dtype -> _PackedWeights
+        self._packed = {}          # (dtype, merged) -> _PackedWeights
         self._kv_cache = None      # dict while a kv_cache scope is active, else None
         self._kv_static = False
         self.last_fusion = (1.0, 1.0)
@@ -121,14 +119,15 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         return kv
 
     # ------------------------------------------------------------------------------------------
-    def _weights(self, attn, dtype, device):
-        """Packed weights of this layer in the compute dtype, LoRA merged (W + s B A).  Each of the four operands is
-        re-packed only when one of ITS OWN sources changed (parameter version counters): in training the optimizer
-        touches the LoRA factors and to_k_ip / to_v_ip every step, the frozen out projection never."""
+    def _weights(self, attn, dtype, device, merged: bool = True):
+        """Packed weights of this layer in the compute dtype: LoRA merged (W + s B A), or with ``merged=False`` the base
+        weights plus the K-extended operands of the LoRA-dropout path.  Each of the four operands is re-packed only when
+        one of ITS OWN sources changed (parameter version counters): in training the optimizer touches the LoRA factors
+        and to_k_ip / to_v_ip every step, the frozen out projection never."""
         wq, qa, qb, qs, qp = linear_parts(attn.to_q)
         wk, ka, kb, ks, kp = linear_parts(attn.to_k)
         wv, va, vb, vs, vp = linear_parts(attn.to_v)
-        if max(qp, kp, vp) > 0.0:
+        if merged and max(qp, kp, vp) > 0.0:
             raise RuntimeError("internal: merged weights requested while LoRA dropout is active")
         wo, bo = attn.to_out[0].weight, attn.to_out[0].bias
         kip, vip = self.to_k_ip[0].weight, self.to_v_ip[0].weight
@@ -138,7 +137,7 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
 
         keys = {"wq": vkey([wq, qa, qb], qs), "wkv_text": vkey([wk, ka, kb, wv, va, vb], ks, vs),
                 "wkv_img": vkey([kip, vip]), "wo": vkey([wo, bo])}
-        pk = self._packed.get(dtype)
+        pk = self._packed.get((dtype, merged))
         if pk is not None and pk.key == keys:
             return pk
         C, Dc = wq.shape[0], wk.shape[1]
@@ -149,36 +148,60 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         def m(t):   # fp32 master view of a parameter (a cast happens only if the module was .to(bf16)'d)
             return None if t is None else t.detach().float().contiguous()
 
+        def lora(a, b, s):     # the LoRA operands of pack_weight: none when the branch stays a K-extension
+            return (m(a), m(b), s) if merged else ()
+
+        def sb(b, s, r8):      # s * B, rank columns zero-padded to r8 (weight layout only, no activation math)
+            out = torch.zeros(C, r8, device=device, dtype=dtype)
+            out[:, :b.shape[1]] = (b.detach().float() * s).to(dtype)
+            return out
+
         old = pk.key if pk is not None else {}
+        fresh = {name for name in keys if old.get(name) != keys[name]}
         with torch.no_grad():
             if pk is None:
                 pk = _PackedWeights()
                 pk._t = {}
+                # bf16: the attention kernel always applies a [C,C] projection; the already-projected Q goes through I
+                pk.eye = torch.eye(C, device=device, dtype=dtype) if dtype == torch.bfloat16 and not merged else None
             else:                      # a NEW object per key set: autograd contexts of earlier calls keep the old one
-                npk = _PackedWeights()
-                npk.wq, npk.wkv_text, npk.wkv_img, npk.wo, npk.bo = pk.wq, pk.wkv_text, pk.wkv_img, pk.wo, pk.bo
-                npk._t = dict(pk._t)
-                pk = npk
-            if old.get("wq") != keys["wq"]:
-                pk.wq = ops.pack_weight(m(wq), torch.empty(C, C, device=device, dtype=dtype), m(qa), m(qb), qs)
+                pk = copy.copy(pk)
+                pk._t = dict(pk._t)
+            if "wq" in fresh:
+                pk.wq = ops.pack_weight(m(wq), torch.empty(C, C, device=device, dtype=dtype), *lora(qa, qb, qs))
                 pk._t.pop("wq_t", None)
-            if old.get("wkv_text") != keys["wkv_text"]:
+            if "wkv_text" in fresh:
                 pk.wkv_text = torch.empty(2 * C, Dc, device=device, dtype=dtype)
-                ops.pack_weight(m(wk), pk.wkv_text[:C], m(ka), m(kb), ks)
-                ops.pack_weight(m(wv), pk.wkv_text[C:], m(va), m(vb), vs)
+                ops.pack_weight(m(wk), pk.wkv_text[:C], *lora(ka, kb, ks))
+                ops.pack_weight(m(wv), pk.wkv_text[C:], *lora(va, vb, vs))
                 pk._t.pop("wkv_text_t", None)
-            if old.get("wkv_img") != keys["wkv_img"]:
+            if "wkv_img" in fresh:
                 pk.wkv_img = torch.empty(2 * C, Dc, device=device, dtype=dtype)
                 ops.pack_weight(m(kip), pk.wkv_img[:C])
                 ops.pack_weight(m(vip), pk.wkv_img[C:])
                 pk._t.pop("wkv_img_t", None)
-            if old.get("wo") != keys["wo"]:
+            if "wo" in fresh:
                 pk.wo = ops.pack_weight(m(wo), torch.empty(C, C, device=device, dtype=dtype))
                 pk.bo = m(bo) if bo is not None else torch.zeros(C, device=device, dtype=torch.float32)
                 pk._t.pop("wo_t", None)
+            if not merged:
+                pk.ranks = rq, rk, rv = tuple(0 if a is None else _pad8(a.shape[0]) for a in (qa, ka, va))
+                if "wq" in fresh:
+                    pk.wq_aug = torch.cat([pk.wq, sb(qb, qs, rq)], 1).contiguous() if rq else pk.wq
+                if fresh & {"wkv_text", "wkv_img"}:
+                    if rk or rv:       # K/V of the text branch with their low-rank columns, image branch zero-extended
+                        ext = torch.zeros(2 * C, rk + rv, device=device, dtype=dtype)
+                        if rk:
+                            ext[:C, :rk] = sb(kb, ks, rk)
+                        if rv:
+                            ext[C:, rk:] = sb(vb, vs, rv)
+                        pk.wkv_text_aug = torch.cat([pk.wkv_text, ext], 1).contiguous()
+                        pk.wkv_img_aug = torch.cat([pk.wkv_img, torch.zeros_like(ext)], 1).contiguous()
+                    else:
+                        pk.wkv_text_aug, pk.wkv_img_aug = pk.wkv_text, pk.wkv_img
             pk.key = keys
-        self._packed[dtype] = pk
-        if self._kv_cache is not None and (old.get("wkv_text") != keys["wkv_text"] or old.get("wkv_img") != keys["wkv_img"]):
+        self._packed[(dtype, merged)] = pk
+        if self._kv_cache is not None and fresh & {"wkv_text", "wkv_img"}:
             self._kv_cache.clear()
         return pk
 
@@ -186,58 +209,6 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         """True when a LoRA-wrapped projection of ``attn`` is in training mode with dropout p > 0 (peft applies
         ``lora_dropout`` to the low-rank branch input only; train.py:264-269, 348-354)."""
         return any(linear_parts(m)[4] > 0.0 for m in (attn.to_q, attn.to_k, attn.to_v))
-
-    def _weights_unmerged(self, attn, dtype, device):
-        parts = [linear_parts(m) for m in (attn.to_q, attn.to_k, attn.to_v)]
-        (wq, qa, qb, qs, _), (wk, ka, kb, ks, _), (wv, va, vb, vs, _) = parts
-        wo, bo = attn.to_out[0].weight, attn.to_out[0].bias
-        kip, vip = self.to_k_ip[0].weight, self.to_v_ip[0].weight
-        tensors = [wq, qa, qb, wk, ka, kb, wv, va, vb, wo, bo, kip, vip]
-        key = tuple((t.data_ptr(), t._version) if t is not None else None for t in tensors) + (qs, ks, vs)
-        cache = self._packed.get(("unmerged", dtype))
-        if cache is not None and cache.key == key:
-            return cache
-        for t in tensors:
-            if t is not None and not t.is_cuda:
-                raise RuntimeError(f"photoverse_b200 needs its weights on the CUDA device (got {t.device})")
-        C, Dc = wq.shape[0], wk.shape[1]
-        rq, rk, rv = (0 if a is None else _pad8(a.shape[0]) for a in (qa, ka, va))
-
-        def m(t):
-            return t.detach().float().contiguous()
-
-        def sb(b, s, r8):        # s * B, rank columns zero-padded to r8 (weight layout only, no activation math)
-            out = torch.zeros(C, r8, device=device, dtype=dtype)
-            out[:, :b.shape[1]] = (b.detach().float() * s).to(dtype)
-            return out
-
-        with torch.no_grad():
-            u = _UnmergedWeights()
-            u.key, u.ranks = key, (rq, rk, rv)
-            u.wq = ops.pack_weight(m(wq), torch.empty(C, C, device=device, dtype=dtype))
-            u.wq_aug = torch.cat([u.wq, sb(qb, qs, rq)], 1).contiguous() if rq else u.wq
-            u.wkv_text = torch.empty(2 * C, Dc, device=device, dtype=dtype)
-            ops.pack_weight(m(wk), u.wkv_text[:C])
-            ops.pack_weight(m(wv), u.wkv_text[C:])
-            u.wkv_img = torch.empty(2 * C, Dc, device=device, dtype=dtype)
-            ops.pack_weight(m(kip), u.wkv_img[:C])
-            ops.pack_weight(m(vip), u.wkv_img[C:])
-            if rk or rv:
-                ext = torch.zeros(2 * C, rk + rv, device=device, dtype=dtype)
-                if rk:
-                    ext[:C, :rk] = sb(kb, ks, rk)
-                if rv:
-                    ext[C:, rk:] = sb(vb, vs, rv)
-                u.wkv_text_aug = torch.cat([u.wkv_text, ext], 1).contiguous()
-                u.wkv_img_aug = torch.cat([u.wkv_img, torch.zeros_like(ext)], 1).contiguous()
-            else:
-                u.wkv_text_aug, u.wkv_img_aug = u.wkv_text, u.wkv_img
-            u.wo = ops.pack_weight(m(wo), torch.empty(C, C, device=device, dtype=dtype))
-            u.bo = m(bo) if bo is not None else torch.zeros(C, device=device, dtype=torch.float32)
-            # bf16: the attention kernel always applies a [C,C] projection; the already-projected Q goes through I
-            u.eye = torch.eye(C, device=device, dtype=dtype) if dtype == torch.bfloat16 else None
-        self._packed[("unmerged", dtype)] = u
-        return u
 
     def _fusion_weights(self):
         """(w_text, w_image) -- reference attention_processor.py:411-420, including its RNG draw."""

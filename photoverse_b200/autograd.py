@@ -16,13 +16,9 @@ from typing import List
 import torch
 
 from . import ops
+from .adapters import HIDDEN, LRELU_SLOPE
+from .attention_processor import _pad8
 from .lora import linear_parts
-
-HIDDEN = 1024
-
-
-def _pad8(n: int) -> int:
-    return (n + 7) // 8 * 8
 
 
 def _skinny_linear(a2d: torch.Tensor, w: torch.Tensor, full: bool = False) -> torch.Tensor:
@@ -66,26 +62,18 @@ def convert(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
 
 
 class _DualAttnFn(torch.autograd.Function):
-    """inputs: x, text, img, to_k_ip.w, to_v_ip.w, (A, B) of to_q, to_k, to_v (None when not injected), ctx object."""
+    """inputs: x, text, img, to_k_ip.w, to_v_ip.w, (A, B) of to_q, to_k, to_v (None when not injected), ctx object.
+    LoRA is merged into the packed weights and the Q projection runs inside the attention kernel."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda")
     def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, meta):
         proc, attn = meta["proc"], meta["attn"]
-        dtype, dev = x.dtype, x.device
-        pk = proc._weights(attn, dtype, dev)
+        pk = proc._weights(attn, x.dtype, x.device)
         kv = ops.kv_pack(text, img, pk.wkv_text, pk.wkv_img, attn.heads)
         y, o, stats, q = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, meta["w_text"], meta["w_img"], want_stats=True)
-        ctx.meta = meta
-        ctx.pk = pk
-        ctx.dims = (kv.Lt, kv.Li, attn.heads)
-        ctx.has = (qA is not None, kA is not None, vA is not None)
-        saved = [x, text, img, stats, kv.kv_text, kv.kv_img, kv.v_ip_norm]
-        if q is not None:
-            saved.append(q)                      # fp32 mode keeps Q; the bf16 kernel never writes it (recomputed)
-        ctx.save_for_backward(*saved, *[t for t in (qA, qB, kA, kB, vA, vB) if t is not None])
-        ctx.n_saved = len(saved)
-        ctx.pdt = (w_kip.dtype, w_vip.dtype)
+        # fp32 mode keeps Q; the bf16 kernel never writes it (q is None: recomputed in backward)
+        _save(ctx, meta, pk, kv, stats, q, (x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB))
         return y, kv.v_ip_norm.clone()
 
     @staticmethod
@@ -93,26 +81,25 @@ class _DualAttnFn(torch.autograd.Function):
     def backward(ctx, dy, dvn):
         meta, pk = ctx.meta, ctx.pk
         Lt, Li, H = ctx.dims
-        tensors = ctx.saved_tensors
-        x, text, img, stats, kv_text, kv_img, v_ip_norm = tensors[:7]
-        q_saved = tensors[7] if ctx.n_saved == 8 else None
-        lora = list(tensors[ctx.n_saved:])
+        x, text, img, stats, kv_text, kv_img, v_ip_norm, q, *rest = ctx.saved_tensors
+        lora, drop = rest[:6], rest[6:]          # drop: dropout(x) of to_q / to_k / to_v, then their keep-masks
         dtype = x.dtype
         B, S, C = x.shape
         Dc = text.shape[2]
         x2, text2, img2 = x.view(B * S, C), text.view(B * Lt, Dc), img.view(B * Li, Dc)
-        tw = _transposed(pk, dtype)
+        tw = _transposed(pk)
 
         dy2 = dy.contiguous().view(B * S, C).to(dtype)
         d_o = ops.linear(dy2, tw["wo_t"]).view(B, S, C)                                  # dO = dY Wo
-        q = q_saved if q_saved is not None else ops.linear(x2, pk.wq).view(B, S, C)      # recompute Q = X Wq^T
+        if q is None:
+            q = ops.linear(x2, pk.wq).view(B, S, C)                                      # recompute Q = X Wq^T
         d_vn = dvn if (dvn is not None and meta["vnorm_grad"]) else None
         dq, dkv_text, dkv_img = ops.dual_attn_bwd(d_o, q, kv_text, kv_img, stats, v_ip_norm, d_vn, H, Lt, Li,
                                                   meta["w_text"], meta["w_img"])
         dq2 = dq.view(B * S, C)
         need = ctx.needs_input_grad
-        dx = ops.linear(dq2, tw["wq_t"]).view(B, S, C) if need[0] else None              # dX = dQ Wq
-        dtext = ops.linear(dkv_text, tw["wkv_text_t"]).view(B, Lt, Dc) if need[1] else None
+        dx = ops.linear(dq2, tw["wq_t"]) if need[0] else None                            # dX = dQ Wq (base weights)
+        dtext = ops.linear(dkv_text, tw["wkv_text_t"]) if need[1] else None
         dimg = ops.linear(dkv_img, tw["wkv_img_t"]).view(B, Li, Dc) if need[2] else None
         # to_k_ip / to_v_ip : [dK_img | dV_img]^T img in one weight-gradient call -> rows [0, C) / [C, 2C)
         dkip = dvip = None
@@ -122,29 +109,44 @@ class _DualAttnFn(torch.autograd.Function):
             dvip = dkv_w[C:] if need[4] else None
         # LoRA factors: y = W x + s B (A x)  ->  dB = s dY^T (x A^T),  dA = s (dY B)^T x
         grads = [None] * 6
-        it = iter(lora)
-        srcs = ((x2, dq2, meta["scal"][0]), (text2, dkv_text[:, :C], meta["scal"][1]), (text2, dkv_text[:, C:], meta["scal"][2]))
-        for j, (inp, g, s) in enumerate(srcs):
-            if not ctx.has[j]:
+        srcs = ((x2, dq2, dx, need[0]), (text2, dkv_text[:, :C], dtext, need[1]), (text2, dkv_text[:, C:], dtext, need[1]))
+        for j, (inp, g, dinp, need_inp) in enumerate(srcs):
+            A, Bm = lora[2 * j], lora[2 * j + 1]
+            if A is None:
                 continue
-            A, Bm = next(it), next(it)
-            if j > 0 and meta["w_text"] == 0.0:
-                continue                                                     # text branch dropped: no gradient (see below)
-            if need[5 + 2 * j] and need[5 + 2 * j + 1]:
-                fused = ops.lora_bwd(inp, g, A, Bm, s)                       # both factors, one pass over x and dY (rank <= 16)
-                if fused is not None:
-                    grads[2 * j], grads[2 * j + 1] = fused[0].to(A.dtype), fused[1].to(Bm.dtype)
-                    continue
+            s, need_a, need_b = meta["scal"][j], need[5 + 2 * j], need[5 + 2 * j + 1]
+            if not drop:
+                if j > 0 and meta["w_text"] == 0.0:
+                    continue                                                 # text branch dropped: no gradient (see below)
+                if need_a and need_b:
+                    fused = ops.lora_bwd(inp, g, A, Bm, s)                   # both factors, one pass over x and dY (rank <= 16)
+                    if fused is not None:
+                        grads[2 * j:2 * j + 2] = fused
+                        continue
+            else:
+                inp = drop[j]                                                # dropout(x): what the branch saw
             a_c = A.detach().to(dtype).contiguous()                          # [r, in]
             bt_c = ops.transpose(Bm.detach().to(dtype).contiguous())         # [r, out]
-            if need[5 + 2 * j + 1]:
+            if need_b:
                 t = _skinny_linear(inp, a_c)                                 # x A^T            [M, r]
-                grads[2 * j + 1] = ops.linear_bwd_weight(g, t, alpha=s).to(Bm.dtype)      # dB [out, r]
-            if need[5 + 2 * j]:
-                u = _skinny_linear(g, bt_c)                                  # dY B             [M, r]
-                grads[2 * j] = ops.linear_bwd_weight(u, inp, alpha=s).to(A.dtype)         # dA [r, in]
-        dkip = None if dkip is None else dkip.to(ctx.pdt[0])
-        dvip = None if dvip is None else dvip.to(ctx.pdt[1])
+                grads[2 * j + 1] = ops.linear_bwd_weight(g, t, alpha=s)      # dB [out, r]
+            grad_inp = bool(drop) and need_inp
+            if need_a or grad_inp:
+                ub = _skinny_linear(g, bt_c, full=grad_inp)                  # dY B             [M, r] (padded: pad8(r))
+                r = a_c.shape[0]
+                if need_a:
+                    grads[2 * j] = ops.linear_bwd_weight(ub[:, :r], inp, alpha=s)        # dA [r, in]
+                if grad_inp:
+                    # d dropout(x) = s (dY B) A, then through the mask:  d x += keep / (1 - p) * that
+                    at8 = ops.transpose(_pad_rows8(a_c * s))                 # [in, pad8(r)]
+                    v = ops.linear(ub, at8)                                  # [M, in]
+                    mask = drop[3 + j]
+                    if mask is not None:
+                        ops.dropout_bwd_acc(dinp, v, mask, meta["drop"][j])
+                    else:
+                        ops.dropout_bwd_acc(dinp, v, torch.ones_like(v, dtype=torch.bool), 0.0)
+        dx = None if dx is None else dx.view(B, S, C)
+        dtext = None if dtext is None else dtext.view(B, Lt, Dc)
         # A branch the fusion rule dropped (attention_processor.py:413-418) is not part of the reference's graph: its
         # parameters get NO gradient there (``.grad`` stays None and AdamW skips them -- no weight decay, no stale-momentum
         # update), not a zero one.  to_v_ip still receives the ``to_v_ip_norm`` regulariser term (:397, train.py:512-513).
@@ -154,27 +156,29 @@ class _DualAttnFn(torch.autograd.Function):
                 dvip = None
         if meta["w_text"] == 0.0:
             grads[2:6] = [None] * 4                   # LoRA factors of to_k / to_v (text branch)
-        return (dx, dtext, dimg, dkip, dvip, *grads, None)
+        pgrads = [None if gr is None else gr.to(dt) for gr, dt in zip((dkip, dvip, *grads), ctx.pdt)]
+        return (dx, dtext, dimg, *pgrads, None)
 
 
-class _DualAttnDropoutFn(torch.autograd.Function):
+class _DualAttnDropoutFn(_DualAttnFn):
     """Training step with LoRA dropout p > 0 (the reference default, train.py:264-269): peft's
     ``W x + s B A dropout(x)`` cannot be merged into one weight, so the low-rank branch rides along as a K-extension of
     the projection GEMMs: ``Q = [x | dropout(x) A^T] [W | s B]^T`` (same for K_text / V_text, each with its own mask).
 
     The keep-masks come from ``torch.native_dropout`` -- the kernel ``nn.Dropout`` dispatches to -- drawn in the
     reference's order (to_q, to_k, to_v; attention_processor.py:297, 304-305) on same-shaped tensors, so a seeded run
-    consumes the CUDA Philox stream exactly like the reference.  Everything downstream of the masks is C-ABI calls."""
+    consumes the CUDA Philox stream exactly like the reference.  Everything downstream of the masks is C-ABI calls.
+    The backward is :class:`_DualAttnFn`'s, with the LoRA factors' gradients taken from dropout(x) and the low-rank
+    branch's input gradient added through the keep-masks."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda")
     def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, meta):
         proc, attn = meta["proc"], meta["attn"]
         dtype, dev = x.dtype, x.device
-        u = proc._weights_unmerged(attn, dtype, dev)
+        u = proc._weights(attn, dtype, dev, merged=False)
         B, S, C = x.shape
         Lt, Li, Dc = text.shape[1], img.shape[1], text.shape[2]
-        H = attn.heads
         rq, rk, rv = u.ranks
         pq, pk_, pv = meta["drop"]
         x2, text2 = x.view(B * S, C), text.view(B * Lt, Dc)
@@ -212,97 +216,25 @@ class _DualAttnDropoutFn(torch.autograd.Function):
             ia[..., :Dc] = img
         else:
             ta, ia = text, img
-        kv = ops.kv_pack(ta, ia, u.wkv_text_aug, u.wkv_img_aug, H)
+        kv = ops.kv_pack(ta, ia, u.wkv_text_aug, u.wkv_img_aug, attn.heads)
         o, stats = ops.dual_attn_core(q, u.eye, kv, meta["w_text"], meta["w_img"], want_stats=True)
         y = ops.linear(o.view(B * S, C), u.wo, u.bo).view(B, S, C)
-
-        ctx.meta, ctx.u = meta, u
-        ctx.dims = (Lt, Li, H)
-        ctx.has = (qA is not None, kA is not None, vA is not None)
-        ctx.masked = (m_q is not None, m_k is not None, m_v is not None)
-        saved = [x, text, img, stats, kv.kv_text, kv.kv_img, kv.v_ip_norm, q]
-        saved += [t for t in (xd_q, xd_k, xd_v) if t is not None]
-        saved += [t for t in (m_q, m_k, m_v) if t is not None]
-        ctx.save_for_backward(*saved, *[t for t in (qA, qB, kA, kB, vA, vB) if t is not None])
-        ctx.pdt = (w_kip.dtype, w_vip.dtype)
+        _save(ctx, meta, u, kv, stats, q, (x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB),
+              (xd_q, xd_k, xd_v, m_q, m_k, m_v))
         return y, kv.v_ip_norm.clone()
 
-    @staticmethod
-    @torch.amp.custom_bwd(device_type="cuda")
-    def backward(ctx, dy, dvn):
-        meta, u = ctx.meta, ctx.u
-        Lt, Li, H = ctx.dims
-        it = iter(ctx.saved_tensors)
-        x, text, img, stats, kv_text, kv_img, v_ip_norm, q = (next(it) for _ in range(8))
-        xd = [next(it) if h else None for h in ctx.has]
-        masks = [next(it) if mk else None for mk in ctx.masked]
-        lora = [(next(it), next(it)) if h else None for h in ctx.has]
-        dtype = x.dtype
-        B, S, C = x.shape
-        Dc = text.shape[2]
-        img2 = img.view(B * Li, Dc)
-        tw = getattr(u, "_t", None)
-        if tw is None:
-            tw = {"wq_t": ops.transpose(u.wq), "wo_t": ops.transpose(u.wo),
-                  "wkv_text_t": ops.transpose(u.wkv_text), "wkv_img_t": ops.transpose(u.wkv_img)}
-            u._t = tw
 
-        dy2 = dy.contiguous().view(B * S, C).to(dtype)
-        d_o = ops.linear(dy2, tw["wo_t"]).view(B, S, C)
-        d_vn = dvn if (dvn is not None and meta["vnorm_grad"]) else None
-        dq, dkv_text, dkv_img = ops.dual_attn_bwd(d_o, q, kv_text, kv_img, stats, v_ip_norm, d_vn, H, Lt, Li,
-                                                  meta["w_text"], meta["w_img"])
-        dq2 = dq.view(B * S, C)
-        need = ctx.needs_input_grad
-        dx = ops.linear(dq2, tw["wq_t"]) if need[0] else None                    # base-weight terms
-        dtext = ops.linear(dkv_text, tw["wkv_text_t"]) if need[1] else None
-        dimg = ops.linear(dkv_img, tw["wkv_img_t"]).view(B, Li, Dc) if need[2] else None
-        dkip = ops.linear_bwd_weight(dkv_img[:, :C], img2) if need[3] else None
-        dvip = ops.linear_bwd_weight(dkv_img[:, C:], img2) if need[4] else None
-
-        grads = [None] * 6
-        srcs = ((dq2, dx, need[0]), (dkv_text[:, :C], dtext, need[1]), (dkv_text[:, C:], dtext, need[1]))
-        pdrop = meta["drop"]
-        for j, (g, dinp, need_inp) in enumerate(srcs):
-            if not ctx.has[j]:
-                continue
-            A, Bm = lora[j]
-            s = meta["scal"][j]
-            a_c = A.detach().to(dtype).contiguous()                              # [r, in]
-            bt_c = ops.transpose(Bm.detach().to(dtype).contiguous())             # [r, out]
-            inp = xd[j]                                                          # dropout(x): what the branch saw
-            ub = _skinny_linear(g, bt_c, full=True)                              # dY B   [M, pad8(r)], zero-padded
-            r = a_c.shape[0]
-            if need[5 + 2 * j + 1]:
-                t = _skinny_linear(inp, a_c)                                     # dropout(x) A^T   [M, r]
-                grads[2 * j + 1] = ops.linear_bwd_weight(g, t, alpha=s).to(Bm.dtype)          # dB
-            if need[5 + 2 * j]:
-                grads[2 * j] = ops.linear_bwd_weight(ub[:, :r], inp, alpha=s).to(A.dtype)     # dA
-            if need_inp:
-                # d dropout(x) = s (dY B) A, then through the mask:  d x += keep / (1 - p) * that
-                at8 = ops.transpose(_pad_rows8(a_c * s))                         # [in, pad8(r)]
-                v = ops.linear(ub, at8)                                          # [M, in]
-                if masks[j] is not None:
-                    ops.dropout_bwd_acc(dinp, v, masks[j], pdrop[j])
-                else:
-                    ops.dropout_bwd_acc(dinp, v, torch.ones_like(v, dtype=torch.bool), 0.0)
-        dx = None if dx is None else dx.view(B, S, C)
-        dtext = None if dtext is None else dtext.view(B, Lt, Dc)
-        dkip = None if dkip is None else dkip.to(ctx.pdt[0])
-        dvip = None if dvip is None else dvip.to(ctx.pdt[1])
-        # A branch the fusion rule dropped (attention_processor.py:413-418) is not part of the reference's graph: its
-        # parameters get NO gradient there (``.grad`` stays None and AdamW skips them -- no weight decay, no stale-momentum
-        # update), not a zero one.  to_v_ip still receives the ``to_v_ip_norm`` regulariser term (:397, train.py:512-513).
-        if meta["w_img"] == 0.0:
-            dkip = None
-            if dvn is None or not meta["vnorm_grad"]:
-                dvip = None
-        if meta["w_text"] == 0.0:
-            grads[2:6] = [None] * 4                   # LoRA factors of to_k / to_v (text branch)
-        return (dx, dtext, dimg, dkip, dvip, *grads, None)
+def _save(ctx, meta, pk, kv, stats, q, inputs, drop=()):
+    """What :meth:`_DualAttnFn.backward` reads: the pack the forward ran with (a re-pack makes a new object, so later
+    parameter updates do not reach this backward), the saved tensors and the parameter dtypes of the gradients."""
+    x, text, img, w_kip, w_vip, *lora = inputs
+    ctx.meta, ctx.pk = meta, pk
+    ctx.dims = (text.shape[1], img.shape[1], kv.H)
+    ctx.save_for_backward(x, text, img, stats, kv.kv_text, kv.kv_img, kv.v_ip_norm, q, *lora, *drop)
+    ctx.pdt = [None if t is None else t.dtype for t in (w_kip, w_vip, *lora)]
 
 
-def _transposed(pk, dtype):
+def _transposed(pk):
     """Transposed copies of the packed forward weights (the weights of the input-gradient GEMMs), cached per operand on the
     pack: the processor drops an entry when it re-packs that operand (attention_processor._weights)."""
     tw = pk._t
@@ -341,47 +273,18 @@ class _AdapterFn(torch.autograd.Function):
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda")
     def forward(ctx, meta, *params):
-        ad, embs_sel, heads = meta["adapter"], meta["embs"], meta["heads"]
-        dtype, dev = embs_sel[0].dtype, embs_sel[0].device
-        B, tokens, D = embs_sel[0].shape
-        P, T = tokens - 1, len(heads)
-        pk = ad._weights(dtype, dev)
-        sel = slice(heads[0], heads[0] + 1) if T == 1 else slice(0, T)
-        stacked = torch.stack([e.to(dtype) for e in embs_sel]) if T > 1 else embs_sel[0].to(dtype).unsqueeze(0)
-        xin = {"cls": stacked[:, :, 0, :].contiguous(), "patch": stacked[:, :, 1:, :].reshape(T, B * P, D)}
-        cat = torch.empty(T, B, 2 * HIDDEN, device=dev, dtype=dtype)
-        saved = {}
-        for branch in ("cls", "patch"):
-            x = xin[branch]
-            M = x.shape[1]
-            h1 = torch.empty(T, M, HIDDEN, device=dev, dtype=torch.float32)
-            a1 = torch.empty(T, M, HIDDEN, device=dev, dtype=dtype)
-            h2 = torch.empty(T, M, HIDDEN, device=dev, dtype=torch.float32)
-            ops.linear(x, pk[f"{branch}_w1"][sel], pk[f"{branch}_b1"][sel], out=h1)
-            _, m1, r1 = ops.ln_lrelu(h1.view(T * M, HIDDEN), pk[f"{branch}_g1"][sel], pk[f"{branch}_be1"][sel],
-                                     a1.view(T * M, HIDDEN), rows_per_group=M, save_stats=True)
-            ops.linear(a1, pk[f"{branch}_w2"][sel], pk[f"{branch}_b2"][sel], out=h2)
-            if branch == "cls":
-                a2 = cat.view(T * B, 2 * HIDDEN)[:, :HIDDEN]
-            else:
-                a2 = torch.empty(T * M, HIDDEN, device=dev, dtype=dtype)
-            _, m2, r2 = ops.ln_lrelu(h2.view(T * M, HIDDEN), pk[f"{branch}_g2"][sel], pk[f"{branch}_be2"][sel], a2,
-                                     rows_per_group=M, save_stats=True)
-            if branch == "patch":
-                ops.group_mean(a2.view(T * B, P, HIDDEN), cat.view(T * B, 2 * HIDDEN)[:, HIDDEN:])
-            saved[branch] = (x, h1, m1, r1, a1, h2, m2, r2)
-        out = torch.empty(B, T, ad.cross_attention_dim, device=dev, dtype=dtype)
-        ops.linear(cat, pk["w3"][sel], pk["b3"][sel], out=out.permute(1, 0, 2))
-        ctx.meta, ctx.pk, ctx.sel, ctx.saved, ctx.cat = meta, pk, sel, saved, cat
-        ctx.geom = (B, P, T, D)
+        out, ctx.saved = meta["adapter"]._forward_impl(meta["embs"], meta["heads"], save=True)
+        ctx.meta = meta
         return out
 
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, dout):
-        meta, pk, sel, cat = ctx.meta, ctx.pk, ctx.sel, ctx.cat
+        meta = ctx.meta
+        pk, sel, saved, cat = ctx.saved
         ad = meta["adapter"]
-        B, P, T, D = ctx.geom
+        T, B = cat.shape[:2]
+        P = saved["patch"][0].shape[1] // B
         dtype = cat.dtype
         E = ad.cross_attention_dim
         tw = _adapter_transposed(pk, dtype)
@@ -395,17 +298,18 @@ class _AdapterFn(torch.autograd.Function):
             g[(t, "cls", 6, "b")] = g[(t, "patch", 6, "b")] = db3
         dcat2 = dcat.view(T * B, 2 * HIDDEN)
         for branch in ("cls", "patch"):
-            x, h1, m1, r1, a1, h2, m2, r2 = ctx.saved[branch]
+            x, h1, m1, r1, a1, h2, m2, r2 = saved[branch]
             M = x.shape[1]
             if branch == "cls":
                 da2 = dcat2[:, :HIDDEN].contiguous()                                # [T*B, HIDDEN]
             else:
                 da2 = ops.group_mean_bwd(dcat2[:, HIDDEN:], P).view(T * M, HIDDEN)  # mean over patches, backwards
             dh2, dg2, dbe2 = ops.ln_lrelu_bwd(da2, h2.view(T * M, HIDDEN), m2, r2, pk[f"{branch}_g2"][sel].contiguous(),
-                                              pk[f"{branch}_be2"][sel].contiguous(), T, M)
+                                              pk[f"{branch}_be2"][sel].contiguous(), T, M, slope=LRELU_SLOPE)
             da1 = ops.linear(dh2.view(T, M, HIDDEN), tw[f"{branch}_w2_t"][sel])     # [T, M, HIDDEN]
             dh1, dg1, dbe1 = ops.ln_lrelu_bwd(da1.view(T * M, HIDDEN), h1.view(T * M, HIDDEN), m1, r1,
-                                              pk[f"{branch}_g1"][sel].contiguous(), pk[f"{branch}_be1"][sel].contiguous(), T, M)
+                                              pk[f"{branch}_g1"][sel].contiguous(), pk[f"{branch}_be1"][sel].contiguous(), T, M,
+                                              slope=LRELU_SLOPE)
             dh2v, dh1v = dh2.view(T, M, HIDDEN), dh1.view(T, M, HIDDEN)
             for t in range(T):
                 g[(t, branch, 3, "w")] = ops.linear_bwd_weight(dh2v[t], a1[t])

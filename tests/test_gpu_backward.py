@@ -279,6 +279,41 @@ def test_backward_is_deterministic(cuda_device):
         assert torch.equal(a, b)
 
 
+@pytest.mark.parametrize("p_drop", [0.0, 0.1], ids=["merged", "lora_dropout"])
+def test_backward_uses_the_weights_its_forward_ran_with(cuda_device, p_drop):
+    """A parameter changed in place between a training forward and its backward -- here to_k_ip, which is part of the
+    packed weights but not of the saved tensors -- re-packs the layer on the next call.  The pending backward must keep
+    the packed weights (and their transposed copies) of its own forward: its input gradients equal a fresh layer's."""
+    case = cases.ProcCase("repack", B=2, S=200, C=320, Li=5, lora_r=8, seed=85)
+
+    def run(change_between):
+        attn, proc = build_product_layer(case, cuda_device)
+        if p_drop:
+            for name in ("to_q", "to_k", "to_v"):
+                getattr(attn, name).lora_dropout["default"] = torch.nn.Dropout(p_drop)
+            attn.train()
+        for n, p in attn.named_parameters():
+            p.requires_grad_("lora_" in n or "to_k_ip" in n or "to_v_ip" in n)
+        assert proc.lora_dropout_active(attn) == (p_drop > 0)
+        x, text, img = (t.to(cuda_device, torch.bfloat16).requires_grad_(True)
+                        for t in cases.proc_inputs(case, torch.float32))
+        force_fusion_seed(1.0, 1.0)
+        torch.cuda.manual_seed(1000 + case.seed)
+        with torch.enable_grad():
+            y = attn(x, encoder_hidden_states=(text, img))
+            loss = y.float().square().sum() + proc.to_v_ip_norm.float().sum()
+            if change_between:
+                with torch.no_grad():
+                    proc.to_k_ip[0].weight.mul_(-2.0)
+                attn(x, encoder_hidden_states=(text, img))
+        loss.backward()
+        return y.detach(), x.grad, text.grad, img.grad
+
+    fresh, changed = run(False), run(True)
+    for name, a, b in zip(("y", "x", "text", "img"), fresh, changed):
+        assert torch.equal(a, b), name
+
+
 def test_tensor_core_backward_agrees_with_simt_backward(cuda_device):
     """bf16 training path: the mma.sync attention backward (pv_bwd_mma.cu, default) and the fp32-accumulating SIMT kernel
     (pv_set_option('bwd_mma', 0)) on identical inputs -- two independent implementations of reference :317-420's

@@ -9,7 +9,8 @@ and diffusers' ``Attention.forward`` can install and call it unchanged.  All ari
 Differences in *how* (not what) it computes, see DESIGN.md:
   * the two SDPA calls + add (:317-319, :400-402, :412) are one kernel: QK^T over the concatenated text+image keys,
     softmax normalised per segment, branch weights folded into P, one PV contraction;
-  * LoRA on to_q/to_k/to_v is merged into the packed bf16/fp16/fp32 weights on the GPU whenever a factor changes;
+  * LoRA on to_q/to_k/to_v and to_out[0] is merged into the packed bf16/fp16/fp32 weights on the GPU whenever a factor
+    changes;
   * float16 models run the bf16 tensor-core kernels with fp16 operands (inference only: grad mode raises);
   * under CUDA autocast, float32 hidden states compute in the autocast dtype like the reference's autocast'd Linears and
     SDPA (bf16 always, fp16 without grad; DESIGN.md 4.9): float32 activations are converted by a native kernel;
@@ -64,11 +65,12 @@ class PhotoVerseAttnProcessor(nn.Module):
 
 
 class _PackedWeights:
-    """Packed weights of one layer in one compute dtype.  Merged: LoRA folded into ``wq`` / ``wkv_text`` (W + s B A).
-    Unmerged (the LoRA-dropout training path): ``wq`` / ``wkv_text`` hold the base weights and the low-rank branch is a
-    K-extension of the base GEMM, ``[x | dropout(x) A^T] @ [W | s B]^T`` (``*_aug``, rank columns padded to 8)."""
+    """Packed weights of one layer in one compute dtype.  Merged: LoRA folded into ``wq`` / ``wkv_text`` / ``wo``
+    (W + s B A).  Unmerged (the LoRA-dropout training path): ``wq`` / ``wkv_text`` / ``wo`` hold the base weights and the
+    low-rank branch is a K-extension of the base GEMM, ``[x | dropout(x) A^T] @ [W | s B]^T`` (``*_aug``, rank columns
+    padded to 8)."""
     __slots__ = ("key", "wq", "wkv_text", "wkv_img", "wo", "bo", "_t",
-                 "wq_aug", "wkv_text_aug", "wkv_img_aug", "ranks", "eye")
+                 "wq_aug", "wkv_text_aug", "wkv_img_aug", "wo_aug", "ranks", "eye")
 
 
 def _pad8(n: int) -> int:
@@ -123,25 +125,26 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
         """Packed weights of this layer in the compute dtype: LoRA merged (W + s B A), or with ``merged=False`` the base
         weights plus the K-extended operands of the LoRA-dropout path.  Each of the four operands is re-packed only when
         one of ITS OWN sources changed (parameter version counters): in training the optimizer touches the LoRA factors
-        and to_k_ip / to_v_ip every step, the frozen out projection never."""
+        and to_k_ip / to_v_ip every step, the out projection only when it carries LoRA."""
         wq, qa, qb, qs, qp = linear_parts(attn.to_q)
         wk, ka, kb, ks, kp = linear_parts(attn.to_k)
         wv, va, vb, vs, vp = linear_parts(attn.to_v)
-        if merged and max(qp, kp, vp) > 0.0:
+        wo, oa, ob, os_, op = linear_parts(attn.to_out[0])
+        if merged and max(qp, kp, vp, op) > 0.0:
             raise RuntimeError("internal: merged weights requested while LoRA dropout is active")
-        wo, bo = attn.to_out[0].weight, attn.to_out[0].bias
+        bo = attn.to_out[0].bias
         kip, vip = self.to_k_ip[0].weight, self.to_v_ip[0].weight
 
         def vkey(tensors, *scal):
             return tuple((t.data_ptr(), t._version) if t is not None else None for t in tensors) + scal
 
         keys = {"wq": vkey([wq, qa, qb], qs), "wkv_text": vkey([wk, ka, kb, wv, va, vb], ks, vs),
-                "wkv_img": vkey([kip, vip]), "wo": vkey([wo, bo])}
+                "wkv_img": vkey([kip, vip]), "wo": vkey([wo, bo, oa, ob], os_)}
         pk = self._packed.get((dtype, merged))
         if pk is not None and pk.key == keys:
             return pk
         C, Dc = wq.shape[0], wk.shape[1]
-        for t in (wq, qa, qb, wk, ka, kb, wv, va, vb, wo, bo, kip, vip):
+        for t in (wq, qa, qb, wk, ka, kb, wv, va, vb, wo, oa, ob, bo, kip, vip):
             if t is not None and not t.is_cuda:
                 raise RuntimeError(f"photoverse_b200 needs its weights on the CUDA device (got {t.device})")
 
@@ -181,13 +184,15 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
                 ops.pack_weight(m(vip), pk.wkv_img[C:])
                 pk._t.pop("wkv_img_t", None)
             if "wo" in fresh:
-                pk.wo = ops.pack_weight(m(wo), torch.empty(C, C, device=device, dtype=dtype))
+                pk.wo = ops.pack_weight(m(wo), torch.empty(C, C, device=device, dtype=dtype), *lora(oa, ob, os_))
                 pk.bo = m(bo) if bo is not None else torch.zeros(C, device=device, dtype=torch.float32)
                 pk._t.pop("wo_t", None)
             if not merged:
-                pk.ranks = rq, rk, rv = tuple(0 if a is None else _pad8(a.shape[0]) for a in (qa, ka, va))
+                pk.ranks = rq, rk, rv, ro = tuple(0 if a is None else _pad8(a.shape[0]) for a in (qa, ka, va, oa))
                 if "wq" in fresh:
                     pk.wq_aug = torch.cat([pk.wq, sb(qb, qs, rq)], 1).contiguous() if rq else pk.wq
+                if "wo" in fresh:
+                    pk.wo_aug = torch.cat([pk.wo, sb(ob, os_, ro)], 1).contiguous() if ro else pk.wo
                 if fresh & {"wkv_text", "wkv_img"}:
                     if rk or rv:       # K/V of the text branch with their low-rank columns, image branch zero-extended
                         ext = torch.zeros(2 * C, rk + rv, device=device, dtype=dtype)
@@ -208,7 +213,7 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
     def lora_dropout_active(self, attn) -> bool:
         """True when a LoRA-wrapped projection of ``attn`` is in training mode with dropout p > 0 (peft applies
         ``lora_dropout`` to the low-rank branch input only; train.py:264-269, 348-354)."""
-        return any(linear_parts(m)[4] > 0.0 for m in (attn.to_q, attn.to_k, attn.to_v))
+        return any(linear_parts(m)[4] > 0.0 for m in (attn.to_q, attn.to_k, attn.to_v, attn.to_out[0]))
 
     def _fusion_weights(self):
         """(w_text, w_image) -- reference attention_processor.py:411-420, including its RNG draw."""

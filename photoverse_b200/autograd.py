@@ -3,10 +3,11 @@
 Reference semantics (train.py:495-538): gradients reach
   * the two adapters (every Linear / LayerNorm parameter),
   * ``to_k_ip`` / ``to_v_ip`` of the 16 processors (train.py:366-370),
-  * the LoRA factors on ``attn2.to_q / to_k / to_v`` (train.py:348-354; peft: ``y = W x + scaling * B(A(x))``),
+  * the LoRA factors on ``attn2.to_q / to_k / to_v`` (train.py:348-354; peft: ``y = W x + scaling * B(A(x))``), and on
+    ``attn2.to_out.0`` when it is a LoRA target too (the usual diffusers target set; the reference trains q/k/v only),
 and flow through ``hidden_states`` / ``encoder_hidden_states`` into the rest of the (frozen) UNet, the text encoder and
-the adapters.  The base projections and ``to_out`` are frozen in every reference configuration; asking for their
-gradients raises.
+the adapters.  The base projections and the base ``to_out`` weight and bias are frozen in every reference configuration;
+asking for their gradients raises.
 
 PyTorch is used for tensor ownership and autograd bookkeeping only: every contraction, reduction and elementwise
 derivative below is a C-ABI call (photoverse_b200/csrc/pv_bwd.cu + the tcgen05 GEMM).
@@ -62,18 +63,20 @@ def convert(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
 
 
 class _DualAttnFn(torch.autograd.Function):
-    """inputs: x, text, img, to_k_ip.w, to_v_ip.w, (A, B) of to_q, to_k, to_v (None when not injected), ctx object.
-    LoRA is merged into the packed weights and the Q projection runs inside the attention kernel."""
+    """inputs: x, text, img, to_k_ip.w, to_v_ip.w, (A, B) of to_q, to_k, to_v, to_out[0] (None when not injected), ctx
+    object.  LoRA is merged into the packed weights and the Q projection runs inside the attention kernel."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda")
-    def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, meta):
+    def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, oA, oB, meta):
         proc, attn = meta["proc"], meta["attn"]
         pk = proc._weights(attn, x.dtype, x.device)
         kv = ops.kv_pack(text, img, pk.wkv_text, pk.wkv_img, attn.heads)
         y, o, stats, q = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, meta["w_text"], meta["w_img"], want_stats=True)
-        # fp32 mode keeps Q; the bf16 kernel never writes it (q is None: recomputed in backward)
-        _save(ctx, meta, pk, kv, stats, q, (x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB))
+        # fp32 mode keeps Q; the bf16 kernel never writes it (q is None: recomputed in backward).  O, the input of
+        # to_out, is kept only for the gradients of a LoRA on to_out.
+        _save(ctx, meta, pk, kv, stats, q, o if oA is not None else None,
+              (x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, oA, oB))
         return y, kv.v_ip_norm.clone()
 
     @staticmethod
@@ -81,23 +84,29 @@ class _DualAttnFn(torch.autograd.Function):
     def backward(ctx, dy, dvn):
         meta, pk = ctx.meta, ctx.pk
         Lt, Li, H = ctx.dims
-        x, text, img, stats, kv_text, kv_img, v_ip_norm, q, *rest = ctx.saved_tensors
-        lora, drop = rest[:6], rest[6:]          # drop: dropout(x) of to_q / to_k / to_v, then their keep-masks
+        x, text, img, stats, kv_text, kv_img, v_ip_norm, q, o, *rest = ctx.saved_tensors
+        lora, drop = rest[:8], rest[8:]     # drop: dropout(input) of to_q / to_k / to_v / to_out, then their keep-masks
         dtype = x.dtype
         B, S, C = x.shape
         Dc = text.shape[2]
         x2, text2, img2 = x.view(B * S, C), text.view(B * Lt, Dc), img.view(B * Li, Dc)
         tw = _transposed(pk)
+        need = ctx.needs_input_grad
+        grads = [None] * 8
 
         dy2 = dy.contiguous().view(B * S, C).to(dtype)
         d_o = ops.linear(dy2, tw["wo_t"]).view(B, S, C)                                  # dO = dY Wo
+        if lora[6] is not None:
+            # LoRA on to_out: its factors from (O or dropout(O), dY); with dropout, the branch's share of dO before the
+            # attention backward reads it.  The fusion rule never drops to_out.
+            grads[6:8] = _lora_grads(o if o is None else o.view(B * S, C), dy2, d_o.view(B * S, C), True, lora[6], lora[7], meta["scal"][3], need[11],
+                                     need[12], (drop[3], drop[7], meta["drop"][3]) if drop else None)
         if q is None:
             q = ops.linear(x2, pk.wq).view(B, S, C)                                      # recompute Q = X Wq^T
         d_vn = dvn if (dvn is not None and meta["vnorm_grad"]) else None
         dq, dkv_text, dkv_img = ops.dual_attn_bwd(d_o, q, kv_text, kv_img, stats, v_ip_norm, d_vn, H, Lt, Li,
                                                   meta["w_text"], meta["w_img"])
         dq2 = dq.view(B * S, C)
-        need = ctx.needs_input_grad
         dx = ops.linear(dq2, tw["wq_t"]) if need[0] else None                            # dX = dQ Wq (base weights)
         dtext = ops.linear(dkv_text, tw["wkv_text_t"]) if need[1] else None
         dimg = ops.linear(dkv_img, tw["wkv_img_t"]).view(B, Li, Dc) if need[2] else None
@@ -107,44 +116,13 @@ class _DualAttnFn(torch.autograd.Function):
             dkv_w = ops.linear_bwd_weight(dkv_img, img2)                     # [2C, Dc]
             dkip = dkv_w[:C] if need[3] else None
             dvip = dkv_w[C:] if need[4] else None
-        # LoRA factors: y = W x + s B (A x)  ->  dB = s dY^T (x A^T),  dA = s (dY B)^T x
-        grads = [None] * 6
         srcs = ((x2, dq2, dx, need[0]), (text2, dkv_text[:, :C], dtext, need[1]), (text2, dkv_text[:, C:], dtext, need[1]))
         for j, (inp, g, dinp, need_inp) in enumerate(srcs):
-            A, Bm = lora[2 * j], lora[2 * j + 1]
-            if A is None:
-                continue
-            s, need_a, need_b = meta["scal"][j], need[5 + 2 * j], need[5 + 2 * j + 1]
-            if not drop:
-                if j > 0 and meta["w_text"] == 0.0:
-                    continue                                                 # text branch dropped: no gradient (see below)
-                if need_a and need_b:
-                    fused = ops.lora_bwd(inp, g, A, Bm, s)                   # both factors, one pass over x and dY (rank <= 16)
-                    if fused is not None:
-                        grads[2 * j:2 * j + 2] = fused
-                        continue
-            else:
-                inp = drop[j]                                                # dropout(x): what the branch saw
-            a_c = A.detach().to(dtype).contiguous()                          # [r, in]
-            bt_c = ops.transpose(Bm.detach().to(dtype).contiguous())         # [r, out]
-            if need_b:
-                t = _skinny_linear(inp, a_c)                                 # x A^T            [M, r]
-                grads[2 * j + 1] = ops.linear_bwd_weight(g, t, alpha=s)      # dB [out, r]
-            grad_inp = bool(drop) and need_inp
-            if need_a or grad_inp:
-                ub = _skinny_linear(g, bt_c, full=grad_inp)                  # dY B             [M, r] (padded: pad8(r))
-                r = a_c.shape[0]
-                if need_a:
-                    grads[2 * j] = ops.linear_bwd_weight(ub[:, :r], inp, alpha=s)        # dA [r, in]
-                if grad_inp:
-                    # d dropout(x) = s (dY B) A, then through the mask:  d x += keep / (1 - p) * that
-                    at8 = ops.transpose(_pad_rows8(a_c * s))                 # [in, pad8(r)]
-                    v = ops.linear(ub, at8)                                  # [M, in]
-                    mask = drop[3 + j]
-                    if mask is not None:
-                        ops.dropout_bwd_acc(dinp, v, mask, meta["drop"][j])
-                    else:
-                        ops.dropout_bwd_acc(dinp, v, torch.ones_like(v, dtype=torch.bool), 0.0)
+            if lora[2 * j] is None or (j > 0 and not drop and meta["w_text"] == 0.0):
+                continue                                                     # text branch dropped: no gradient (see below)
+            grads[2 * j:2 * j + 2] = _lora_grads(inp, g, dinp, need_inp, lora[2 * j], lora[2 * j + 1], meta["scal"][j],
+                                                 need[5 + 2 * j], need[6 + 2 * j],
+                                                 (drop[j], drop[4 + j], meta["drop"][j]) if drop else None)
         dx = None if dx is None else dx.view(B, S, C)
         dtext = None if dtext is None else dtext.view(B, Lt, Dc)
         # A branch the fusion rule dropped (attention_processor.py:413-418) is not part of the reference's graph: its
@@ -163,24 +141,26 @@ class _DualAttnFn(torch.autograd.Function):
 class _DualAttnDropoutFn(_DualAttnFn):
     """Training step with LoRA dropout p > 0 (the reference default, train.py:264-269): peft's
     ``W x + s B A dropout(x)`` cannot be merged into one weight, so the low-rank branch rides along as a K-extension of
-    the projection GEMMs: ``Q = [x | dropout(x) A^T] [W | s B]^T`` (same for K_text / V_text, each with its own mask).
+    the projection GEMMs: ``Q = [x | dropout(x) A^T] [W | s B]^T`` (same for K_text / V_text and the out projection
+    ``Y = [O | dropout(O) A_o^T] [Wo | s B_o]^T + bo``, each with its own mask).
 
     The keep-masks come from ``torch.native_dropout`` -- the kernel ``nn.Dropout`` dispatches to -- drawn in the
-    reference's order (to_q, to_k, to_v; attention_processor.py:297, 304-305) on same-shaped tensors, so a seeded run
-    consumes the CUDA Philox stream exactly like the reference.  Everything downstream of the masks is C-ABI calls.
+    reference's order (to_q, to_k, to_v, then to_out after the attention; attention_processor.py:297, 304-305, 423) on
+    same-shaped tensors, so a seeded run consumes the CUDA Philox stream exactly like the reference.  Everything
+    downstream of the masks is C-ABI calls.
     The backward is :class:`_DualAttnFn`'s, with the LoRA factors' gradients taken from dropout(x) and the low-rank
     branch's input gradient added through the keep-masks."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda")
-    def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, meta):
+    def forward(ctx, x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, oA, oB, meta):
         proc, attn = meta["proc"], meta["attn"]
         dtype, dev = x.dtype, x.device
         u = proc._weights(attn, dtype, dev, merged=False)
         B, S, C = x.shape
         Lt, Li, Dc = text.shape[1], img.shape[1], text.shape[2]
-        rq, rk, rv = u.ranks
-        pq, pk_, pv = meta["drop"]
+        rq, rk, rv, ro = u.ranks
+        pq, pk_, pv, po = meta["drop"]
         x2, text2 = x.view(B * S, C), text.view(B * Lt, Dc)
 
         def drop(t, p, has):
@@ -218,19 +198,67 @@ class _DualAttnDropoutFn(_DualAttnFn):
             ta, ia = text, img
         kv = ops.kv_pack(ta, ia, u.wkv_text_aug, u.wkv_img_aug, attn.heads)
         o, stats = ops.dual_attn_core(q, u.eye, kv, meta["w_text"], meta["w_img"], want_stats=True)
-        y = ops.linear(o.view(B * S, C), u.wo, u.bo).view(B, S, C)
-        _save(ctx, meta, u, kv, stats, q, (x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB),
-              (xd_q, xd_k, xd_v, m_q, m_k, m_v))
+        o2 = o.view(B * S, C)
+        od, m_o = drop(o2, po, oA is not None)           # drawn after the q / k / v masks, where the reference calls to_out
+        # Y = [O | od A_o^T] [Wo | s B_o]^T + bo
+        if ro:
+            oa = torch.empty(B * S, C + ro, device=dev, dtype=dtype)
+            oa[:, :C] = o2
+            if oA.shape[0] % 8:
+                oa[:, C + oA.shape[0]:].zero_()      # rank padding: fp32 rows of a rank-4 product end on a 16-byte boundary
+            ops.linear(od, _pad_rows8(oA.detach().to(dtype)), out=oa[:, C:])
+            y = ops.linear(oa, u.wo_aug, u.bo).view(B, S, C)
+            del oa
+        else:
+            y = ops.linear(o2, u.wo, u.bo).view(B, S, C)
+        _save(ctx, meta, u, kv, stats, q, None, (x, text, img, w_kip, w_vip, qA, qB, kA, kB, vA, vB, oA, oB),
+              (xd_q, xd_k, xd_v, od, m_q, m_k, m_v, m_o))
         return y, kv.v_ip_norm.clone()
 
 
-def _save(ctx, meta, pk, kv, stats, q, inputs, drop=()):
+def _lora_grads(inp, g, dinp, need_inp, A, Bm, s, need_a, need_b, drop=None):
+    """(dA, dB) of one LoRA-wrapped projection ``y = W inp + s B A inp`` from its input ``inp`` and ``g`` = dL/dy:
+    dB = s g^T (inp A^T), dA = s (g B)^T inp.  ``drop`` = (dropout(inp), keep-mask or None, p) on the LoRA-dropout path:
+    the factors see dropout(inp), and the branch's input gradient keep / (1 - p) * s (g B) A is added to ``dinp``."""
+    dtype = g.dtype
+    if drop is None:
+        if need_a and need_b:
+            fused = ops.lora_bwd(inp, g, A, Bm, s)                           # both factors, one pass over x and dY (rank <= 16)
+            if fused is not None:
+                return fused
+    else:
+        inp = drop[0]                                                        # dropout(x): what the branch saw
+    dA = dB = None
+    a_c = A.detach().to(dtype).contiguous()                                  # [r, in]
+    bt_c = ops.transpose(Bm.detach().to(dtype).contiguous())                 # [r, out]
+    if need_b:
+        t = _skinny_linear(inp, a_c)                                         # x A^T            [M, r]
+        dB = ops.linear_bwd_weight(g, t, alpha=s)                            # dB [out, r]
+    grad_inp = drop is not None and need_inp
+    if need_a or grad_inp:
+        ub = _skinny_linear(g, bt_c, full=grad_inp)                          # dY B             [M, r] (padded: pad8(r))
+        r = a_c.shape[0]
+        if need_a:
+            dA = ops.linear_bwd_weight(ub[:, :r], inp, alpha=s)              # dA [r, in]
+        if grad_inp:
+            # d dropout(x) = s (dY B) A, then through the mask:  d x += keep / (1 - p) * that
+            at8 = ops.transpose(_pad_rows8(a_c * s))                         # [in, pad8(r)]
+            v = ops.linear(ub, at8)                                          # [M, in]
+            mask, p = drop[1], drop[2]
+            if mask is not None:
+                ops.dropout_bwd_acc(dinp, v, mask, p)
+            else:
+                ops.dropout_bwd_acc(dinp, v, torch.ones_like(v, dtype=torch.bool), 0.0)
+    return dA, dB
+
+
+def _save(ctx, meta, pk, kv, stats, q, o, inputs, drop=()):
     """What :meth:`_DualAttnFn.backward` reads: the pack the forward ran with (a re-pack makes a new object, so later
     parameter updates do not reach this backward), the saved tensors and the parameter dtypes of the gradients."""
     x, text, img, w_kip, w_vip, *lora = inputs
     ctx.meta, ctx.pk = meta, pk
     ctx.dims = (text.shape[1], img.shape[1], kv.H)
-    ctx.save_for_backward(x, text, img, stats, kv.kv_text, kv.kv_img, kv.v_ip_norm, q, *lora, *drop)
+    ctx.save_for_backward(x, text, img, stats, kv.kv_text, kv.kv_img, kv.v_ip_norm, q, o, *lora, *drop)
     ctx.pdt = [None if t is None else t.dtype for t in (w_kip, w_vip, *lora)]
 
 
@@ -246,8 +274,8 @@ def _transposed(pk):
 
 def dual_attn_autograd(proc, attn, x, text, img, w_text, w_img):
     """Differentiable dual-branch attention: returns (Y [B,S,C], ||V_img|| [B,H,Li] fp32)."""
-    frozen = [attn.to_out[0].weight, attn.to_out[0].bias]
-    parts = [linear_parts(m) for m in (attn.to_q, attn.to_k, attn.to_v)]
+    frozen = [attn.to_out[0].bias]
+    parts = [linear_parts(m) for m in (attn.to_q, attn.to_k, attn.to_v, attn.to_out[0])]
     frozen += [p[0] for p in parts]
     if any(t is not None and t.requires_grad for t in frozen):
         raise NotImplementedError(

@@ -4,7 +4,9 @@ One ``torch.save`` dict:
     "image_adapter" / "text_adapter"   adapter state dicts (``mapping_{i}.{0,1,3,4,6}.{weight,bias}``)
     "cross_attention_adapter"          every unet key that contains "attn2" AND one of "processor", "to_q", "to_k",
                                        "to_v" -- i.e. ``...attn2.processor.to_k_ip.0.weight`` plus, with LoRA, the peft
-                                       keys ``...attn2.to_q.base_layer.weight / lora_A.default.weight / lora_B.default.weight``
+                                       keys ``...attn2.to_q.base_layer.weight / lora_A.default.weight / lora_B.default.weight``;
+                                       and the keys of ``attn2.to_out.0`` when it is LoRA-wrapped (``...attn2.to_out.0.
+                                       base_layer.weight / base_layer.bias / lora_A.default.weight / lora_B.default.weight``)
     "optimizer" (optional), "lora_config" (optional dict: r, lora_alpha, lora_dropout, target_modules)
 Files written by the reference load here (tests/test_host_logic.py::test_checkpoint_written_by_the_reference_loads:
 a file produced by the verbatim ``save_progress`` with a peft-0.10-shaped ``lora_config`` -- enum + set included) and
@@ -76,9 +78,14 @@ def read_checkpoint(path: str) -> dict:
 
 
 def cross_attention_state_dict(unet) -> dict:
+    """The reference's attn2 key filter (modeling_utils.py:29-50), plus a LoRA-wrapped ``attn2.to_out.0``: the reference
+    trains no out-projection LoRA, so its filter has no term for one, but a trained one must survive a save and load."""
+    out_lora = tuple(f"{name}." for name, m in unet.named_modules()
+                     if name.endswith("attn2.to_out.0") and hasattr(m, "base_layer") and hasattr(m, "lora_A"))
     out = {}
     for key, value in unet.state_dict().items():
-        if "attn2" in key and ("processor" in key or "to_q" in key or "to_k" in key or "to_v" in key):
+        if ("attn2" in key and ("processor" in key or "to_q" in key or "to_k" in key or "to_v" in key)) \
+                or key.startswith(out_lora):
             out[key] = value
     return out
 

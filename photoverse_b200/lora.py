@@ -1,13 +1,16 @@
 """LoRA on the cross-attention projections (reference: train.py:348-354, models/modeling_utils.py:86-88).
 
-The reference injects peft==0.10.0 ``lora.Linear`` wrappers into ``attn2.to_q / to_k / to_v``.  peft is not
+The reference injects peft==0.10.0 ``lora.Linear`` wrappers into ``attn2.to_q / to_k / to_v``; ``attn2.to_out.0`` (the
+usual diffusers target set adds it) is supported as a fourth target in inference and training.  peft is not
 installable here, so this module provides a wrapper with the SAME attribute layout and state-dict key names
 (``base_layer.weight``, ``lora_A.default.weight``, ``lora_B.default.weight``, ``scaling['default']``,
 ``lora_dropout.default``) so that reference checkpoints (modeling_utils.py:29-50) load unchanged, and the
 B200 processor reads the factors straight out of whichever wrapper (ours or real peft) it finds.
 
 The wrapper never does arithmetic on the hot path: the processor merges W + scaling*B*A inside
-``pv_pack_weight`` (CUDA) whenever a factor's version counter changes.
+``pv_pack_weight`` (CUDA) whenever a factor's version counter changes.  Only ``attn2`` modules can be targets: the host
+UNet runs ``attn1`` and the feed-forward layers as stock modules, which would call :meth:`LoraLinear.forward` (it
+raises), so write the targets with the ``attn2.`` prefix.
 """
 import math
 from typing import Iterable, Optional, Tuple

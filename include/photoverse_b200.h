@@ -21,10 +21,16 @@
  *        PV_F32   fp32 storage, fp32 FFMA arithmetic (parity mode: <= 1e-4 of the fp32 reference)
  *        PV_F16   fp16 storage, the PV_BF16 kernels with fp16 operands (kind::f16 MMAs, fp32 accumulation), for models
  *                 run in float16.  Inference only: pv_pack_weight, pv_linear_fwd, pv_kv_tile_bytes, pv_kv_pack_fwd,
- *                 pv_dual_attn_fwd, pv_dual_attn_core_fwd, pv_ln_lrelu_fwd and pv_group_mean_fwd accept it (wherever
+ *                 pv_dual_attn_fwd, pv_dual_attn_core_fwd, pv_dual_attn_masked_fwd, pv_dual_attn_masked_core_fwd,
+ *                 pv_ln_lrelu_fwd and pv_group_mean_fwd accept it (wherever
  *                 they say PV_BF16 below, the same holds for PV_F16); every other entry point returns PV_ERR_UNSUPPORTED.
  *                 Values are rounded to fp16 (to nearest) exactly where the PV_BF16 path rounds to bf16.
  *   - there is NO CPU fallback: without a CUDA device every compute entry point returns PV_ERR_CUDA
+ *   - img_row_weight (the *_masked_* entry points): fp32 [B,S] factor of each query row's image segment, the regional
+ *     identity mask of diffusers' `ip_adapter_masks` downsampled to the layer's query grid by pv_ip_mask_downsample.  The
+ *     image term of row s of sample b becomes w_img * img_row_weight[b,s] * softmax(Q K_i^T / sqrt(d)) V_i; the text term,
+ *     the saved statistics and the launch sequence are those of the unmasked call.  NULL selects the unmasked kernels;
+ *     an all-ones row weight gives results bit-identical to them.
  */
 #ifndef PHOTOVERSE_B200_H_
 #define PHOTOVERSE_B200_H_
@@ -131,6 +137,24 @@ int pv_dual_attn_core_fwd(pv_dtype dt, const void* XorQ, const void* Wq, const v
                           float* stats, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
                           void* stream);
 
+/* ---- regional identity masks (diffusers' `ip_adapter_masks`) ------------------------------------------------------
+ * pv_ip_mask_downsample: row_weight [B,S] fp32 from mask [mask_batch, mask_h, mask_w] fp32 (mask_batch 1 or B), by the
+ * rule of diffusers 0.27.2 IPAdapterMaskProcessor.downsample: grid mask_h' = int(sqrt(S / (mask_w / mask_h))) (+1 when
+ * it does not divide S) by mask_w' = S / mask_h', bicubic (A = -0.75, align_corners=False, no antialias, border-clamped
+ * taps, fp64 arithmetic), repeated to the batch, flattened row-major and zero-padded to S.  A mask with no such grid
+ * (mask_h' or mask_w' would be 0) returns PV_ERR_INVALID.  One launch.
+ * pv_dual_attn_masked_fwd / pv_dual_attn_masked_core_fwd: pv_dual_attn_fwd / pv_dual_attn_core_fwd with img_row_weight
+ * (see Conventions; dtypes, kernels, launch sequence and ws_sync protocol unchanged).                                  */
+int pv_ip_mask_downsample(const float* mask, int mask_batch, int mask_h, int mask_w, float* row_weight, int B, int S,
+                          void* stream);
+int pv_dual_attn_masked_fwd(pv_dtype dt, const void* X, const void* Wq, const void* Kp, const void* Vp, const void* Wo,
+                            const float* bo, void* Y, float* ws_q, void* ws_o, float* stats, unsigned int* ws_sync, int B,
+                            int S, int C, int H, int Lt, int Li, float w_text, float w_img, const float* img_row_weight,
+                            void* stream);
+int pv_dual_attn_masked_core_fwd(pv_dtype dt, const void* XorQ, const void* Wq, const void* Kp, const void* Vp, void* O,
+                                 float* stats, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
+                                 const float* img_row_weight, void* stream);
+
 /* ---- adapter epilogues (adapters.py:15-16,18-19: LayerNorm(1024) -> LeakyReLU(0.01)) ----------------
  * y = leaky_relu(layer_norm(x) * gamma + beta); x:[rows,cols] fp32 (row stride ldx), y:[rows,cols] out_dt
  * (row stride ldy; PV_F32, PV_BF16 or PV_F16); cols % 128 == 0, cols <= 4096.  Optional mean / rstd [rows] fp32 saved for backward.
@@ -199,6 +223,11 @@ int64_t pv_dual_attn_bwd_ws_bytes(int B, int S, int C, int H, int Lt, int Li);
 int pv_dual_attn_bwd(pv_dtype dt, const void* dO, const void* Q, const float* kv_text, const float* kv_img,
                      const float* stats, void* dQ, void* ws, int B, int S, int C, int H, int Lt, int Li, float w_text,
                      float w_img, void* stream);
+/* ... with the image keys of row s weighted w_img * img_row_weight[b,s] (NULL: pv_dual_attn_bwd).  The row weight gets no
+ * gradient; PV_F16 returns PV_ERR_UNSUPPORTED like every backward entry point.                                         */
+int pv_dual_attn_masked_bwd(pv_dtype dt, const void* dO, const void* Q, const float* kv_text, const float* kv_img,
+                            const float* stats, void* dQ, void* ws, int B, int S, int C, int H, int Lt, int Li,
+                            float w_text, float w_img, const float* img_row_weight, void* stream);
 int pv_kv_pack_bwd(pv_dtype dt, const void* ws, const float* kv_img, const float* v_ip_norm, const float* d_v_ip_norm,
                    void* dkv_text, void* dkv_img, int B, int S, int Lt, int Li, int C, int H, void* stream);
 

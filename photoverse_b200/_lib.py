@@ -34,6 +34,9 @@ _SIGNATURES = {
     "pv_dual_attn_sync_words": (c_int64, [c_int, c_int]),
     "pv_dual_attn_fwd": (c_int, [c_int] + [c_void_p] * 11 + [c_int] * 6 + [c_float, c_float, c_void_p]),
     "pv_dual_attn_core_fwd": (c_int, [c_int] + [c_void_p] * 6 + [c_int] * 6 + [c_float, c_float, c_void_p]),
+    "pv_ip_mask_downsample": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p]),
+    "pv_dual_attn_masked_fwd": (c_int, [c_int] + [c_void_p] * 11 + [c_int] * 6 + [c_float, c_float, c_void_p, c_void_p]),
+    "pv_dual_attn_masked_core_fwd": (c_int, [c_int] + [c_void_p] * 6 + [c_int] * 6 + [c_float, c_float, c_void_p, c_void_p]),
     "pv_ln_lrelu_fwd": (c_int, [c_int] + [c_void_p] * 6 + [c_int64, c_int, c_int64, c_int64, c_int64, c_float, c_float, c_void_p]),
     "pv_group_mean_fwd": (c_int, [c_int, c_int, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64, c_void_p]),
     "pv_inject_concept_fwd": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
@@ -60,6 +63,7 @@ _SIGNATURES = {
     "pv_group_mean_bwd": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64, c_void_p]),
     "pv_dual_attn_bwd_ws_bytes": (c_int64, [c_int] * 6),
     "pv_dual_attn_bwd": (c_int, [c_int] + [c_void_p] * 7 + [c_int] * 6 + [c_float, c_float, c_void_p]),
+    "pv_dual_attn_masked_bwd": (c_int, [c_int] + [c_void_p] * 7 + [c_int] * 6 + [c_float, c_float, c_void_p, c_void_p]),
     "pv_kv_pack_bwd": (c_int, [c_int] + [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
     "pv_group_norm_nhwc_ws_bytes": (c_int64, [c_int64, c_int64, c_int, c_int]),
     "pv_group_norm_nhwc_fwd": (c_int, [c_int] + [c_void_p] * 7 + [c_int64, c_int64, c_int, c_int, c_float, c_int, c_void_p]),

@@ -15,7 +15,9 @@ Differences in *how* (not what) it computes, see DESIGN.md:
   * under CUDA autocast, float32 hidden states compute in the autocast dtype like the reference's autocast'd Linears and
     SDPA (bf16 always, fp16 without grad; DESIGN.md 4.9): float32 activations are converted by a native kernel;
   * K/V projections can be cached across denoising steps (``kv_cache`` context) because
-    ``encoder_hidden_states`` is constant during generation (models/infer.py:89-98).
+    ``encoder_hidden_states`` is constant during generation (models/infer.py:89-98);
+  * ``ip_adapter_masks`` (diffusers' regional IP-adapter masks) are downsampled to each query grid by a native kernel,
+    cached, and folded into the attention kernels as a per-row factor of the image branch (DESIGN.md 4.10).
 """
 import copy
 from typing import Optional
@@ -27,6 +29,8 @@ from . import ops
 from .lora import linear_parts
 
 _SUPPORTED = (torch.bfloat16, torch.float16, torch.float32)
+# downsampled masks, shared by every processor: (mask storage, version, shape, dtype, device, B, S) -> fp32 [B, S]
+_MASK_ROWS = {}
 _F16_TRAINING = ("float16 runs the inference (no_grad) path only: training runs in bfloat16 or float32 "
                  "(cast the model, or run the forward under torch.no_grad() without LoRA dropout)")
 
@@ -253,9 +257,10 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
                 encoder_hidden_states[:, :end_pos, :], [encoder_hidden_states[:, end_pos:, :]])
         if len(ip_hidden_states) != 1 or len(self.to_k_ip) != 1:
             raise NotImplementedError("PhotoVerse installs exactly one image adapter per layer (models/unet.py:29-33)")
+        mask = _check_ip_masks(ip_adapter_masks, len(self.scale), len(ip_hidden_states), hidden_states.shape[0])
         # ---- features of diffusers' Attention that are inactive for SD-1.5 attn2: refuse, never fall back ----
-        if attention_mask is not None or ip_adapter_masks is not None:
-            raise NotImplementedError("attention_mask / ip_adapter_masks are never passed on the PhotoVerse path")
+        if attention_mask is not None:
+            raise NotImplementedError("attention_mask is never passed on the PhotoVerse path")
         if hidden_states.ndim != 3:
             raise NotImplementedError("only [B, S, C] hidden states (SD-1.5 attn2) are supported")
         if getattr(attn, "spatial_norm", None) is not None or getattr(attn, "group_norm", None) is not None \
@@ -270,6 +275,7 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
 
         dev = hidden_states.device
         text_in, img_in = encoder_hidden_states, ip_hidden_states[0]
+        rw = None if mask is None else _mask_rows(mask, hidden_states.shape[0], hidden_states.shape[1], dev)
         w_text, w_img = self._fusion_weights()
         self.last_fusion = (w_text, w_img)
 
@@ -286,7 +292,7 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
                 raise NotImplementedError(_F16_TRAINING)
             from .autograd import dual_attn_autograd
             x, text, img = (_cast(t, dtype, autocast, True) for t in (hidden_states, text_in, img_in))
-            y, vnorm = dual_attn_autograd(self, attn, x, text, img, w_text, w_img)
+            y, vnorm = dual_attn_autograd(self, attn, x, text, img, w_text, w_img, rw)
             # side output (:397): [B, H, Li, 1] in the activation dtype, float32 under autocast (torch.norm's autocast dtype)
             self.to_v_ip_norm = (vnorm if autocast else vnorm.to(dtype)).unsqueeze(-1)
             return y
@@ -304,10 +310,66 @@ class PhotoVerseAttnProcessor2_0(PhotoVerseAttnProcessor):
             if self._kv_cache is not None:
                 kv._keepalive = (text_in, img_in)      # pin the storage so the data_ptr key cannot be recycled
                 self._kv_cache[ck] = kv
-        y, _, _, _ = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, w_text, w_img)
+        y, _, _, _ = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, w_text, w_img, img_row_weight=rw)
         # side output (:397): [B, H, Li, 1] in the activation dtype, float32 under autocast
         self.to_v_ip_norm = kv.v_ip_norm.unsqueeze(-1) if autocast else kv.vnorm_act
         return y
+
+
+def _check_ip_masks(ip_adapter_masks, n_scale: int, n_images: int, batch: int) -> Optional[torch.Tensor]:
+    """diffusers' validation of ``ip_adapter_masks`` (IPAdapterAttnProcessor2_0): a list with one 4-D tensor
+    [1 or B, num_images, H, W] per adapter, or a tensor that becomes that list through ``list(masks.unsqueeze(1))``.
+    Returns the adapter's mask or None.  Runs before any CUDA work."""
+    if ip_adapter_masks is None:
+        return None
+    if isinstance(ip_adapter_masks, torch.Tensor):
+        ip_adapter_masks = list(ip_adapter_masks.unsqueeze(1))
+    if not isinstance(ip_adapter_masks, (list, tuple)) or not (len(ip_adapter_masks) == n_scale == n_images):
+        n = len(ip_adapter_masks) if isinstance(ip_adapter_masks, (list, tuple)) else type(ip_adapter_masks).__name__
+        raise ValueError(f"Length of ip_adapter_masks array ({n}) must match length of self.scale array ({n_scale}) "
+                         f"and number of ip_hidden_states ({n_images})")
+    mask = ip_adapter_masks[0]
+    if not isinstance(mask, torch.Tensor) or mask.ndim != 4:
+        raise ValueError("Each element of the ip_adapter_masks array should be a tensor with shape "
+                         "[1, num_images_for_ip_adapter, height, width]. Please use `IPAdapterMaskProcessor` to "
+                         "preprocess your mask")
+    if mask.shape[1] > 1:
+        raise NotImplementedError(
+            f"ip_adapter_masks with {mask.shape[1]} images per adapter: several images per adapter, each with its own "
+            "softmax segment, are not supported (PhotoVerse conditions each adapter on one image)")
+    if mask.shape[1] != 1:
+        raise ValueError(f"Number of masks ({mask.shape[1]}) does not match number of ip images (1) at index 0")
+    if mask.shape[0] not in (1, batch):
+        raise ValueError(f"ip_adapter_masks: the mask batch ({mask.shape[0]}) must be 1 or the batch of the hidden "
+                         f"states ({batch})")
+    if not mask.is_floating_point():
+        raise TypeError(f"ip_adapter_masks must be a floating-point tensor, got {mask.dtype}")
+    return mask
+
+
+def _mask_rows(mask: torch.Tensor, B: int, S: int, device) -> torch.Tensor:
+    """The fp32 [B, S] row weights of ``mask`` [1|B, 1, H, W] on a query grid of S rows, computed once per (mask
+    storage, version, S, B) by the native downsample kernel and shared by every processor (four query grids per SD-1.5
+    UNet evaluation).  The entry keeps the mask alive, so its storage address cannot be reused while it is cached."""
+    key = (mask.data_ptr(), mask._version, tuple(mask.shape), mask.stride(), mask.dtype, mask.device, str(device), B, S)
+    hit = _MASK_ROWS.get(key)
+    if hit is not None:
+        return hit[1]
+    if len(_MASK_ROWS) >= 64:
+        _MASK_ROWS.clear()
+    m = mask[:, 0].to(device=device, dtype=torch.float32).contiguous()
+    rows = ops.ip_mask_rows(m, B, S)
+    _MASK_ROWS[key] = (mask, rows)
+    return rows
+
+
+def release_mask_rows(mask: torch.Tensor) -> list:
+    """Remove the cached row weights of ``mask``'s storage and return them.  A captured CUDA graph whose masked
+    processor calls must re-run the downsample on every replay (a static mask buffer refreshed between replays) calls
+    this before the capture, and keeps what it returns after it."""
+    ptr = mask.data_ptr()
+    keys = [k for k in _MASK_ROWS if k[0] == ptr]
+    return [_MASK_ROWS.pop(k)[1] for k in keys]
 
 
 def _cast(t: torch.Tensor, dtype: torch.dtype, autocast: bool, grad: bool) -> torch.Tensor:

@@ -72,7 +72,8 @@ class _DualAttnFn(torch.autograd.Function):
         proc, attn = meta["proc"], meta["attn"]
         pk = proc._weights(attn, x.dtype, x.device)
         kv = ops.kv_pack(text, img, pk.wkv_text, pk.wkv_img, attn.heads)
-        y, o, stats, q = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, meta["w_text"], meta["w_img"], want_stats=True)
+        y, o, stats, q = ops.dual_attn(x, pk.wq, kv, pk.wo, pk.bo, meta["w_text"], meta["w_img"], want_stats=True,
+                                       img_row_weight=meta["rw"])
         # fp32 mode keeps Q; the bf16 kernel never writes it (q is None: recomputed in backward).  O, the input of
         # to_out, is kept only for the gradients of a LoRA on to_out.
         _save(ctx, meta, pk, kv, stats, q, o if oA is not None else None,
@@ -105,7 +106,7 @@ class _DualAttnFn(torch.autograd.Function):
             q = ops.linear(x2, pk.wq).view(B, S, C)                                      # recompute Q = X Wq^T
         d_vn = dvn if (dvn is not None and meta["vnorm_grad"]) else None
         dq, dkv_text, dkv_img = ops.dual_attn_bwd(d_o, q, kv_text, kv_img, stats, v_ip_norm, d_vn, H, Lt, Li,
-                                                  meta["w_text"], meta["w_img"])
+                                                  meta["w_text"], meta["w_img"], meta["rw"])
         dq2 = dq.view(B * S, C)
         dx = ops.linear(dq2, tw["wq_t"]) if need[0] else None                            # dX = dQ Wq (base weights)
         dtext = ops.linear(dkv_text, tw["wkv_text_t"]) if need[1] else None
@@ -197,7 +198,8 @@ class _DualAttnDropoutFn(_DualAttnFn):
         else:
             ta, ia = text, img
         kv = ops.kv_pack(ta, ia, u.wkv_text_aug, u.wkv_img_aug, attn.heads)
-        o, stats = ops.dual_attn_core(q, u.eye, kv, meta["w_text"], meta["w_img"], want_stats=True)
+        o, stats = ops.dual_attn_core(q, u.eye, kv, meta["w_text"], meta["w_img"], want_stats=True,
+                                      img_row_weight=meta["rw"])
         o2 = o.view(B * S, C)
         od, m_o = drop(o2, po, oA is not None)           # drawn after the q / k / v masks, where the reference calls to_out
         # Y = [O | od A_o^T] [Wo | s B_o]^T + bo
@@ -272,8 +274,9 @@ def _transposed(pk):
     return tw
 
 
-def dual_attn_autograd(proc, attn, x, text, img, w_text, w_img):
-    """Differentiable dual-branch attention: returns (Y [B,S,C], ||V_img|| [B,H,Li] fp32)."""
+def dual_attn_autograd(proc, attn, x, text, img, w_text, w_img, img_row_weight=None):
+    """Differentiable dual-branch attention: returns (Y [B,S,C], ||V_img|| [B,H,Li] fp32).  ``img_row_weight``: fp32
+    [B, S] regional mask weights of the image branch (ops.ip_mask_rows; a constant: no gradient) or None."""
     frozen = [attn.to_out[0].bias]
     parts = [linear_parts(m) for m in (attn.to_q, attn.to_k, attn.to_v, attn.to_out[0])]
     frozen += [p[0] for p in parts]
@@ -282,7 +285,7 @@ def dual_attn_autograd(proc, attn, x, text, img, w_text, w_img):
             "gradients for the base attn2 projections / to_out are not part of the PhotoVerse training set "
             "(train.py:348-370 trains to_k_ip, to_v_ip and LoRA factors only)")
     meta = {"proc": proc, "attn": attn, "w_text": float(w_text), "w_img": float(w_img),
-            "scal": [p[3] for p in parts], "drop": [p[4] for p in parts], "vnorm_grad": True}
+            "scal": [p[3] for p in parts], "drop": [p[4] for p in parts], "vnorm_grad": True, "rw": img_row_weight}
     lora_args = []
     for p in parts:
         lora_args += [p[1], p[2]]

@@ -18,21 +18,23 @@ int gemm_bf16(const void* A, const void* W, const float* bias, void* D, bool out
 int gemm_f32(const float* A, const float* W, const float* bias, float* D, long long M, long long N, long long K,
              long long batch, long long lda, long long ldw, long long ldd, long long strideA, long long strideW,
              long long strideBias, long long strideD, cudaStream_t stream);
-// The tcgen05 launchers below take bf16 operands, or fp16 ones with f16 = true.
+// The tcgen05 launchers below take bf16 operands, or fp16 ones with f16 = true.  img_row_weight: optional [B, S] fp32
+// factor of each query row's image segment (ip_adapter_masks); nullptr runs the unmasked kernels.
 int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats,
                                    int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                                   cudaStream_t stream, bool f16);
+                                   cudaStream_t stream, bool f16, const float* img_row_weight);
 bool dual_attn_pair_roles_supported(int S, int C, int H);
 bool dual_attn_pair_roles_fused_supported(int S, int C, int H);
 int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats,
                                    int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
                                    cudaStream_t stream, const void* Wo, const float* bo, void* Y, unsigned int* sync,
-                                   bool f16);
+                                   bool f16, const float* img_row_weight);
 int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats, int B,
                              int S, int C, int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream,
-                             const void* Wo, const float* bo, void* Y, unsigned int* sync, bool f16);
+                             const void* Wo, const float* bo, void* Y, unsigned int* sync, bool f16,
+                             const float* img_row_weight);
 int dual_attn_core_f32(const float* Q, const float* Kp, const float* Vp, float* O, float* stats, int B, int S, int C,
-                       int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream);
+                       int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream, const float* img_row_weight);
 static int64_t attn_kv_tile_bytes(int d) { return static_cast<int64_t>(PV_KEYS_PAD) * ((d + 15) / 16 * 16) * 2; }
 int pack_weight(pv_dtype out_dt, const float* W, const float* A, const float* Bm, float scaling, void* out, int out_f,
                 int in_f, int r, cudaStream_t stream);
@@ -73,7 +75,7 @@ int lora_bwd(bool bf16, const void* X, const void* G, const float* A, const floa
 int attn_bwd_chunks_used(bool bf16, int S, int d);
 int dual_attn_bwd(bool bf16, const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats,
                   void* dQ, float* part, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                  cudaStream_t stream);
+                  cudaStream_t stream, const float* img_row_weight);
 int kv_pack_bwd(bool bf16, const float* part, const float* kv_img, const float* v_ip_norm, const float* d_vnorm,
                 void* dkv_text, void* dkv_img, int nchunk, int B, int Lt, int Li, int C, int H, cudaStream_t stream);
 
@@ -239,7 +241,7 @@ static inline bool is_16bit(pv_dtype dt) { return dt == PV_BF16 || dt == PV_F16;
 static int attn_core_bf16(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats, int B,
                           int S, int C, int H, int Lt, int Li, float w_text, float w_img, cudaStream_t st, bool f16,
                           const void* Wo = nullptr, const float* bo = nullptr, void* Y = nullptr, unsigned int* sync = nullptr,
-                          bool* fused = nullptr) {
+                          bool* fused = nullptr, const float* rw = nullptr) {
   if (fused) *fused = false;
   if (S > 128) {
     // Single launch where it pays: with G = C / 160 <= 2 column groups the pairs that share a row block run in lockstep and
@@ -250,13 +252,13 @@ static int attn_core_bf16(const void* X, const void* Wq, const void* Kp, const v
       const bool f = want && dual_attn_pair_roles_fused_supported(S, C, H);
       if (fused) *fused = f;
       return dual_attn_core_bf16_pair_roles(X, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, st,
-                                            f ? Wo : nullptr, bo, f ? Y : nullptr, f ? sync : nullptr, f16);
+                                            f ? Wo : nullptr, bo, f ? Y : nullptr, f ? sync : nullptr, f16, rw);
     }
     if (fused) *fused = want;
     return dual_attn_core_bf16_pair(X, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, st, want ? Wo : nullptr, bo,
-                                    want ? Y : nullptr, want ? sync : nullptr, f16);
+                                    want ? Y : nullptr, want ? sync : nullptr, f16, rw);
   }
-  return dual_attn_core_bf16_persistent(X, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, st, f16);
+  return dual_attn_core_bf16_persistent(X, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, st, f16, rw);
 }
 
 }  // namespace pv
@@ -366,13 +368,22 @@ int64_t pv_dual_attn_sync_words(int B, int S) {
 int pv_dual_attn_fwd(pv_dtype dt, const void* X, const void* Wq, const void* Kp, const void* Vp, const void* Wo,
                      const float* bo, void* Y, float* ws_q, void* ws_o, float* stats, unsigned int* ws_sync, int B, int S,
                      int C, int H, int Lt, int Li, float w_text, float w_img, void* stream) {
+  return pv_dual_attn_masked_fwd(dt, X, Wq, Kp, Vp, Wo, bo, Y, ws_q, ws_o, stats, ws_sync, B, S, C, H, Lt, Li, w_text,
+                                 w_img, nullptr, stream);
+}
+
+int pv_dual_attn_masked_fwd(pv_dtype dt, const void* X, const void* Wq, const void* Kp, const void* Vp, const void* Wo,
+                            const float* bo, void* Y, float* ws_q, void* ws_o, float* stats, unsigned int* ws_sync, int B,
+                            int S, int C, int H, int Lt, int Li, float w_text, float w_img, const float* img_row_weight,
+                            void* stream) {
   PV_REQUIRE(X && Wq && Kp && Vp && Wo && Y && ws_o, "null pointer");
   cudaStream_t st = as_stream(stream);
   int rc;
   if (is_16bit(dt)) {
     const bool f16 = dt == PV_F16;
     bool fused = false;
-    rc = attn_core_bf16(X, Wq, Kp, Vp, ws_o, stats, B, S, C, H, Lt, Li, w_text, w_img, st, f16, Wo, bo, Y, ws_sync, &fused);
+    rc = attn_core_bf16(X, Wq, Kp, Vp, ws_o, stats, B, S, C, H, Lt, Li, w_text, w_img, st, f16, Wo, bo, Y, ws_sync, &fused,
+                        img_row_weight);
     if (rc || fused) return rc;
     return gemm_bf16(ws_o, Wo, bo, Y, false, (long long)B * S, C, C, 1, C, C, C, 0, 0, 0, 0, st, /*w_static=*/true, f16);
   }
@@ -382,7 +393,7 @@ int pv_dual_attn_fwd(pv_dtype dt, const void* X, const void* Wq, const void* Kp,
                 C, C, 0, 0, 0, 0, st);
   if (rc) return rc;
   rc = dual_attn_core_f32(ws_q, static_cast<const float*>(Kp), static_cast<const float*>(Vp),
-                          static_cast<float*>(ws_o), stats, B, S, C, H, Lt, Li, w_text, w_img, st);
+                          static_cast<float*>(ws_o), stats, B, S, C, H, Lt, Li, w_text, w_img, st, img_row_weight);
   if (rc) return rc;
   return gemm_f32(static_cast<const float*>(ws_o), static_cast<const float*>(Wo), bo, static_cast<float*>(Y),
                   (long long)B * S, C, C, 1, C, C, C, 0, 0, 0, 0, st);
@@ -391,15 +402,22 @@ int pv_dual_attn_fwd(pv_dtype dt, const void* X, const void* Wq, const void* Kp,
 int pv_dual_attn_core_fwd(pv_dtype dt, const void* XorQ, const void* Wq, const void* Kp, const void* Vp, void* O,
                           float* stats, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
                           void* stream) {
+  return pv_dual_attn_masked_core_fwd(dt, XorQ, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, nullptr, stream);
+}
+
+int pv_dual_attn_masked_core_fwd(pv_dtype dt, const void* XorQ, const void* Wq, const void* Kp, const void* Vp, void* O,
+                                 float* stats, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
+                                 const float* img_row_weight, void* stream) {
   PV_REQUIRE(XorQ && Kp && Vp && O, "null pointer");
   if (is_16bit(dt)) {
     PV_REQUIRE(Wq != nullptr, "PV_BF16 / PV_F16 fuse the Q projection: Wq required");
-    return attn_core_bf16(XorQ, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, as_stream(stream), dt == PV_F16);
+    return attn_core_bf16(XorQ, Wq, Kp, Vp, O, stats, B, S, C, H, Lt, Li, w_text, w_img, as_stream(stream), dt == PV_F16,
+                          nullptr, nullptr, nullptr, nullptr, nullptr, img_row_weight);
   }
   PV_REQUIRE(dt == PV_F32, "unknown dtype %d", (int)dt);
   return dual_attn_core_f32(static_cast<const float*>(XorQ), static_cast<const float*>(Kp),
                             static_cast<const float*>(Vp), static_cast<float*>(O), stats, B, S, C, H, Lt, Li, w_text,
-                            w_img, as_stream(stream));
+                            w_img, as_stream(stream), img_row_weight);
 }
 
 int pv_ln_lrelu_fwd(pv_dtype out_dt, const float* x, const float* gamma, const float* beta, void* y, float* save_mean,
@@ -495,9 +513,17 @@ int pv_dual_attn_bwd(pv_dtype dt, const void* dO, const void* Q, const float* kv
                      const float* stats, void* dQ, void* ws, int B, int S, int C, int H, int Lt, int Li, float w_text,
                      float w_img, void* stream) {
   PV_NO_F16(dt);
+  return pv_dual_attn_masked_bwd(dt, dO, Q, kv_text, kv_img, stats, dQ, ws, B, S, C, H, Lt, Li, w_text, w_img, nullptr,
+                                 stream);
+}
+
+int pv_dual_attn_masked_bwd(pv_dtype dt, const void* dO, const void* Q, const float* kv_text, const float* kv_img,
+                            const float* stats, void* dQ, void* ws, int B, int S, int C, int H, int Lt, int Li, float w_text,
+                            float w_img, const float* img_row_weight, void* stream) {
+  PV_NO_F16(dt);
   PV_REQUIRE(dO && Q && kv_text && kv_img && stats && dQ && ws, "null pointer");
   return dual_attn_bwd(dt == PV_BF16, dO, Q, kv_text, kv_img, stats, dQ, static_cast<float*>(ws), B, S, C, H, Lt, Li, w_text,
-                       w_img, as_stream(stream));
+                       w_img, as_stream(stream), img_row_weight);
 }
 
 int pv_kv_pack_bwd(pv_dtype dt, const void* ws, const float* kv_img, const float* v_ip_norm, const float* d_v_ip_norm,

@@ -84,9 +84,10 @@ struct Attn3Params {
   float w_text, w_img, scale_log2e;
   unsigned long long* trace;   // optional [1 + 3*n] event buffer (CTA 0 only): count, then (event, index, clock) triples
   int trace_cap;
+  const float* img_row_weight; // MASK kernels: [B, S] fp32 factor of each query row's image segment (ip_adapter_masks)
 };
 
-template <int D, bool LT77, bool WSTAT, typename T>
+template <int D, bool LT77, bool WSTAT, typename T, bool MASK>
 __global__ void __launch_bounds__(A3_THREADS, 1)
 dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmWq,
                                 const __grid_constant__ CUtensorMap tmO, const Attn3Params p) {
@@ -450,6 +451,9 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
 
       const bool row_ok = (m0 + row) < p.S;
       bool had_head = false;
+      // image segment weight of this row: w_img, times the row's mask weight in the MASK kernels (w_img * 1 is exact)
+      float wi = p.w_img;
+      if constexpr (MASK) wi *= row_ok ? __ldg(p.img_row_weight + static_cast<size_t>(b) * p.S + m0 + row) : 0.f;
 
 #pragma unroll 1
       for (int j = 0; j < HPC; ++j) {
@@ -541,7 +545,7 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
         const float lt = (l0 + l1) + (l2 + l3);
         const float li = li0 + li1;
         const float at = p.w_text / lt;
-        const float ai = p.w_img / li;
+        const float ai = wi / li;
         if (p.stats != nullptr && row_ok) {
           const size_t idx = ((static_cast<size_t>(b) * p.H + (g * HPC + j)) * p.S + (m0 + row));
           reinterpret_cast<float4*>(p.stats)[idx] = make_float4(mts, lt, mis, li);
@@ -608,11 +612,11 @@ dual_attn_fwd_persistent_kernel(const __grid_constant__ CUtensorMap tmX, const _
 extern unsigned long long* g_attn3_trace;
 extern int g_attn3_trace_cap;
 
-template <int D, bool LT77, bool WSTAT, typename T>
+template <int D, bool LT77, bool WSTAT, typename T, bool MASK>
 static int launch_attn3(const CUtensorMap& tmX, const CUtensorMap& tmWq, const CUtensorMap& tmO, const Attn3Params& p,
                         cudaStream_t stream) {
   using Cfg = Attn3Cfg<D, WSTAT>;
-  auto kern = dual_attn_fwd_persistent_kernel<D, LT77, WSTAT, T>;
+  auto kern = dual_attn_fwd_persistent_kernel<D, LT77, WSTAT, T, MASK>;
   PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
   const long long sms = sm_count();
   const int grid = static_cast<int>(p.units < sms ? p.units : sms);
@@ -623,7 +627,7 @@ static int launch_attn3(const CUtensorMap& tmX, const CUtensorMap& tmWq, const C
 
 int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats,
                                    int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                                   cudaStream_t stream, bool f16) {
+                                   cudaStream_t stream, bool f16, const float* img_row_weight) {
   PV_REQUIRE(B > 0 && S > 0 && H > 0 && C % H == 0, "bad shape B=%d S=%d C=%d H=%d", B, S, C, H);
   const int d = C / H;
   PV_REQUIRE(d == 40 || d == 80 || d == 160, "head_dim %d unsupported (40/80/160)", d);
@@ -651,9 +655,12 @@ int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp
   p.trace = g_attn3_trace;
   p.trace_cap = g_attn3_trace_cap;
   p.scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(d));
-#define PV_A3_LAUNCH(DD, LT, WS)                                                                  \
-  (f16 ? launch_attn3<DD, LT, WS, __half>(tmX, tmWq, tmO, p, stream)                              \
-       : launch_attn3<DD, LT, WS, __nv_bfloat16>(tmX, tmWq, tmO, p, stream))
+  p.img_row_weight = img_row_weight;
+#define PV_A3_LAUNCH_M(DD, LT, WS, M)                                                             \
+  (f16 ? launch_attn3<DD, LT, WS, __half, M>(tmX, tmWq, tmO, p, stream)                           \
+       : launch_attn3<DD, LT, WS, __nv_bfloat16, M>(tmX, tmWq, tmO, p, stream))
+#define PV_A3_LAUNCH(DD, LT, WS) \
+  (img_row_weight ? PV_A3_LAUNCH_M(DD, LT, WS, true) : PV_A3_LAUNCH_M(DD, LT, WS, false))
   switch (d) {
     case 40:
       if (C == A3_KB_WSTAT * A3_BK) return Lt == 77 ? PV_A3_LAUNCH(40, true, true) : PV_A3_LAUNCH(40, false, true);
@@ -662,6 +669,7 @@ int dual_attn_core_bf16_persistent(const void* X, const void* Wq, const void* Kp
     default: return Lt == 77 ? PV_A3_LAUNCH(160, true, false) : PV_A3_LAUNCH(160, false, false);
   }
 #undef PV_A3_LAUNCH
+#undef PV_A3_LAUNCH_M
 }
 
 }  // namespace pv

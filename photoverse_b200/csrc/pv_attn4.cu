@@ -77,9 +77,10 @@ struct Attn4Params {
   // fused out projection (FUSE kernels only)
   const float* bias;           // [C] or nullptr
   unsigned int* sync;          // [2 * V] row-block counters, zero between launches (pv_outproj.cuh)
+  const float* img_row_weight; // MASK kernels: [B, S] fp32 factor of each query row's image segment (ip_adapter_masks)
 };
 
-template <int D, bool LT77, bool WSTAT, bool FUSE, typename T>
+template <int D, bool LT77, bool WSTAT, bool FUSE, typename T, bool MASK>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(A4_THREADS, 1)
 dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmWq,
                           const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmOa,
@@ -493,6 +494,9 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
 
       const bool row_ok = (m0 + row) < p.S;
       bool had_head = false;
+      // image segment weight of this row: w_img, times the row's mask weight in the MASK kernels (w_img * 1 is exact)
+      float wi = p.w_img;
+      if constexpr (MASK) wi *= row_ok ? __ldg(p.img_row_weight + static_cast<size_t>(b) * p.S + m0 + row) : 0.f;
 
 #pragma unroll 1
       for (int j = 0; j < HPC; ++j) {
@@ -584,7 +588,7 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
         const float lt = (l0 + l1) + (l2 + l3);
         const float li = li0 + li1;
         const float at = p.w_text / lt;
-        const float ai = p.w_img / li;
+        const float ai = wi / li;
         if (p.stats != nullptr && row_ok) {
           const size_t idx = ((static_cast<size_t>(b) * p.H + (g * HPC + j)) * p.S + (m0 + row));
           reinterpret_cast<float4*>(p.stats)[idx] = make_float4(mts, lt, mis, li);
@@ -695,12 +699,12 @@ dual_attn_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_
 extern unsigned long long* g_attn3_trace;
 extern int g_attn3_trace_cap;
 
-template <int D, bool LT77, bool WSTAT, bool FUSE, typename T>
+template <int D, bool LT77, bool WSTAT, bool FUSE, typename T, bool MASK>
 static int launch_attn4(const CUtensorMap& tmX, const CUtensorMap& tmWq, const CUtensorMap& tmO, const CUtensorMap& tmOa,
                         const CUtensorMap& tmWo, const CUtensorMap& tmY, const Attn4Params& p, long long unit_pairs,
                         cudaStream_t stream) {
   using Cfg = Attn4Cfg<D, WSTAT>;
-  auto kern = dual_attn_fwd_pair_kernel<D, LT77, WSTAT, FUSE, T>;
+  auto kern = dual_attn_fwd_pair_kernel<D, LT77, WSTAT, FUSE, T, MASK>;
   PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
   const long long max_pairs = sm_count() / 2;
   const int npairs = static_cast<int>(unit_pairs < max_pairs ? unit_pairs : max_pairs);
@@ -714,7 +718,8 @@ static int launch_attn4(const CUtensorMap& tmX, const CUtensorMap& tmWq, const C
 // (pv_outproj.cuh), O also left in global memory, `sync` = 2 * B * ceil(S / 256) zeroed counters (left zeroed).
 int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats, int B,
                              int S, int C, int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream,
-                             const void* Wo, const float* bo, void* Y, unsigned int* sync, bool f16) {
+                             const void* Wo, const float* bo, void* Y, unsigned int* sync, bool f16,
+                             const float* img_row_weight) {
   PV_REQUIRE(B > 0 && S > 0 && H > 0 && C % H == 0, "bad shape B=%d S=%d C=%d H=%d", B, S, C, H);
   const int d = C / H;
   PV_REQUIRE(d == 40 || d == 80 || d == 160, "head_dim %d unsupported (40/80/160)", d);
@@ -754,9 +759,12 @@ int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, cons
   p.scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(d));
   p.bias = bo;
   p.sync = sync;
-#define PV_A4_LAUNCH(DD, LT, WS, FU)                                                                          \
-  (f16 ? launch_attn4<DD, LT, WS, FU, __half>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)         \
-       : launch_attn4<DD, LT, WS, FU, __nv_bfloat16>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream))
+  p.img_row_weight = img_row_weight;
+#define PV_A4_LAUNCH_M(DD, LT, WS, FU, M)                                                                     \
+  (f16 ? launch_attn4<DD, LT, WS, FU, __half, M>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)      \
+       : launch_attn4<DD, LT, WS, FU, __nv_bfloat16, M>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream))
+#define PV_A4_LAUNCH(DD, LT, WS, FU) \
+  (img_row_weight ? PV_A4_LAUNCH_M(DD, LT, WS, FU, true) : PV_A4_LAUNCH_M(DD, LT, WS, FU, false))
 #define PV_A4_LT(DD, WS, FU) (Lt == 77 ? PV_A4_LAUNCH(DD, true, WS, FU) : PV_A4_LAUNCH(DD, false, WS, FU))
   switch (d) {
     case 40:
@@ -769,6 +777,7 @@ int dual_attn_core_bf16_pair(const void* X, const void* Wq, const void* Kp, cons
   }
 #undef PV_A4_LT
 #undef PV_A4_LAUNCH
+#undef PV_A4_LAUNCH_M
 }
 
 }  // namespace pv

@@ -90,9 +90,10 @@ struct Attn6Params {
   unsigned int* sync;      // [2 * V] row-block counters, zero between launches (pv_outproj.cuh)
   int prefetch_s;          // softmax warps fetch the next head's S row under the current head's P pack
   int mufu_token;          // d = 40: the two softmax groups take turns on the exponentials
+  const float* img_row_weight;   // MASK kernels: [B, S] fp32 factor of each query row's image segment (ip_adapter_masks)
 };
 
-template <int D, bool LT77, bool FUSE, typename T>
+template <int D, bool LT77, bool FUSE, typename T, bool MASK>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(A6_THREADS, 1)
 dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmWq,
                                 const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmOa,
@@ -453,6 +454,9 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
       const int mt = 2 * (u0 + i - b * p.MTP) + static_cast<int>(rank);
       const int m0 = mt * A6_BM;
       const bool row_ok = (m0 + row) < p.S;
+      // image segment weight of this row: w_img, times the row's mask weight in the MASK kernels (w_img * 1 is exact)
+      float wi = p.w_img;
+      if constexpr (MASK) wi *= row_ok ? __ldg(p.img_row_weight + static_cast<size_t>(b) * p.S + m0 + row) : 0.f;
 #pragma unroll 1
       for (int jj = 0; jj < A6_HPC / 2; ++jj) {
         const int j = wg + 2 * jj;                   // this group's heads of the unit
@@ -572,7 +576,7 @@ dual_attn_fwd_pair_roles_kernel(const __grid_constant__ CUtensorMap tmX, const _
           const float lt = (l0 + l1) + (l2 + l3);
           const float li = li0 + li1;
           const float at = __fdividef(p.w_text, lt);      // l >= 1 (the max term), far from the ranges where the fast
-          const float ai = __fdividef(p.w_img, li);       // division loses accuracy
+          const float ai = __fdividef(wi, li);            // division loses accuracy
           if (p.stats != nullptr && row_ok) {
             const size_t idx = ((static_cast<size_t>(b) * p.H + (g * A6_HPC + j)) * p.S + (m0 + row));
             reinterpret_cast<float4*>(p.stats)[idx] = make_float4(mts, lt, mis, li);
@@ -838,11 +842,11 @@ extern int g_opt_trace_block;
 extern int g_opt_attn6_prefetch;
 extern int g_opt_attn6_token;
 
-template <int D, bool LT77, bool FUSE, typename T>
+template <int D, bool LT77, bool FUSE, typename T, bool MASK>
 static int launch_attn6(const CUtensorMap& tmX, const CUtensorMap& tmWq, const CUtensorMap& tmO, const CUtensorMap& tmOa,
                         const CUtensorMap& tmWo, const CUtensorMap& tmY, const Attn6Params& p, long long unit_pairs,
                         cudaStream_t stream) {
-  auto kern = dual_attn_fwd_pair_roles_kernel<D, LT77, FUSE, T>;
+  auto kern = dual_attn_fwd_pair_roles_kernel<D, LT77, FUSE, T, MASK>;
   PV_CUDA(set_max_smem_once(kern, Attn6Cfg<D>::SMEM_BYTES));
   const long long max_pairs = sm_count() / 2;
   const int npairs = static_cast<int>(unit_pairs < max_pairs ? unit_pairs : max_pairs);
@@ -870,7 +874,7 @@ bool dual_attn_pair_roles_fused_supported(int S, int C, int H) {
 int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp, const void* Vp, void* O, float* stats,
                                    int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
                                    cudaStream_t stream, const void* Wo, const float* bo, void* Y, unsigned int* sync,
-                                   bool f16) {
+                                   bool f16, const float* img_row_weight) {
   PV_REQUIRE(B > 0 && dual_attn_pair_roles_supported(S, C, H), "needs head_dim 40 with C=320 or head_dim 80, S>128 (B=%d S=%d C=%d H=%d)",
              B, S, C, H);
   const bool fuse = Wo != nullptr;
@@ -913,9 +917,12 @@ int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp
   p.sync = sync;
   p.prefetch_s = g_opt_attn6_prefetch;
   p.mufu_token = g_opt_attn6_token;
-#define PV_A6_LAUNCH(DD, LT, FU)                                                                         \
-  (f16 ? launch_attn6<DD, LT, FU, __half>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)        \
-       : launch_attn6<DD, LT, FU, __nv_bfloat16>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream))
+  p.img_row_weight = img_row_weight;
+#define PV_A6_LAUNCH_M(DD, LT, FU, M)                                                                    \
+  (f16 ? launch_attn6<DD, LT, FU, __half, M>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream)     \
+       : launch_attn6<DD, LT, FU, __nv_bfloat16, M>(tmX, tmWq, tmO, tmOa, tmWo, tmY, p, unit_pairs, stream))
+#define PV_A6_LAUNCH(DD, LT, FU) \
+  (img_row_weight ? PV_A6_LAUNCH_M(DD, LT, FU, true) : PV_A6_LAUNCH_M(DD, LT, FU, false))
   if (d == 40) {
     if (fuse) return Lt == 77 ? PV_A6_LAUNCH(40, true, true) : PV_A6_LAUNCH(40, false, true);
     return Lt == 77 ? PV_A6_LAUNCH(40, true, false) : PV_A6_LAUNCH(40, false, false);
@@ -923,6 +930,7 @@ int dual_attn_core_bf16_pair_roles(const void* X, const void* Wq, const void* Kp
   if (fuse) return Lt == 77 ? PV_A6_LAUNCH(80, true, true) : PV_A6_LAUNCH(80, false, true);
   return Lt == 77 ? PV_A6_LAUNCH(80, true, false) : PV_A6_LAUNCH(80, false, false);
 #undef PV_A6_LAUNCH
+#undef PV_A6_LAUNCH_M
 }
 
 }  // namespace pv

@@ -420,12 +420,13 @@ constexpr int AB_TQ = 32;         // queries per tile
 constexpr int AB_CHUNK = 128;     // queries per block (== the row tile of the tensor-core kernel in pv_bwd_mma.cu)
 constexpr int AB_LP = PV_KEYS_PAD + 1;
 
-template <int D, typename T>
+// MASK: the image keys of query row s are weighted w_img * img_row_weight[b, s] (ip_adapter_masks)
+template <int D, typename T, bool MASK>
 __global__ void __launch_bounds__(256, 1)
 attn_bwd_kernel(const T* __restrict__ dO, const T* __restrict__ Q, const float* __restrict__ kv_text,
                 const float* __restrict__ kv_img, const float* __restrict__ stats, T* __restrict__ dQ,
                 float* __restrict__ part, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                float scale, float scale_log2e) {
+                float scale, float scale_log2e, const float* __restrict__ img_row_weight) {
   constexpr int DP = D + 1;
   constexpr int R = (PV_KEYS_PAD * D + 255) / 256;
   extern __shared__ float sm[];
@@ -475,6 +476,7 @@ attn_bwd_kernel(const T* __restrict__ dO, const T* __restrict__ Q, const float* 
         const float* dr = dos + rr * DP;
         float ph[3], dp[3];
         float delt = 0.f, deli = 0.f;
+        const float wi = MASK ? w_img * __ldg(img_row_weight + static_cast<size_t>(b) * S + srow) : w_img;
 #pragma unroll
         for (int t = 0; t < 3; ++t) {
           const int k = lane + 32 * t;
@@ -499,7 +501,7 @@ attn_bwd_kernel(const T* __restrict__ dO, const T* __restrict__ Q, const float* 
         for (int t = 0; t < 3; ++t) {
           const int k = lane + 32 * t;
           const bool is_t = k < Lt;
-          const float w = is_t ? w_text : w_img;
+          const float w = is_t ? w_text : wi;
           pw[t] = w * ph[t];
           dsv[t] = scale * w * ph[t] * (dp[t] - (is_t ? delt : deli));
         }
@@ -560,34 +562,35 @@ int attn_bwd_chunks_used(bool bf16, int S, int d) {
 template <int D, typename T>
 static int launch_attn_bwd(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats,
                            void* dQ, float* part, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                           cudaStream_t stream) {
-  auto kern = attn_bwd_kernel<D, T>;
+                           cudaStream_t stream, const float* img_row_weight) {
+  auto kern = img_row_weight ? attn_bwd_kernel<D, T, true> : attn_bwd_kernel<D, T, false>;
   const size_t smem = (2 * PV_KEYS_PAD * (D + 1) + 2 * AB_TQ * (D + 1) + 2 * AB_TQ * AB_LP) * sizeof(float);
   PV_CUDA(set_max_smem_once(kern, static_cast<int>(smem)));
   dim3 grid(attn_bwd_chunks(S), H, B);
   const float scale = 1.f / sqrtf(static_cast<float>(D));
   kern<<<grid, 256, smem, stream>>>(static_cast<const T*>(dO), static_cast<const T*>(Q), kv_text, kv_img, stats,
                                     static_cast<T*>(dQ), part, B, S, C, H, Lt, Li, w_text, w_img, scale,
-                                    scale * 1.4426950408889634f);
+                                    scale * 1.4426950408889634f, img_row_weight);
   PV_LAUNCHED();
   return PV_OK;
 }
 
 int dual_attn_bwd_mma(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats, void* dQ,
                       float* part, int nchunk, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                      cudaStream_t stream);
+                      cudaStream_t stream, const float* img_row_weight);
 
+// img_row_weight: optional [B, S] fp32 factor of each query row's image keys (nullptr: the unmasked kernels)
 int dual_attn_bwd(bool bf16, const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats,
                   void* dQ, float* part, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                  cudaStream_t stream) {
+                  cudaStream_t stream, const float* img_row_weight) {
   PV_REQUIRE(B > 0 && S > 0 && H > 0 && C % H == 0 && B <= 65535 && H <= 65535, "bad shape");
   PV_REQUIRE(Lt >= 1 && Li >= 1 && Lt + Li <= PV_KEYS_PAD, "need 1 <= Lt, 1 <= Li, Lt+Li <= %d", PV_KEYS_PAD);
   const int d = C / H;
   if (bf16 && g_opt_bwd_mma != 0)       // tensor-core kernel (pv_bwd_mma.cu); the SIMT kernel below is the fp32 parity path
-    return dual_attn_bwd_mma(dO, Q, kv_text, kv_img, stats, dQ, part, attn_bwd_mma_chunks(S, d), B, S, C, H, Lt, Li, w_text, w_img, stream);
+    return dual_attn_bwd_mma(dO, Q, kv_text, kv_img, stats, dQ, part, attn_bwd_mma_chunks(S, d), B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
 #define PV_AB(DD)                                                                                                        \
-  return bf16 ? launch_attn_bwd<DD, __nv_bfloat16>(dO, Q, kv_text, kv_img, stats, dQ, part, B, S, C, H, Lt, Li, w_text, w_img, stream) \
-              : launch_attn_bwd<DD, float>(dO, Q, kv_text, kv_img, stats, dQ, part, B, S, C, H, Lt, Li, w_text, w_img, stream)
+  return bf16 ? launch_attn_bwd<DD, __nv_bfloat16>(dO, Q, kv_text, kv_img, stats, dQ, part, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight) \
+              : launch_attn_bwd<DD, float>(dO, Q, kv_text, kv_img, stats, dQ, part, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight)
   switch (d) {
     case 40: PV_AB(40);
     case 80: PV_AB(80);

@@ -61,12 +61,14 @@ struct BwdMmaCfg {
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
 
-template <int D>
+// MASK: the image keys of query row s are weighted w_img * img_row_weight[b, s] (ip_adapter_masks)
+template <int D, bool MASK>
 __global__ void __launch_bounds__(256, 1)
 attn_bwd_mma_kernel(const __nv_bfloat16* __restrict__ dO, const __nv_bfloat16* __restrict__ Q,
                     const float* __restrict__ kv_text, const float* __restrict__ kv_img, const float* __restrict__ stats,
                     __nv_bfloat16* __restrict__ dQ, float* __restrict__ part, int B, int S, int C, int H, int Lt, int Li,
-                    float w_text, float w_img, float scale, float scale_log2e, int tiles_per_block) {
+                    float w_text, float w_img, float scale, float scale_log2e, int tiles_per_block,
+                    const float* __restrict__ img_row_weight) {
   using Cfg = BwdMmaCfg<D>;
   constexpr int DP = Cfg::DP, PD = Cfg::PD, NT_D = Cfg::NT_D;
   extern __shared__ __align__(16) uint8_t smem_b[];
@@ -186,6 +188,11 @@ attn_bwd_mma_kernel(const __nv_bfloat16* __restrict__ dO, const __nv_bfloat16* _
     }
     // w p^ and scale * ds, packed to bf16: A operands of dQ (from registers) and of phase 2 (through shared memory)
     uint32_t pw[BM_KEYS / 8][2], dsr[BM_KEYS / 8][2];
+    float wi_a = w_img, wi_b = w_img;
+    if constexpr (MASK) {
+      if (row_a < S) wi_a *= __ldg(img_row_weight + static_cast<size_t>(b) * S + row_a);
+      if (row_b < S) wi_b *= __ldg(img_row_weight + static_cast<size_t>(b) * S + row_b);
+    }
 #pragma unroll
     for (int n = 0; n < BM_KEYS / 8; ++n) {
       float pv[4], dv[4];
@@ -194,7 +201,7 @@ attn_bwd_mma_kernel(const __nv_bfloat16* __restrict__ dO, const __nv_bfloat16* _
         const int key = 8 * n + 2 * t + (e & 1);
         const bool lo = e < 2;
         const bool is_t = key < Lt;
-        const float w = is_t ? w_text : w_img;
+        const float w = is_t ? w_text : (lo ? wi_a : wi_b);
         const float delta = lo ? (is_t ? dt_a : di_a) : (is_t ? dt_b : di_b);
         pv[e] = w * sacc[n][e];
         dv[e] = scale * w * sacc[n][e] * (pacc[n][e] - delta);
@@ -318,7 +325,7 @@ int attn_bwd_tc_chunks(int S, int d);
 bool attn_bwd_tc_supported(int d, int C);
 int dual_attn_bwd_tc(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats, void* dQ,
                      float* part, int nchunk, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                     cudaStream_t stream);
+                     cudaStream_t stream, const float* img_row_weight);
 extern int g_opt_bwd_tc;
 
 int attn_bwd_mma_chunks(int S, int d) {
@@ -330,15 +337,15 @@ int attn_bwd_mma_chunks(int S, int d) {
 template <int D>
 static int launch_attn_bwd_mma(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats,
                                void* dQ, float* part, int nchunk, int B, int S, int C, int H, int Lt, int Li, float w_text,
-                               float w_img, cudaStream_t stream) {
-  auto kern = attn_bwd_mma_kernel<D>;
+                               float w_img, cudaStream_t stream, const float* img_row_weight) {
+  auto kern = img_row_weight ? attn_bwd_mma_kernel<D, true> : attn_bwd_mma_kernel<D, false>;
   PV_CUDA(set_max_smem_once(kern, BwdMmaCfg<D>::SMEM_BYTES));
   dim3 grid(nchunk, H, B);
   const float scale = 1.f / sqrtf(static_cast<float>(D));
   kern<<<grid, 256, BwdMmaCfg<D>::SMEM_BYTES, stream>>>(static_cast<const __nv_bfloat16*>(dO), static_cast<const __nv_bfloat16*>(Q),
                                                        kv_text, kv_img, stats, static_cast<__nv_bfloat16*>(dQ), part, B, S, C, H,
                                                        Lt, Li, w_text, w_img, scale, scale * 1.4426950408889634f,
-                                                       attn_bwd_mma_tiles(S, C / H));
+                                                       attn_bwd_mma_tiles(S, C / H), img_row_weight);
   PV_LAUNCHED();
   return PV_OK;
 }
@@ -346,15 +353,15 @@ static int launch_attn_bwd_mma(const void* dO, const void* Q, const float* kv_te
 // bf16 only; nchunk must be attn_bwd_mma_chunks(S, head_dim).  Needs 16-byte aligned Q / dO rows per head (C, head_dim % 8 == 0).
 int dual_attn_bwd_mma(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats, void* dQ,
                       float* part, int nchunk, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                      cudaStream_t stream) {
+                      cudaStream_t stream, const float* img_row_weight) {
   const int d = C / H;
   PV_REQUIRE(nchunk == attn_bwd_mma_chunks(S, d), "chunk count mismatch (%d for S=%d)", nchunk, S);
   if (g_opt_bwd_tc != 0 && attn_bwd_tc_supported(d, d * 8))
-    return dual_attn_bwd_tc(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream);
+    return dual_attn_bwd_tc(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
   switch (d) {
-    case 40: return launch_attn_bwd_mma<40>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream);
-    case 80: return launch_attn_bwd_mma<80>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream);
-    case 160: return launch_attn_bwd_mma<160>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream);
+    case 40: return launch_attn_bwd_mma<40>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
+    case 80: return launch_attn_bwd_mma<80>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
+    case 160: return launch_attn_bwd_mma<160>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
     default: PV_FAIL(PV_ERR_UNSUPPORTED, "head_dim %d unsupported (40/80/160)", d);
   }
 }

@@ -59,9 +59,12 @@ struct BtParams {
   float* part;
   int B, S, C, H, Lt, Li, T;
   float w_text, w_img, scale, scale_log2e;
+  const float* img_row_weight;     // MASK kernels: [B, S] fp32 factor of each query row's image keys (ip_adapter_masks)
 };
 
-template <int D, bool LT77>      // LT77: 77 text keys (CLIP) -- the segment of every key slot is known at compile time
+// LT77: 77 text keys (CLIP) -- the segment of every key slot is known at compile time.  MASK: the image keys of row s are
+// weighted w_img * img_row_weight[b, s].
+template <int D, bool LT77, bool MASK>
 __global__ void __launch_bounds__(BT_THREADS, 1)
 attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmdO, const BtParams p) {
   using Cfg = BtCfg<D>;
@@ -344,7 +347,9 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         // ---- the previous tile: its gradient contractions have completed (the P / dS images are free again) -> my share of dQ
         if (t > 0) drain_dq(t - 1);
         // ---- pass 2: w p^ and scale w p^ (dp - delta) as bf16, 8 keys (16 bytes) at a time
-        const float swt = p.scale * p.w_text, swi = p.scale * p.w_img;
+        float wi = p.w_img;
+        if constexpr (MASK) wi *= grow < S ? __ldg(p.img_row_weight + static_cast<size_t>(b) * S + grow) : 0.f;
+        const float swt = p.scale * p.w_text, swi = p.scale * wi;
 #pragma unroll
         for (int c = 0; c < 6; ++c) {
           uint32_t pw[4], dw[4];
@@ -356,13 +361,13 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
               const bool txt = key + 1 < 77;
               const uint64_t e2 = f2_pack(e[i], e[i + 1]);
               const uint64_t pd = f2_pack(__uint_as_float(dp[i]), __uint_as_float(dp[i + 1]));
-              const float w = txt ? p.w_text : p.w_img, sw = txt ? swt : swi, nd = txt ? -dsum_t : -dsum_i;
+              const float w = txt ? p.w_text : wi, sw = txt ? swt : swi, nd = txt ? -dsum_t : -dsum_i;
               f2_unpack(f2_mul(e2, f2_pack(w, w)), a, b2);
               f2_unpack(f2_mul(f2_mul(e2, f2_pack(sw, sw)), f2_add(pd, f2_pack(nd, nd))), c1, d1);
             } else {
               const bool t0 = LT77 ? true : key < Lt, t1 = LT77 ? false : key + 1 < Lt;
-              a = (t0 ? p.w_text : p.w_img) * e[i];
-              b2 = (t1 ? p.w_text : p.w_img) * e[i + 1];
+              a = (t0 ? p.w_text : wi) * e[i];
+              b2 = (t1 ? p.w_text : wi) * e[i + 1];
               c1 = (t0 ? swt : swi) * e[i] * (__uint_as_float(dp[i]) - (t0 ? dsum_t : dsum_i));
               d1 = (t1 ? swt : swi) * e[i + 1] * (__uint_as_float(dp[i + 1]) - (t1 ? dsum_t : dsum_i));
             }
@@ -421,7 +426,7 @@ bool attn_bwd_tc_supported(int d, int C) { return (d == 40 || d == 80) && C % 8 
 template <int D>
 static int launch_attn_bwd_tc(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats, void* dQ,
                               float* part, int nchunk, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                              cudaStream_t stream) {
+                              cudaStream_t stream, const float* img_row_weight) {
   using Cfg = BtCfg<D>;
   CUtensorMap tmQ, tmdO;
   if (make_tmap_3d(&tmQ, Q, 2, C, S, B, C * 2ull, static_cast<uint64_t>(S) * C * 2, 64, 128, 1, Swz::B128)) return PV_ERR_CUDA;
@@ -433,28 +438,25 @@ static int launch_attn_bwd_tc(const void* dO, const void* Q, const float* kv_tex
   p.w_text = w_text; p.w_img = w_img;
   p.scale = 1.f / sqrtf(static_cast<float>(D));
   p.scale_log2e = p.scale * 1.4426950408889634f;
-  if (Lt == 77) {
-    auto kern = attn_bwd_tc_kernel<D, true>;
-    PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
-    kern<<<dim3(nchunk, H, B), BT_THREADS, Cfg::SMEM_BYTES, stream>>>(tmQ, tmdO, p);
-  } else {
-    auto kern = attn_bwd_tc_kernel<D, false>;
-    PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
-    kern<<<dim3(nchunk, H, B), BT_THREADS, Cfg::SMEM_BYTES, stream>>>(tmQ, tmdO, p);
-  }
+  p.img_row_weight = img_row_weight;
+  const bool mask = img_row_weight != nullptr;
+  auto kern = Lt == 77 ? (mask ? attn_bwd_tc_kernel<D, true, true> : attn_bwd_tc_kernel<D, true, false>)
+                       : (mask ? attn_bwd_tc_kernel<D, false, true> : attn_bwd_tc_kernel<D, false, false>);
+  PV_CUDA(set_max_smem_once(kern, Cfg::SMEM_BYTES));
+  kern<<<dim3(nchunk, H, B), BT_THREADS, Cfg::SMEM_BYTES, stream>>>(tmQ, tmdO, p);
   PV_LAUNCHED();
   return PV_OK;
 }
 
 int dual_attn_bwd_tc(const void* dO, const void* Q, const float* kv_text, const float* kv_img, const float* stats, void* dQ,
                      float* part, int nchunk, int B, int S, int C, int H, int Lt, int Li, float w_text, float w_img,
-                     cudaStream_t stream) {
+                     cudaStream_t stream, const float* img_row_weight) {
   const int d = C / H;
   PV_REQUIRE(nchunk == attn_bwd_tc_chunks(S, d), "chunk count mismatch (%d for S=%d)", nchunk, S);
   PV_REQUIRE((reinterpret_cast<uintptr_t>(dO) | reinterpret_cast<uintptr_t>(Q) | reinterpret_cast<uintptr_t>(dQ)) % 16 == 0,
              "pointers must be 16-byte aligned");
-  if (d == 40) return launch_attn_bwd_tc<40>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream);
-  if (d == 80) return launch_attn_bwd_tc<80>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream);
+  if (d == 40) return launch_attn_bwd_tc<40>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
+  if (d == 80) return launch_attn_bwd_tc<80>(dO, Q, kv_text, kv_img, stats, dQ, part, nchunk, B, S, C, H, Lt, Li, w_text, w_img, stream, img_row_weight);
   PV_FAIL(PV_ERR_UNSUPPORTED, "head_dim %d: tcgen05 backward supports 40 / 80", d);
 }
 

@@ -99,10 +99,12 @@ int gemm_f32(const float* A, const float* W, const float* bias, float* D, long l
 // ------------------------------------------------------------------------------------------------
 constexpr int SA_QPB = 32;
 
+// MASK: the image segment of query row s is weighted w_img * img_row_weight[b, s] (ip_adapter_masks)
+template <bool MASK>
 __global__ void __launch_bounds__(128)
 simt_dual_attn_f32_kernel(const float* __restrict__ Q, const float* __restrict__ Kg, const float* __restrict__ Vg,
                           float* __restrict__ O, float* __restrict__ stats, int S, int C, int H, int d, int Lt, int Li,
-                          float w_text, float w_img, float scale_log2e) {
+                          float w_text, float w_img, float scale_log2e, const float* __restrict__ img_row_weight) {
   extern __shared__ float sm[];
   const int L = Lt + Li;
   const int dk = d + 1;                     // padded K row: conflict-free when lanes walk keys
@@ -162,7 +164,8 @@ simt_dual_attn_f32_kernel(const float* __restrict__ Q, const float* __restrict__
       li += __shfl_xor_sync(0xffffffffu, li, o);
     }
     const float at = w_text / lt;
-    const float ai = (Li > 0) ? w_img / li : 0.f;
+    const float wi = MASK ? w_img * __ldg(img_row_weight + static_cast<size_t>(b) * S + srow) : w_img;
+    const float ai = (Li > 0) ? wi / li : 0.f;
 #pragma unroll
     for (int t = 0; t < 3; ++t) {
       const int k = lane + 32 * t;
@@ -184,21 +187,23 @@ simt_dual_attn_f32_kernel(const float* __restrict__ Q, const float* __restrict__
 }
 
 int dual_attn_core_f32(const float* Q, const float* Kp, const float* Vp, float* O, float* stats, int B, int S, int C,
-                       int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream) {
+                       int H, int Lt, int Li, float w_text, float w_img, cudaStream_t stream, const float* img_row_weight) {
   PV_REQUIRE(B > 0 && S > 0 && H > 0 && C % H == 0, "bad shape");
   PV_REQUIRE(Lt >= 1 && Li >= 1 && Lt + Li <= PV_KEYS_PAD, "need 1 <= Lt, 1 <= Li, Lt+Li <= %d", PV_KEYS_PAD);
   const int d = C / H, L = Lt + Li;
   const size_t smem = (static_cast<size_t>(L) * (d + 1) + static_cast<size_t>(L) * d + 4 * d + 4 * PV_KEYS_PAD) * sizeof(float);
   PV_REQUIRE(smem <= 200 * 1024, "head_dim %d too large for the fp32 kernel", d);
-  static size_t attr_smem = 0;
-  if (smem > attr_smem) {
-    PV_CUDA(cudaFuncSetAttribute(simt_dual_attn_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem = smem;
+  const bool mask = img_row_weight != nullptr;
+  auto kern = mask ? simt_dual_attn_f32_kernel<true> : simt_dual_attn_f32_kernel<false>;
+  static size_t attr_smem[2] = {0, 0};
+  if (smem > attr_smem[mask]) {
+    PV_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr_smem[mask] = smem;
   }
   PV_REQUIRE(B <= 65535 && H <= 65535, "grid too large");
   dim3 grid((S + SA_QPB - 1) / SA_QPB, H, B);
-  simt_dual_attn_f32_kernel<<<grid, 128, smem, stream>>>(Q, Kp, Vp, O, stats, S, C, H, d, Lt, Li, w_text, w_img,
-                                                         1.4426950408889634f / sqrtf(static_cast<float>(d)));
+  kern<<<grid, 128, smem, stream>>>(Q, Kp, Vp, O, stats, S, C, H, d, Lt, Li, w_text, w_img,
+                                    1.4426950408889634f / sqrtf(static_cast<float>(d)), img_row_weight);
   PV_LAUNCHED();
   return PV_OK;
 }

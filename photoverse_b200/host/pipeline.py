@@ -22,6 +22,7 @@ from typing import List, Optional
 import torch
 
 from .. import _lib
+from ..attention_processor import release_mask_rows
 from ..unet import prepare_kv, set_kv_cache
 from .ddim import make_ddim_schedule
 from .dpm_solver import make_dpmpp_2m_schedule
@@ -49,7 +50,7 @@ class GenInputs:
 class _GraphedUNet:
     """One UNet evaluation captured in a CUDA graph (static input buffers, replayed every step)."""
 
-    def __init__(self, unet, latent_shape, ctx, dtype, device):
+    def __init__(self, unet, latent_shape, ctx, dtype, device, cak=None):
         self.unet = unet
         self.ctx = ctx
         self.x = torch.zeros(latent_shape, device=device, dtype=dtype)
@@ -57,12 +58,12 @@ class _GraphedUNet:
         s = torch.cuda.Stream(device=device)
         s.wait_stream(torch.cuda.current_stream(device))
         with torch.cuda.stream(s):
-            for _ in range(2):       # warm-up outside capture: packs weights, fills the K/V cache, cuDNN autotune
-                unet(self.x, self.t, encoder_hidden_states=ctx)
+            for _ in range(2):       # warm-up outside capture: packs weights, fills the K/V (and mask) caches, cuDNN autotune
+                unet(self.x, self.t, encoder_hidden_states=ctx, cross_attention_kwargs=cak)
         torch.cuda.current_stream(device).wait_stream(s)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
-            self.out = unet(self.x, self.t, encoder_hidden_states=ctx).sample
+            self.out = unet(self.x, self.t, encoder_hidden_states=ctx, cross_attention_kwargs=cak).sample
 
     def __call__(self, x, t_dev):
         self.x.copy_(x)
@@ -84,17 +85,30 @@ def _autocast(dtype: Optional[torch.dtype]):
 def run_generation(unet, image_adapter, text_adapter, inputs: GenInputs, num_steps: int = 50,
                    guidance_scale: float = 1.0, token_index=0, mode: str = "batched", use_cuda_graph: bool = True,
                    kv_cache: bool = True, return_aux: bool = False, scheduler: str = "ddim",
-                   autocast_dtype: Optional[torch.dtype] = None):
+                   autocast_dtype: Optional[torch.dtype] = None, ip_adapter_masks=None):
     """Returns the final latents [B,4,h,w] (and the adapter outputs if ``return_aux``).  ``autocast_dtype``: run the
     adapters and every UNet evaluation (warm-up, graph capture and replay) under ``torch.autocast("cuda", autocast_dtype)``
-    -- a float32 model in the reference's mixed precision."""
+    -- a float32 model in the reference's mixed precision.  ``ip_adapter_masks``: diffusers' regional identity masks
+    (a list with one [1 or B, 1, H, W] tensor), passed to every UNet evaluation as ``cross_attention_kwargs``; with
+    batched CFG a mask of batch B is repeated for the unconditional half, as the diffusers pipeline does."""
     with _autocast(autocast_dtype):
         return _run_generation(unet, image_adapter, text_adapter, inputs, num_steps, guidance_scale, token_index, mode,
-                               use_cuda_graph, kv_cache, return_aux, scheduler)
+                               use_cuda_graph, kv_cache, return_aux, scheduler, ip_adapter_masks)
+
+
+def _mask_kwargs(ip_adapter_masks, batched: bool):
+    """``cross_attention_kwargs`` of the UNet evaluations: with batched CFG the rows are [uncond | cond], so a mask of
+    batch B > 1 is concatenated with itself (a mask of batch 1 broadcasts already)."""
+    if ip_adapter_masks is None:
+        return None
+    masks = list(ip_adapter_masks.unsqueeze(1)) if isinstance(ip_adapter_masks, torch.Tensor) else list(ip_adapter_masks)
+    if batched:
+        masks = [m if (not isinstance(m, torch.Tensor) or m.shape[0] == 1) else torch.cat([m, m]) for m in masks]
+    return {"ip_adapter_masks": masks}
 
 
 def _run_generation(unet, image_adapter, text_adapter, inputs, num_steps, guidance_scale, token_index, mode,
-                    use_cuda_graph, kv_cache, return_aux, scheduler):
+                    use_cuda_graph, kv_cache, return_aux, scheduler, ip_adapter_masks=None):
     assert mode in ("batched", "two_call", "cond_only")
     if mode == "cond_only" and guidance_scale != 1.0:
         raise ValueError("mode='cond_only' drops the unconditional branch: only valid for guidance_scale == 1")
@@ -120,13 +134,14 @@ def _run_generation(unet, image_adapter, text_adapter, inputs, num_steps, guidan
     else:
         ctxs = [(inputs.text.contiguous(), img_tokens.contiguous())]
 
+    cak = _mask_kwargs(ip_adapter_masks, mode == "batched")
     set_kv_cache(unet, kv_cache)
     ts_dev = torch.tensor(sched.timesteps, device=dev, dtype=torch.float32)
     rows = 2 * B if mode == "batched" else B
     lat_shape = (rows,) + tuple(latents.shape[1:])
     evals = None
     if use_cuda_graph and dev.type == "cuda":
-        evals = [_GraphedUNet(unet, lat_shape, c, dtype, dev) for c in ctxs]
+        evals = [_GraphedUNet(unet, lat_shape, c, dtype, dev, cak) for c in ctxs]
     try:
         for i in range(num_steps):
             t_dev = ts_dev[i:i + 1]
@@ -136,7 +151,7 @@ def _run_generation(unet, image_adapter, text_adapter, inputs, num_steps, guidan
                 if evals is not None:
                     outs.append(evals[j](x_in, t_dev))
                 else:
-                    outs.append(unet(x_in, t_dev, encoder_hidden_states=c).sample)
+                    outs.append(unet(x_in, t_dev, encoder_hidden_states=c, cross_attention_kwargs=cak).sample)
             if mode == "batched":
                 eps_u, eps_c = outs[0].chunk(2)
             elif mode == "two_call":
@@ -191,9 +206,11 @@ class GenerationEngine:
     def __init__(self, unet, image_adapter, text_adapter, batch: int, latent: int = 64, num_steps: int = 50,
                  guidance_scale: float = 1.0, token_index=0, mode: str = "batched", dtype=torch.bfloat16,
                  device="cuda", num_heads_T: int = 5, use_cuda_graph: bool = True,
-                 autocast_dtype: Optional[torch.dtype] = None):
+                 autocast_dtype: Optional[torch.dtype] = None, ip_mask_shape=None):
         """``dtype``: the model's and the encoder buffers' dtype; ``autocast_dtype``: run the adapters and the UNet
-        evaluations (warm-up, capture, replay) under ``torch.autocast("cuda", autocast_dtype)`` (None: off)."""
+        evaluations (warm-up, capture, replay) under ``torch.autocast("cuda", autocast_dtype)`` (None: off).
+        ``ip_mask_shape`` (H, W): every generation applies a regional identity mask (diffusers' ``ip_adapter_masks``) of
+        that size, a static fp32 input set by :meth:`load_inputs`; it is downsampled inside the captured evaluation."""
         assert mode in ("batched", "two_call", "cond_only")
         if mode == "cond_only" and guidance_scale != 1.0:
             raise ValueError("mode='cond_only' is only valid for guidance_scale == 1")
@@ -216,17 +233,27 @@ class GenerationEngine:
         self.outs = None
         self.launches_per_eval = 0      # native kernels inside one captured UNet evaluation
         self.replays = 0
+        self.ip_mask = None
+        if ip_mask_shape is not None:
+            self.ip_mask = torch.ones(1, 1, *ip_mask_shape, device=self.dev, dtype=torch.float32)
+        self._mask_rows = []
         set_kv_cache(unet, True, static=True)
 
-    def load_inputs(self, host_inputs: GenInputs):
-        """Host (pinned) -> static device buffers; asynchronous on the current stream."""
+    def load_inputs(self, host_inputs: GenInputs, ip_mask: Optional[torch.Tensor] = None):
+        """Host (pinned) -> static device buffers; asynchronous on the current stream.  ``ip_mask`` [1, 1, H, W]: the
+        regional identity mask of the following generations (engines built with ``ip_mask_shape`` only)."""
         for dst, src in zip(self.inp.clip_hidden + self.inp.clip_hidden_uncond + [self.inp.text, self.inp.text_uncond, self.inp.noise],
                             host_inputs.clip_hidden + host_inputs.clip_hidden_uncond
                             + [host_inputs.text, host_inputs.text_uncond, host_inputs.noise]):
             dst.copy_(src, non_blocking=True)
+        if ip_mask is not None:
+            if self.ip_mask is None:
+                raise ValueError("this GenerationEngine was built without ip_mask_shape")
+            self.ip_mask.copy_(ip_mask.reshape(self.ip_mask.shape), non_blocking=True)
 
     def _eval(self, j):
-        return self.unet(self.x_in, self.t_in, encoder_hidden_states=self.ctx[j]).sample
+        cak = None if self.ip_mask is None else {"ip_adapter_masks": [self.ip_mask]}
+        return self.unet(self.x_in, self.t_in, encoder_hidden_states=self.ctx[j], cross_attention_kwargs=cak).sample
 
     def _build_graphs(self):
         s = torch.cuda.Stream(device=self.dev)
@@ -239,9 +266,13 @@ class GenerationEngine:
         self.graphs, self.outs = [], []
         for j in range(len(self.ctx)):
             g = torch.cuda.CUDAGraph()
+            if self.ip_mask is not None:      # the capture downsamples the static mask: every replay sees its contents
+                release_mask_rows(self.ip_mask)
             n0 = _lib.launch_count()
             with torch.cuda.graph(g):
                 out = self._eval(j)
+            if self.ip_mask is not None:
+                self._mask_rows += release_mask_rows(self.ip_mask)      # the graph's row buffers, kept alive here
             self.launches_per_eval = _lib.launch_count() - n0
             self.graphs.append(g)
             self.outs.append(out)

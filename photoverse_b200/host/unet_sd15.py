@@ -260,18 +260,20 @@ class BasicTransformerBlock(nn.Module):
         self.norm3 = nn.LayerNorm(dim)
         self.ff = FeedForward(dim)
 
-    def forward(self, x, encoder_hidden_states):
+    def forward(self, x, encoder_hidden_states, cross_attention_kwargs=None):
+        # diffusers passes cross_attention_kwargs (e.g. ip_adapter_masks) to both attention layers
+        kw = cross_attention_kwargs or {}
         if (_fused(self.norm2, x) and _fused(self.norm3, x) and x.is_contiguous() and x.shape[-1] % 8 == 0
                 and x.shape[-1] <= 1280):
             # inference: each residual sum rides in the pass of the LayerNorm that follows it
             from .. import ops
-            h = self.attn1(layer_norm(self.norm1, x))
+            h = self.attn1(layer_norm(self.norm1, x), **kw)
             x, n = ops.add_layer_norm(h.contiguous(), x, *_f32_params(self.norm2, "weight", "bias"), self.norm2.eps)
-            h = self.attn2(n, encoder_hidden_states=encoder_hidden_states)
+            h = self.attn2(n, encoder_hidden_states=encoder_hidden_states, **kw)
             x, n = ops.add_layer_norm(h.contiguous(), x, *_f32_params(self.norm3, "weight", "bias"), self.norm3.eps)
             return self.ff(n) + x
-        x = self.attn1(layer_norm(self.norm1, x)) + x
-        x = self.attn2(layer_norm(self.norm2, x), encoder_hidden_states=encoder_hidden_states) + x
+        x = self.attn1(layer_norm(self.norm1, x), **kw) + x
+        x = self.attn2(layer_norm(self.norm2, x), encoder_hidden_states=encoder_hidden_states, **kw) + x
         return self.ff(layer_norm(self.norm3, x)) + x
 
 
@@ -283,7 +285,7 @@ class Transformer2DModel(nn.Module):
         self.transformer_blocks = nn.ModuleList([BasicTransformerBlock(channels, heads, cross_attention_dim)])
         self.proj_out = nn.Conv2d(channels, channels, 1)
 
-    def forward(self, x, encoder_hidden_states):
+    def forward(self, x, encoder_hidden_states, cross_attention_kwargs=None):
         B, C, H, W = x.shape
         res = x
         if _enabled(self.norm, x) and _nhwc(x):
@@ -292,14 +294,14 @@ class Transformer2DModel(nn.Module):
             h = group_norm_act(self.norm, x, False).permute(0, 2, 3, 1).reshape(B, H * W, C)
             h = F.linear(h, self.proj_in.weight.view(C, C), self.proj_in.bias)
             for blk in self.transformer_blocks:
-                h = blk(h, encoder_hidden_states)
+                h = blk(h, encoder_hidden_states, cross_attention_kwargs)
             h = F.linear(h, self.proj_out.weight.view(C, C), self.proj_out.bias)
             h = h + res.permute(0, 2, 3, 1).reshape(B, H * W, C)
             return h.reshape(B, H, W, C).permute(0, 3, 1, 2)
         h = self.proj_in(group_norm_act(self.norm, x, False))
         h = h.permute(0, 2, 3, 1).reshape(B, H * W, C)
         for blk in self.transformer_blocks:
-            h = blk(h, encoder_hidden_states)
+            h = blk(h, encoder_hidden_states, cross_attention_kwargs)
         h = h.reshape(B, H, W, C).permute(0, 3, 1, 2)      # NHWC-strided view: free under channels_last
         return self.proj_out(h) + res
 
@@ -383,12 +385,12 @@ class DownBlock(nn.Module):
             [Transformer2DModel(cout, heads, cross_dim) for _ in range(layers)]) if has_attn else None
         self.downsamplers = nn.ModuleList([Downsample2D(cout)]) if add_down else None
 
-    def forward(self, x, temb, ctx):
+    def forward(self, x, temb, ctx, cross_attention_kwargs=None):
         outs = []
         for i, r in enumerate(self.resnets):
             x = r(x, temb)
             if self.attentions is not None:
-                x = self.attentions[i](x, ctx)
+                x = self.attentions[i](x, ctx, cross_attention_kwargs)
             outs.append(x)
         if self.downsamplers is not None:
             x = self.downsamplers[0](x)
@@ -409,12 +411,12 @@ class UpBlock(nn.Module):
             [Transformer2DModel(cout, heads, cross_dim) for _ in range(layers)]) if has_attn else None
         self.upsamplers = nn.ModuleList([Upsample2D(cout)]) if add_up else None
 
-    def forward(self, x, skips, temb, ctx):
+    def forward(self, x, skips, temb, ctx, cross_attention_kwargs=None):
         for i, r in enumerate(self.resnets):
             x = torch.cat([x, skips.pop()], dim=1)
             x = r(x, temb)
             if self.attentions is not None:
-                x = self.attentions[i](x, ctx)
+                x = self.attentions[i](x, ctx, cross_attention_kwargs)
         if self.upsamplers is not None:
             x = self.upsamplers[0](x)
         return x
@@ -426,9 +428,9 @@ class MidBlock(nn.Module):
         self.resnets = nn.ModuleList([ResnetBlock2D(ch, ch, temb_ch), ResnetBlock2D(ch, ch, temb_ch)])
         self.attentions = nn.ModuleList([Transformer2DModel(ch, heads, cross_dim)])
 
-    def forward(self, x, temb, ctx):
+    def forward(self, x, temb, ctx, cross_attention_kwargs=None):
         x = self.resnets[0](x, temb)
-        x = self.attentions[0](x, ctx)
+        x = self.attentions[0](x, ctx, cross_attention_kwargs)
         return self.resnets[1](x, temb)
 
 
@@ -514,7 +516,9 @@ class UNetSD15(nn.Module):
                 m._pv_fused = bool(enabled)
         return self
 
-    def forward(self, sample, timestep, encoder_hidden_states):
+    def forward(self, sample, timestep, encoder_hidden_states, cross_attention_kwargs=None):
+        """``cross_attention_kwargs``: extra keyword arguments of every attention processor call, as diffusers'
+        ``UNet2DConditionModel`` passes them (e.g. ``{"ip_adapter_masks": [mask]}``)."""
         if not torch.is_tensor(timestep):
             timestep = torch.tensor([timestep], device=sample.device)
         t = timestep.reshape(-1).expand(sample.shape[0]) if timestep.numel() == 1 else timestep
@@ -522,10 +526,10 @@ class UNetSD15(nn.Module):
         x = self.conv_in(sample)
         skips = [x]
         for blk in self.down_blocks:
-            x, outs = blk(x, temb, encoder_hidden_states)
+            x, outs = blk(x, temb, encoder_hidden_states, cross_attention_kwargs)
             skips += outs
-        x = self.mid_block(x, temb, encoder_hidden_states)
+        x = self.mid_block(x, temb, encoder_hidden_states, cross_attention_kwargs)
         for blk in self.up_blocks:
-            x = blk(x, skips, temb, encoder_hidden_states)
+            x = blk(x, skips, temb, encoder_hidden_states, cross_attention_kwargs)
         x = self.conv_out(group_norm_act(self.conv_norm_out, x, True))
         return SimpleNamespace(sample=x)

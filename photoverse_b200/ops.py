@@ -189,9 +189,30 @@ def _sync_words(B: int, S: int, device) -> torch.Tensor:
     return buf
 
 
+def ip_mask_rows(mask: torch.Tensor, B: int, S: int) -> torch.Tensor:
+    """fp32 [B, S] row weights of a regional identity mask ``mask`` [1|B, H_m, W_m] (CUDA, float32) on a query grid of S
+    rows: diffusers 0.27.2 ``IPAdapterMaskProcessor.downsample`` (bicubic to its mask_h x mask_w grid, repeated to the
+    batch, zero-padded to S) in one pv_ip_mask_downsample launch."""
+    if not mask.is_cuda or mask.dtype != torch.float32 or mask.dim() != 3:
+        raise _lib.PhotoverseB200Error("ip_mask_rows: a float32 CUDA mask [1|B, H, W] is required")
+    m = mask.contiguous()
+    out = torch.empty(B, S, device=m.device, dtype=torch.float32)
+    check(_lib.lib().pv_ip_mask_downsample(_ptr(m), m.shape[0], m.shape[1], m.shape[2], _ptr(out), B, S, _stream()),
+          "pv_ip_mask_downsample")
+    return out
+
+
+def _row_weight(rw: Optional[torch.Tensor], B: int, S: int, device):
+    if rw is not None:
+        assert rw.dtype == torch.float32 and rw.is_contiguous() and rw.shape == (B, S) and rw.device == device
+    return _ptr(rw)
+
+
 def dual_attn(x: torch.Tensor, wq: torch.Tensor, kv: PackedKV, wo: torch.Tensor, bo: torch.Tensor,
-              w_text: float = 1.0, w_img: float = 1.0, want_stats: bool = False):
-    """Y = (w_t softmax(QK_t^T/sqrt d) V_t + w_i softmax(QK_i^T/sqrt d) V_i) Wo^T + bo with Q = x Wq^T.
+              w_text: float = 1.0, w_img: float = 1.0, want_stats: bool = False,
+              img_row_weight: Optional[torch.Tensor] = None):
+    """Y = (w_t softmax(QK_t^T/sqrt d) V_t + w_i m softmax(QK_i^T/sqrt d) V_i) Wo^T + bo with Q = x Wq^T and m the
+    fp32 [B, S] ``img_row_weight`` of :func:`ip_mask_rows` (None: 1).
     Returns (Y, O, stats|None, Q|None); O (pre-out-projection) and Q (fp32 mode only) are kept for backward."""
     B, S, C = x.shape
     sync = _sync_words(B, S, x.device) if x.dtype in HALF_DTYPES else None
@@ -202,25 +223,28 @@ def dual_attn(x: torch.Tensor, wq: torch.Tensor, kv: PackedKV, wo: torch.Tensor,
     o = torch.empty_like(x)
     q = torch.empty(B, S, C, device=x.device, dtype=torch.float32) if x.dtype == torch.float32 else None
     stats = torch.empty(B, kv.H, S, 4, device=x.device, dtype=torch.float32) if want_stats else None
-    check(_lib.lib().pv_dual_attn_fwd(_dt(x), _ptr(x), _ptr(wq), _ptr(kv.Kp), _ptr(kv.Vp), _ptr(wo), _ptr(bo),
-                                      _ptr(y), _ptr(q), _ptr(o), _ptr(stats), _ptr(sync), B, S, C, kv.H, kv.Lt, kv.Li,
-                                      float(w_text), float(w_img), _stream()), "pv_dual_attn_fwd")
+    rw = _row_weight(img_row_weight, B, S, x.device)
+    check(_lib.lib().pv_dual_attn_masked_fwd(_dt(x), _ptr(x), _ptr(wq), _ptr(kv.Kp), _ptr(kv.Vp), _ptr(wo), _ptr(bo),
+                                             _ptr(y), _ptr(q), _ptr(o), _ptr(stats), _ptr(sync), B, S, C, kv.H, kv.Lt,
+                                             kv.Li, float(w_text), float(w_img), rw, _stream()), "pv_dual_attn_masked_fwd")
     return y, o, stats, q
 
 
 def dual_attn_core(x_or_q: torch.Tensor, wq: Optional[torch.Tensor], kv: PackedKV, w_text: float = 1.0,
-                   w_img: float = 1.0, want_stats: bool = False):
+                   w_img: float = 1.0, want_stats: bool = False, img_row_weight: Optional[torch.Tensor] = None):
     """The attention kernel alone (no out projection).  bf16 / fp16: ``x_or_q`` = X and ``wq`` is applied inside the
-    kernel; fp32: ``x_or_q`` = Q (already projected), ``wq`` ignored.  Returns (O [B,S,C], stats|None)."""
+    kernel; fp32: ``x_or_q`` = Q (already projected), ``wq`` ignored.  ``img_row_weight`` as in :func:`dual_attn`.
+    Returns (O [B,S,C], stats|None)."""
     B, S, C = x_or_q.shape
     assert x_or_q.is_contiguous() and x_or_q.dtype == kv.dtype and (kv.B, kv.C) == (B, C)
     if x_or_q.dtype in HALF_DTYPES:
         assert wq is not None and wq.is_contiguous() and wq.dtype == x_or_q.dtype and wq.shape == (C, C)
     o = torch.empty_like(x_or_q)
     stats = torch.empty(B, kv.H, S, 4, device=o.device, dtype=torch.float32) if want_stats else None
-    check(_lib.lib().pv_dual_attn_core_fwd(_dt(x_or_q), _ptr(x_or_q), _ptr(wq), _ptr(kv.Kp), _ptr(kv.Vp), _ptr(o),
-                                           _ptr(stats), B, S, C, kv.H, kv.Lt, kv.Li, float(w_text), float(w_img),
-                                           _stream()), "pv_dual_attn_core_fwd")
+    rw = _row_weight(img_row_weight, B, S, x_or_q.device)
+    check(_lib.lib().pv_dual_attn_masked_core_fwd(_dt(x_or_q), _ptr(x_or_q), _ptr(wq), _ptr(kv.Kp), _ptr(kv.Vp), _ptr(o),
+                                                  _ptr(stats), B, S, C, kv.H, kv.Lt, kv.Li, float(w_text), float(w_img),
+                                                  rw, _stream()), "pv_dual_attn_masked_core_fwd")
     return o, stats
 
 
@@ -355,8 +379,9 @@ def group_mean_bwd(dy: torch.Tensor, P: int) -> torch.Tensor:
 
 def dual_attn_bwd(d_o: torch.Tensor, q: torch.Tensor, kv_text: torch.Tensor, kv_img: torch.Tensor, stats: torch.Tensor,
                   v_ip_norm: torch.Tensor, d_vnorm: Optional[torch.Tensor], H: int, Lt: int, Li: int, w_text: float,
-                  w_img: float):
-    """(dQ [B,S,C], dkv_text [B*Lt,2C], dkv_img [B*Li,2C]) in the compute dtype."""
+                  w_img: float, img_row_weight: Optional[torch.Tensor] = None):
+    """(dQ [B,S,C], dkv_text [B*Lt,2C], dkv_img [B*Li,2C]) in the compute dtype.  ``img_row_weight``: the forward's row
+    weights (no gradient flows to them)."""
     B, S, C = d_o.shape
     assert d_o.is_contiguous() and q.is_contiguous() and q.dtype == d_o.dtype and stats.is_contiguous()
     dq = torch.empty_like(d_o)
@@ -364,8 +389,10 @@ def dual_attn_bwd(d_o: torch.Tensor, q: torch.Tensor, kv_text: torch.Tensor, kv_
     dkv_img = torch.empty(B * Li, 2 * C, device=d_o.device, dtype=d_o.dtype)
     lib = _lib.lib()
     ws = _workspace(lib.pv_dual_attn_bwd_ws_bytes(B, S, C, H, Lt, Li), d_o.device)
-    check(lib.pv_dual_attn_bwd(_dt(d_o), _ptr(d_o), _ptr(q), _ptr(kv_text), _ptr(kv_img), _ptr(stats), _ptr(dq), _ptr(ws),
-                               B, S, C, H, Lt, Li, float(w_text), float(w_img), _stream()), "pv_dual_attn_bwd")
+    rw = _row_weight(img_row_weight, B, S, d_o.device)
+    check(lib.pv_dual_attn_masked_bwd(_dt(d_o), _ptr(d_o), _ptr(q), _ptr(kv_text), _ptr(kv_img), _ptr(stats), _ptr(dq),
+                                      _ptr(ws), B, S, C, H, Lt, Li, float(w_text), float(w_img), rw, _stream()),
+          "pv_dual_attn_masked_bwd")
     if d_vnorm is not None:
         d_vnorm = d_vnorm.to(torch.float32).contiguous()
     check(lib.pv_kv_pack_bwd(_dt(d_o), _ptr(ws), _ptr(kv_img), _ptr(v_ip_norm), _ptr(d_vnorm), _ptr(dkv_text), _ptr(dkv_img),
